@@ -2,6 +2,7 @@
 """bench.py — the reference's headline metric on B200: octree build nodes-fitted/s (+ Query points/s) vs CPU.
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            our arm (CUDA through the C ABI)
+    python bench.py ... --dump-outputs DIR                         + the headline tree of the last timed step as DIR/*.npy
     python bench.py --impl reference [--steps K] [--warmup W]      the reference's own CPU implementation (oracle/_ref)
     torchrun --nproc-per-node N ... bench.py --gpus N ...          N > 1: one rank per GPU (NCCL)
 
@@ -328,6 +329,19 @@ def bench_c3(cx, args, clk_holder):
     return out, tree, mesh, verts, tris, box, cfg
 
 
+def dump_outputs(hp, tree, out_dir):
+    """The tree of the last timed Create as its caller reads it back (ToMemoryBlock), leaves in canonical order (depth first
+    by child slot), so that two builds compare array for array even where they number their nodes differently. The headline
+    tree holds about 0.8 MB of coefficients."""
+    paths, depth, deg, cs = leaf_table(hp.parse_block(tree.ToMemoryBlockBytes()), hp.COEFF_COUNT)
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"leaf_code": np.array([path_code(p) for p in paths], np.float64),       # 3 bits per level: exact in float64
+              "leaf_depth": depth.astype(np.float64), "leaf_degree": deg.astype(np.float64),
+              "leaf_coeffs": np.concatenate(cs).astype(np.float64)}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def bench_c5(cx, tree, box):
     """configs[4]: 1e9 Philox points (key = seed, counter = global point index) on the C3 octree, replicated tree, points sharded
     contiguously, generated on the device in chunks of 2^26 (untimed); every N evaluates the same point set."""
@@ -619,6 +633,7 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--only", default="", help="comma list of legs to run besides the headline: c1,c2,c4,c5,query (default: all)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the headline tree of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference_arm(args)
@@ -632,6 +647,8 @@ def main():
     fp64_peak = hp.measure_fp64_peak(cx.local, cx.stream)
     clk = []
     c3, tree3, mesh3, verts3, tris3, box3, cfg3 = bench_c3(cx, args, clk)
+    if args.dump_outputs and cx.rank == 0:
+        dump_outputs(hp, tree3, args.dump_outputs)
     st = c3["stats"]
     cpu3 = None
     if with_cpu:

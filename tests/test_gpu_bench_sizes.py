@@ -3,9 +3,9 @@
 * C3 (870 000 triangles, threshold 1e-6, continuity strength 8): the whole tree against the CPU oracle (tens of seconds of
   host time on the box's cores).
 * C4 (1.6 M triangles, threshold 1e-8, max degree 6): far too large for a CPU build inside a test, so parity is sampled:
-  200 random leaves of the GPU tree are refitted with the REFERENCE's own FitPolynomial over the reference's own Mesh + BVH
-  (oracle/_ref), replaying each leaf's history from the build's apply log (from-scratch fit, then kept-shell fits), and the
-  reference's FromMemoryBlock + Query reads the GPU tree back.
+  200 random leaves of the GPU tree are refitted with the CPU oracle's FitPolynomial over its Mesh + BVH (the restatement
+  that tests/test_oracle_golden.py pins to the reference's own output), replaying each leaf's history from the build's apply
+  log (from-scratch fit, then kept-shell fits), and the oracle's FromMemoryBlock + Query reads the GPU tree back.
 * C5: the Philox point stream is the numpy statement's, chunking / sharding do not change a single value.
 """
 import os
@@ -79,7 +79,18 @@ def leaf_histories(blk, log):
     return out
 
 
-def test_c4_full_size_sampled_refit_with_the_reference(hp, ref):
+def refit_chain(oracle, cfg, prog, mn, mx, d0, d1, depth):
+    """One leaf's history replayed with the oracle's FitPolynomial: from scratch at degree d0, then kept-shell fits up to d1."""
+    coeffs, kept = None, 0
+    for d in range(d0, d1 + 1):
+        coeffs, _ = oracle.oracle_fit(cfg, prog, mn, mx, d, depth, kept, coeffs)
+        kept = d
+    return coeffs
+
+
+def test_c4_full_size_sampled_refit_with_the_oracle(hp, oracle):
+    from concurrent.futures import ThreadPoolExecutor
+    from oracle import hpref
     v, t = bumpy_torus(1000, 800)
     lo, hi = mesh_root(v)
     m = hp.Mesh(v, t)
@@ -92,25 +103,27 @@ def test_c4_full_size_sampled_refit_with_the_reference(hp, ref):
     leaves = np.array(sorted(hist))
     assert blk["nodes"]["deg"][leaves].max() <= 6
     pick = np.random.default_rng(11).choice(leaves, 200, replace=False)
-    rm = ref.RefMesh.create(v, t, True)
-    rcfg = ref.make_config(threshold=1e-8, continuity=False, root_min=lo, root_max=hi, threads=THREADS)
-    rprog = ref.make_program([("mesh", [], rm.h)])
+    om = oracle.OracleMesh(v, t)
+    ocfg = hpref.make_config(threshold=1e-8, continuity=False, root_min=lo, root_max=hi, threads=THREADS)
+    oprog = hpref.make_program([("mesh", [], om.h)])
     nodes = blk["nodes"]
-    coeffs, _ = ref.ref_fit_chain_batch(rcfg, rprog, nodes["mn"][pick], nodes["mx"][pick], [hist[int(i)][0] for i in pick],
-                                        [hist[int(i)][1] for i in pick], nodes["depth"][pick], threads=THREADS)
+    oracle.tables()                   # initialises the oracle's constant tables before the threads below share them
+    with ThreadPoolExecutor(THREADS) as pool:       # ctypes releases the GIL: the fits run in parallel
+        coeffs = list(pool.map(lambda i: refit_chain(oracle, ocfg, oprog, nodes["mn"][i], nodes["mx"][i], hist[int(i)][0], hist[int(i)][1],
+                                                     int(nodes["depth"][i])), pick))
     worst = 0.0
     for k, i in enumerate(pick):
         s, n = int(nodes["cstart"][i]), hp.COEFF_COUNT[int(nodes["deg"][i])]
         worst = max(worst, rel_inf(blk["coeffs"][s:s + n], coeffs[k]))
     assert worst <= 1e-10, worst
-    # the reference's own FromMemoryBlock + Query on the GPU-built tree
-    rt = ref.RefTree.from_block(raw)
+    # the oracle's FromMemoryBlock + Query on the GPU-built tree
+    ot = oracle.OracleTree.from_block(raw)
     pts = np.random.default_rng(12).uniform(lo, hi, (200000, 3))
-    dq = np.abs(rt.query(pts, THREADS) - tree.Query(pts)).max()
+    dq = np.abs(ot.query(pts, THREADS) - tree.Query(pts)).max()
     assert dq <= 1e-9, dq
     st = tree.stats()
-    print("C4 full size: nodes", st["n_nodes"], "coeffs", st["n_coeffs"], "ms", st["total_ms"], "| 200 leaves refitted by the reference: worst |dc|/|c|",
-          worst, "| reference Query of the GPU tree: max |d|", dq, "| degrees of the sample", np.bincount(nodes["deg"][pick], minlength=7).tolist())
+    print("C4 full size: nodes", st["n_nodes"], "coeffs", st["n_coeffs"], "ms", st["total_ms"], "| 200 leaves refitted by the oracle: worst |dc|/|c|",
+          worst, "| oracle Query of the GPU tree: max |d|", dq, "| degrees of the sample", np.bincount(nodes["deg"][pick], minlength=7).tolist())
 
 
 def test_philox_points_are_the_numpy_stream_and_sharding_invariant(hp):
