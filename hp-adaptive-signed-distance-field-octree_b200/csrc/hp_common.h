@@ -180,7 +180,7 @@ namespace hpsdf
     {
         const BvhNode*  nodes;
         const void*     obb;          // 4 float4 per node: oriented box in the frame of the node's mean normal (mesh.cpp), see mesh_eval.cuh
-        const void*     wide;         // 4-wide collapse of the same tree for meshSampleKernel: 17 float4 per node = {4 child refs} + 4 x oriented box
+        const void*     wide;         // 4-wide collapse of the same tree for meshSampleKernel: one 128-byte record per node = {4 child refs} + 4 x oriented box (frame code, centre, extents; mesh_build.cuh)
         const void*     triVerts;     // 3 float4 per triangle SLOT (BVH order): a, b, c; .w of a = original triangle index (bits)
         const float*    pseudo;       // 21 floats per ORIGINAL triangle: face normal, 3 edge normals (AB, BC, CA), 3 vertex normals (A, B, C)
         uint32_t        nTris, nNodes;

@@ -136,7 +136,8 @@ extern "C"
         m->device = ctx->device; m->nTris = nT; m->nVerts = nV;
         auto align = [](size_t x) { return (x + 255) & ~(size_t)255; };
         const size_t bNodes = align((size_t)nNodes * sizeof(BvhNode)), bTv = align((size_t)nT * 48), bPs = align((size_t)nT * 84),
-                     bObb = align((size_t)nNodes * 64), bWide = align((size_t)nWide * 272);
+                     bObb = align((size_t)nNodes * 64), bWide = align((size_t)nWide * 128);
+        // every block starts on a 256-byte boundary of the blob: each 128-byte wide node is one cache line (mesh_build.cuh: meshWideKernel)
         // the ~200 MB of a large mesh come from the device's cache of released allocations (cudaMalloc + cudaFree of that size
         // cost 5-25 ms, more than the set-up kernels, when meshes are created and destroyed in a loop)
         m->ctx = ctx;

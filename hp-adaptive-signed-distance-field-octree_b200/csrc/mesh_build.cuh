@@ -333,8 +333,10 @@ namespace hpsdf
     }
 
     // Oriented boxes (see mesh.cpp of round 1 for the rationale): one warp per node with at most 32 768 triangles. Frame =
-    // area-weighted mean normal n and two tangents; half extents measured in exactly the float32 frame the traversal uses,
-    // inflated so that rounding can never cut a triangle off. Nodes whose normals disagree keep only their axis-aligned box.
+    // area-weighted mean normal n, encoded in 4 bytes and decoded again (decodeFrame), so that the binary walk (this array)
+    // and the wide walk (the code alone) use the same float32 frame; half extents measured in exactly that frame, inflated so
+    // that rounding can never cut a triangle off. o = {centre u, v, n, he u | u, he v | v, he n | n, frame code}. Nodes whose
+    // normals disagree keep only their axis-aligned box.
     __global__ void __launch_bounds__(256) meshObbKernel(const MeshBuildIn M, const BvhNode* __restrict__ nodes, const uint32_t* __restrict__ nodeBegin,
                                                          const uint32_t* __restrict__ nodeEnd, const uint32_t* __restrict__ order, uint32_t nNodes,
                                                          double inflate, float* __restrict__ obb)
@@ -365,15 +367,21 @@ namespace hpsdf
         const double len = sqrt(N[0] * N[0] + N[1] * N[1] + N[2] * N[2]);
         if (!(len > 0.5 * total) || !(len > 0.0)) return;
         const double nn[3] = { N[0] / len, N[1] / len, N[2] / len };
-        int ax = 0;
+        int ax = 0;                                              // tangents: the coordinate axis least aligned with n, made orthogonal
         if (fabs(nn[1]) < fabs(nn[ax])) ax = 1;
         if (fabs(nn[2]) < fabs(nn[ax])) ax = 2;
         double u[3] = { -nn[ax] * nn[0], -nn[ax] * nn[1], -nn[ax] * nn[2] };
         u[ax] += 1.0;
         const double ul = sqrt(u[0] * u[0] + u[1] * u[1] + u[2] * u[2]);
         for (int d = 0; d < 3; ++d) u[d] /= ul;
-        const double w[3] = { nn[1] * u[2] - nn[2] * u[1], nn[2] * u[0] - nn[0] * u[2], nn[0] * u[1] - nn[1] * u[0] };
-        const float fu[3] = { (float)u[0], (float)u[1], (float)u[2] }, fw[3] = { (float)w[0], (float)w[1], (float)w[2] }, fn[3] = { (float)nn[0], (float)nn[1], (float)nn[2] };
+        const double frame[3][3] = { { u[0], u[1], u[2] },
+                                     { nn[1] * u[2] - nn[2] * u[1], nn[2] * u[0] - nn[0] * u[2], nn[0] * u[1] - nn[1] * u[0] },
+                                     { nn[0], nn[1], nn[2] } };
+        // the frame the walks use is the one decoded from its 4-byte code (mesh_eval.cuh), and the extents are measured in it
+        const uint32_t code = encodeFrame(frame);
+        F3 du, dw, dn;
+        decodeFrame(code, du, dw, dn);
+        const float fu[3] = { du.x, du.y, du.z }, fw[3] = { dw.x, dw.y, dw.z }, fn[3] = { dn.x, dn.y, dn.z };
         double lo[3] = { 1e300, 1e300, 1e300 }, hi[3] = { -1e300, -1e300, -1e300 };
         for (uint32_t k = b + lane; k < e; k += 32u)
         {
@@ -406,7 +414,7 @@ namespace hpsdf
             }
             o[4] = fu[0]; o[5] = fu[1]; o[6] = fu[2];
             o[8] = fw[0]; o[9] = fw[1]; o[10] = fw[2];
-            o[12] = fn[0]; o[13] = fn[1]; o[14] = fn[2];
+            o[12] = fn[0]; o[13] = fn[1]; o[14] = fn[2]; o[15] = __uint_as_float(code);
         }
     }
 
@@ -427,14 +435,29 @@ namespace hpsdf
     }
 
     // 4-wide collapse for meshSampleKernel: a wide node holds the grandchildren of a binary node (or its children where they are
-    // leaves): 68 floats = 4 child references (kWideNone | leaf: 0x80000000 | count << 28 | first slot | wide index) + 4 x
-    // oriented box (nodes without one get their axis-aligned box in the same form).
+    // leaves) in one 128-byte record, one float4 per field with child k in component k:
+    //   { child reference (kNoNode | leaf: 0x80000000 | count << 28 | first slot | wide index) }, { frame code (decodeFrame) },
+    //   { centre u }, { centre v }, { centre n }, { half extent u }, { half extent v }, { half extent n }.
+    // Nodes without an oriented box get their axis-aligned box with the identity frame code.
+    constexpr int kWideFloats = 32;
+    __device__ __forceinline__ void putWideChild(float* __restrict__ out, int k, uint32_t ref, uint32_t code, const float* centre, const float* he)
+    {
+        out[k] = __uint_as_float(ref);
+        out[4 + k] = __uint_as_float(code);
+        for (int d = 0; d < 3; ++d) { out[8 + 4 * d + k] = centre[d]; out[20 + 4 * d + k] = he[d]; }
+    }
+    __device__ __forceinline__ void putAbsentChild(float* __restrict__ out, int k)
+    {
+        const float zero[3] = { 0.0f, 0.0f, 0.0f }, never[3] = { -3.0e38f, -3.0e38f, -3.0e38f };     // |q| - he overflows to +inf
+        putWideChild(out, k, 0xFFFFFFFFu, kIdentityFrame, zero, never);
+    }
+
     __global__ void __launch_bounds__(256) meshWideKernel(const BvhNode* __restrict__ nodes, const float* __restrict__ obb, const uint32_t* __restrict__ wideFlag,
                                                           const uint32_t* __restrict__ wideIdx, uint32_t nNodes, double inflate, float* __restrict__ wide)
     {
         const uint32_t b = blockIdx.x * blockDim.x + threadIdx.x;
         if (b >= nNodes || !wideFlag[b]) return;
-        float* out = wide + 68 * (size_t)wideIdx[b];
+        float* out = wide + kWideFloats * (size_t)wideIdx[b];
         uint32_t kids[4], nk = 0;
         const uint32_t two[2] = { nodes[b].a, nodes[b].b };
         for (int s = 0; s < 2; ++s)
@@ -445,43 +468,37 @@ namespace hpsdf
         }
         for (uint32_t k = 0; k < 4; ++k)
         {
-            uint32_t ref = 0xFFFFFFFFu;
-            float box[16];
-            for (int q = 0; q < 16; ++q) box[q] = 0.0f;
-            box[3] = box[7] = box[11] = -3.0e38f;                 // absent child: |q| - he overflows to +inf
-            if (k < nk)
+            if (k >= nk) { putAbsentChild(out, k); continue; }
+            const BvhNode c = nodes[kids[k]];
+            const float* o = obb + 16 * (size_t)kids[k];
+            const uint32_t ref = (c.b & 0x80000000u) ? (0x80000000u | ((c.b & 7u) << 28) | c.a) : wideIdx[kids[k]];
+            if (o[3] < 1e38f)
             {
-                const BvhNode c = nodes[kids[k]];
-                const float* o = obb + 16 * (size_t)kids[k];
-                if (o[3] < 1e38f) for (int q = 0; q < 16; ++q) box[q] = o[q];
-                else
-                {
-                    for (int d = 0; d < 3; ++d)
-                    {
-                        const double lo = c.mn[d], hi = c.mx[d];
-                        box[d] = (float)(0.5 * (lo + hi));
-                        const double ce = (double)box[d];
-                        box[3 + 4 * d] = nextafterf((float)(fmax(hi - ce, ce - lo) + inflate), 3.402823466e+38f);
-                    }
-                    box[4] = 1.0f; box[9] = 1.0f; box[14] = 1.0f;       // u = x, v = y, n = z
-                }
-                ref = (c.b & 0x80000000u) ? (0x80000000u | ((c.b & 7u) << 28) | c.a) : wideIdx[kids[k]];
+                const float centre[3] = { o[0], o[1], o[2] }, he[3] = { o[3], o[7], o[11] };
+                putWideChild(out, k, ref, __float_as_uint(o[15]), centre, he);
             }
-            out[k] = __uint_as_float(ref);
-            for (int q = 0; q < 16; ++q) out[4 + 16 * k + q] = box[q];
+            else
+            {
+                float centre[3], he[3];
+                for (int d = 0; d < 3; ++d)
+                {
+                    const double lo = c.mn[d], hi = c.mx[d];
+                    centre[d] = (float)(0.5 * (lo + hi));
+                    const double ce = (double)centre[d];
+                    he[d] = nextafterf((float)(fmax(hi - ce, ce - lo) + inflate), 3.402823466e+38f);
+                }
+                putWideChild(out, k, ref, kIdentityFrame, centre, he);        // u = x, v = y, n = z
+            }
         }
     }
 
-    // a mesh of at most 4 triangles is one leaf: the wide tree is a root with that single child
+    // a mesh of at most 4 triangles is one leaf: the wide tree is a root with that single child, whose box contains everything
     __global__ void meshWideSingleLeafKernel(const BvhNode* __restrict__ nodes, float* __restrict__ wide)
     {
         if (threadIdx.x != 0 || blockIdx.x != 0) return;
-        for (int q = 0; q < 68; ++q) wide[q] = 0.0f;
-        for (int k = 0; k < 4; ++k)
-        {
-            wide[k] = __uint_as_float(k ? 0xFFFFFFFFu : (0x80000000u | ((nodes[0].b & 7u) << 28) | nodes[0].a));
-            wide[4 + 16 * k + 3] = wide[4 + 16 * k + 7] = wide[4 + 16 * k + 11] = k ? -3.0e38f : 3.0e38f;
-        }
+        const float zero[3] = { 0.0f, 0.0f, 0.0f }, all[3] = { 3.0e38f, 3.0e38f, 3.0e38f };
+        putWideChild(wide, 0, 0x80000000u | ((nodes[0].b & 7u) << 28) | nodes[0].a, kIdentityFrame, zero, all);
+        for (int k = 1; k < 4; ++k) putAbsentChild(wide, k);
     }
 
     // triangle vertices in BVH order: 3 float4 per slot, the original triangle index rides in a.w

@@ -15,8 +15,11 @@
 //     bound against the lane's current best first;
 //   * a lane that finishes its query writes the sample and takes the next one (warps grab 32-128 samples at a time from a
 //     global counter), so lanes do not wait for their neighbours and far / near cells balance across the grid;
-//   * the tree is walked in its 4-wide collapse (mesh.cpp: collapseWide), one 272-byte record and one memory round trip per
-//     step: the walk is latency-bound, and leaf sizes 1 / 2 / 4 / 7 measured 98 / 90 / 83 / 80 ms — node steps are the cost.
+//   * the tree is walked in its 4-wide collapse (mesh_build.cuh: meshWideKernel), one 128-byte record (one cache line: four
+//     child references, four 4-byte frame codes, four oriented boxes in f32) per node step, read as 8 float4; the frames are
+//     decoded in registers (mesh_eval.cuh: decodeFrame). The walk is bound by L1 throughput and latency, and leaf sizes
+//     1 / 2 / 4 / 7 measured 98 / 90 / 83 / 80 ms — node steps are the cost;
+//   * a stack entry is (node, bound) in 8 bytes: one local-memory access per push or pop;
 //   * when the samples run out, lanes without work take sub-trees from lanes that still have a stack (tail phase below);
 // Results are those of meshSignedDistanceF: same exact test, same (smallest f32 d2, lowest triangle index) winner, same
 // conservative pruning — the order in which candidates are met does not matter to that rule.
@@ -30,6 +33,11 @@ namespace hpsdf
     constexpr int      kMeshStack = 48;         // >= 3 pushes x 14 levels: the 4-wide tree of the largest accepted mesh (2^28 triangles, median split)
     constexpr uint32_t kNoNode    = 0xFFFFFFFFu;
 
+    __device__ __forceinline__ unsigned long long stackEntry(uint32_t node, float bound)
+    {
+        return (unsigned long long)node | ((unsigned long long)__float_as_uint(bound) << 32);
+    }
+
     __global__ void __launch_bounds__(256, 4)
     meshSampleKernel(const FitTask* __restrict__ tasks, unsigned long long nSamples, int D, const DeviceMeshView* __restrict__ mesh,
                      const RootMap map, const FitTablesDev tab, double* __restrict__ samples, unsigned long long* __restrict__ counter,
@@ -37,7 +45,7 @@ namespace hpsdf
                      const int handOver,                            // 1 = tail phase on (0: diagnostics, HPSDF_MESH_NO_HANDOVER)
                      unsigned long long* __restrict__ stats)        // diagnostics (HPSDF_MESH_STATS): histogram of node steps per query, or nullptr
     {
-        const float4* __restrict__ wide = (const float4*)mesh->wide;           // 17 float4 per 4-wide node: {child refs}, 4 x oriented box
+        const float4* __restrict__ wide = (const float4*)mesh->wide;           // 8 float4 per 4-wide node (meshWideKernel)
         const float4* __restrict__ tv = (const float4*)mesh->triVerts;
         const double* __restrict__ roots = tab.roots[D];
         const unsigned n = (unsigned)fitRule(D), n2 = n * n, n3 = n2 * n;
@@ -47,7 +55,7 @@ namespace hpsdf
         long long sid = -1;                       // sample index, -1 = idle
         F3 p = f3(0.0f, 0.0f, 0.0f);
         MeshHit h;
-        uint32_t stackN[kMeshStack]; float stackD[kMeshStack];
+        unsigned long long stack[kMeshStack];             // node | bound bits << 32
         int sp = 0;
         uint32_t cur = kNoNode; float curD = 0.0f;       // wide node (or leaf reference, bit 31) to process and its bound
         uint32_t qLeaf[kMeshQueue]; float qD[kMeshQueue];        // circular: head qh, count qn; entry = leaf reference
@@ -62,7 +70,7 @@ namespace hpsdf
         // kernel's stall samples on its dependent local-memory loads.
         auto pop = [&]()
         {
-            if (sp > 0) { --sp; cur = stackN[sp]; curD = stackD[sp]; }
+            if (sp > 0) { --sp; const unsigned long long e = stack[sp]; cur = (uint32_t)e; curD = __uint_as_float((uint32_t)(e >> 32)); }
             else cur = kNoNode;
         };
 
@@ -90,18 +98,21 @@ namespace hpsdf
                     }
                     else
                     {
-                        // one round trip per step: the four child references and their oriented boxes sit in one 272-byte record
-                        // (the walk is latency-bound: ncu showed 10 cycles of long-scoreboard stall per issued instruction)
-                        const float4* __restrict__ w = wide + 17 * (size_t)cur;
-                        const float4 hdr = __ldg(w);
+                        // one cache line per step: the four child references, frame codes and boxes of the node, all requested at once
+                        const float4* __restrict__ w = wide + 8 * (size_t)cur;
+                        const float4 hdr = __ldg(w), code = __ldg(w + 1), cu = __ldg(w + 2), cv = __ldg(w + 3), cn = __ldg(w + 4),
+                                     hu = __ldg(w + 5), hv = __ldg(w + 6), hn = __ldg(w + 7);
                         const uint32_t ref[4] = { __float_as_uint(hdr.x), __float_as_uint(hdr.y), __float_as_uint(hdr.z), __float_as_uint(hdr.w) };
                         const float lim = bound * 1.000001f;
                         float cd[4];
                         #pragma unroll
                         for (int k = 0; k < 4; ++k)
                         {
-                            const float4 o0 = __ldg(w + 1 + 4 * k), o1 = __ldg(w + 2 + 4 * k), o2 = __ldg(w + 3 + 4 * k), o3 = __ldg(w + 4 + 4 * k);
-                            const float d = obbDist2(o0, o1, o2, o3, p);
+                            const auto at = [k](const float4& q) { return k == 0 ? q.x : k == 1 ? q.y : k == 2 ? q.z : q.w; };
+                            F3 u, v, nrm;
+                            decodeFrame(__float_as_uint(at(code)), u, v, nrm);
+                            const float d = obbDist2(make_float4(at(cu), at(cv), at(cn), at(hu)), make_float4(u.x, u.y, u.z, at(hv)),
+                                                     make_float4(v.x, v.y, v.z, at(hn)), make_float4(nrm.x, nrm.y, nrm.z, 0.0f), p);
                             cd[k] = (ref[k] != kNoNode && d <= lim) ? d : 3.402823466e+38f;          // FLT_MAX = "do not visit" (lim < FLT_MAX once a triangle was seen; before that every real child passes)
                         }
                         // visit order: nearest first; the others go on the stack farthest first so that the nearest of them is popped next
@@ -111,9 +122,9 @@ namespace hpsdf
                         HPSDF_CSWAP(d0, r0, d1, r1) HPSDF_CSWAP(d2, r2, d3, r3) HPSDF_CSWAP(d0, r0, d2, r2) HPSDF_CSWAP(d1, r1, d3, r3) HPSDF_CSWAP(d1, r1, d2, r2)
                         #undef HPSDF_CSWAP
                         const bool v0 = d0 < 3.0e38f;
-                        if (d3 < 3.0e38f && sp < kMeshStack) { stackN[sp] = r3; stackD[sp] = d3; ++sp; }
-                        if (d2 < 3.0e38f && sp < kMeshStack) { stackN[sp] = r2; stackD[sp] = d2; ++sp; }
-                        if (d1 < 3.0e38f && sp < kMeshStack) { stackN[sp] = r1; stackD[sp] = d1; ++sp; }
+                        if (d3 < 3.0e38f && sp < kMeshStack) stack[sp++] = stackEntry(r3, d3);
+                        if (d2 < 3.0e38f && sp < kMeshStack) stack[sp++] = stackEntry(r2, d2);
+                        if (d1 < 3.0e38f && sp < kMeshStack) stack[sp++] = stackEntry(r1, d1);
                         if (v0) { cur = r0; curD = d0; }
                         else pop();
                     }
@@ -254,7 +265,7 @@ namespace hpsdf
                     const bool give = canGive && (int)__popc(donors & ltMask) < nPairs;
                     const int src = take ? (int)__fns(donors, 0u, __popc(idle & ltMask) + 1) : (int)lane;
                     uint32_t gN = kNoNode; float gD = 0.0f;
-                    if (give) { --sp; gN = stackN[sp]; gD = stackD[sp]; ++helpers; }
+                    if (give) { --sp; const unsigned long long e = stack[sp]; gN = (uint32_t)e; gD = __uint_as_float((uint32_t)(e >> 32)); ++helpers; }
                     const uint32_t tN = __shfl_sync(0xFFFFFFFFu, gN, src);
                     const float tD = __shfl_sync(0xFFFFFFFFu, gD, src);
                     const int tRoot = __shfl_sync(0xFFFFFFFFu, root, src);
