@@ -44,8 +44,8 @@ namespace hpsdf
         }
     }
 
-    // HPSDF_MESH_STATS=1: a 64-word device buffer collecting the node-step histogram of meshSampleKernel (printed by
-    // hpsdf_debug_mesh_stats); nullptr otherwise.
+    // HPSDF_MESH_STATS=1: a 64-word device buffer collecting the node-step histogram of meshSampleKernel (words 0-41) and
+    // its event counts (words 42.., mesh_sample_kernel.cuh: MeshStat), printed by hpsdf_debug_mesh_stats; nullptr otherwise.
     static unsigned long long* g_meshStats[16] = { nullptr };
     static unsigned long long* meshStatsBuffer()
     {
@@ -73,6 +73,15 @@ namespace hpsdf
         fprintf(stderr, "meshSampleKernel: %llu queries, mean %.1f node steps, max %llu; queries by steps:", n, n ? (double)h[40] / n : 0.0, h[41]);
         for (int b = 0; b < 40; ++b) if (h[b]) fprintf(stderr, " <%llu: %llu", 1ull << b, h[b]);
         fprintf(stderr, "\n");
+        // the event counts include the work of tail-phase helpers, which the histogram above leaves out
+        const unsigned long long* c = h + kMeshStatWord;
+        const double q = n ? (double)n : 1.0;
+        fprintf(stderr, "meshSampleKernel per query: %.2f node steps = %.2f node visits + %.2f stale pops (%.2f more entries dropped with them); "
+                        "%.2f leaves tested, %.2f dequeued already pruned; %.1f lanes per node iteration, %.1f per triangle iteration\n",
+                (c[kStatNodeVisit] + c[kStatStalePop]) / q, c[kStatNodeVisit] / q, c[kStatStalePop] / q, c[kStatGroupDrop] / q,
+                c[kStatLeafTest] / q, c[kStatLeafPruned] / q,
+                c[kStatWarpNodeIter] ? (double)(c[kStatNodeVisit] + c[kStatStalePop]) / c[kStatWarpNodeIter] : 0.0,
+                c[kStatWarpTriIter] ? (double)(c[kStatLeafTest] + c[kStatLeafPruned]) / c[kStatWarpTriIter] : 0.0);
     }
 
     // HPSDF_DEBUG_ROUNDS=3: events around the sample and fit kernels of every degree group (diagnostics only)
@@ -145,9 +154,13 @@ namespace hpsdf
                     if (e != cudaSuccess) return e;
                     // 4 CTAs of 256 per SM (64 registers) and "test triangles once 12 lanes have one waiting" measured best on
                     // B200 (870 k-triangle mesh, binary tree: 2 CTAs/24 lanes 113 ms, 3/24 101 ms, 4/24 95 ms, 4/12 88 ms, 4/4 95 ms;
-                    // 4-wide tree: 8 or 12 lanes 62.8 ms, 16 63.9, 20 66.3, 24 70.5)
-                    meshSampleKernel<<<(unsigned)std::min(want, sms * 4), 256, 0, stream>>>(dTasks + b, total, D, (const DeviceMeshView*)prog.instr[0].handle,
-                                                                                          map, tab, samples, counter, grab, 12, getenv("HPSDF_MESH_NO_HANDOVER") ? 0 : 1, meshStatsBuffer());
+                    // 4-wide tree: 8 or 12 lanes 62.8 ms, 16 63.9, 20 66.3, 24 70.5). With leaves queued straight from the node step
+                    // into an 8-entry queue, 16 lanes measured best on C3: 8 / 12 / 16 / 20 lanes 54.7 / 50.7 / 49.1 / 49.2 ms.
+                    constexpr int triThreshold = 16;
+                    unsigned long long* stats = meshStatsBuffer();
+                    const size_t statSmem = stats ? (size_t)kMeshStatCount * 256 * sizeof(unsigned) : 0;
+                    meshSampleKernel<<<(unsigned)std::min(want, sms * 4), 256, statSmem, stream>>>(dTasks + b, total, D, (const DeviceMeshView*)prog.instr[0].handle,
+                                                                                                 map, tab, samples, counter, grab, triThreshold, getenv("HPSDF_MESH_NO_HANDOVER") ? 0 : 1, stats);
                 }
                 else
                 {

@@ -124,6 +124,8 @@ extern "C"
         const uint32_t nNodes = shape.nodes(nT), levels = shape.levels(nT), nWide = std::max(1u, shape.wideNodes(nT, 0));
         // traversal stacks (mesh_eval.cuh, mesh_sample_kernel.cuh) hold 48 entries: one push per binary level, three per 4-wide level
         if (levels > 47u || 3u * ((levels + 1u) / 2u) > 48u) { setLastError("mesh too deep for the traversal stacks"); return HPSDF_ERR_UNSUPPORTED; }
+        // meshSampleKernel keeps a wide-node index in bits 0-27 of a stack entry and a group count in bits 28-29
+        if (nWide >= (1u << 28)) { setLastError("too many 4-wide BVH nodes for the traversal stack entries"); return HPSDF_ERR_UNSUPPORTED; }
         BvhCountTable counts;
         memset(&counts, 0, sizeof(counts));
         for (const auto& kv : shape.count)

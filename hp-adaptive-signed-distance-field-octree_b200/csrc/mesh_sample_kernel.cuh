@@ -10,16 +10,20 @@
 // Here the warp is a scheduler over 32 independent query state machines:
 //   * every loop iteration is EITHER a node step OR a triangle test for all lanes that have one pending — the choice is
 //     warp-uniform (ballots), so the two instruction streams are never serialised against each other;
-//   * reaching a leaf does not test it: the leaf goes into a 4-entry per-lane queue and the lane keeps walking; triangle
-//     iterations run when at least `triThreshold` (12) lanes have a triangle waiting (or nobody has a node left), re-checking the leaf's
-//     bound against the lane's current best first;
+//   * reaching a leaf does not test it: a node step puts the leaf children that pass the bound straight into an 8-entry
+//     per-lane queue (nearest first, in shared memory) and the lane keeps walking; only inner children become the next node
+//     or go on the stack, so every node step that is not a stale pop reads a node. Triangle iterations run when at least
+//     `triThreshold` (16) lanes have a triangle waiting (or nobody has a node left), re-checking the leaf's bound against the
+//     lane's current best first;
 //   * a lane that finishes its query writes the sample and takes the next one (warps grab 32-128 samples at a time from a
 //     global counter), so lanes do not wait for their neighbours and far / near cells balance across the grid;
 //   * the tree is walked in its 4-wide collapse (mesh_build.cuh: meshWideKernel), one 128-byte record (one cache line: four
 //     child references, four 4-byte frame codes, four oriented boxes in f32) per node step, read as 8 float4; the frames are
 //     decoded in registers (mesh_eval.cuh: decodeFrame). The walk is bound by L1 throughput and latency, and leaf sizes
 //     1 / 2 / 4 / 7 measured 98 / 90 / 83 / 80 ms — node steps are the cost;
-//   * a stack entry is (node, bound) in 8 bytes: one local-memory access per push or pop;
+//   * a stack entry is (node, bound) in 8 bytes: one local-memory access per push or pop; it also records how many entries
+//     below it came from the same node step. Those are its farther siblings, so once its bound is stale theirs are too, and
+//     a stale pop drops them without a step of their own;
 //   * when the samples run out, lanes without work take sub-trees from lanes that still have a stack (tail phase below);
 // Results are those of meshSignedDistanceF: same exact test, same (smallest f32 d2, lowest triangle index) winner, same
 // conservative pruning — the order in which candidates are met does not matter to that rule.
@@ -29,9 +33,18 @@
 
 namespace hpsdf
 {
-    constexpr int      kMeshQueue = 4;
+    constexpr int      kMeshQueue = 8;          // a node step needs room for 4 leaves, so up to 4 earlier ones can wait and the queue never overflows (power of 2: ring index)
     constexpr int      kMeshStack = 48;         // >= 3 pushes x 14 levels: the 4-wide tree of the largest accepted mesh (2^28 triangles, median split)
     constexpr uint32_t kNoNode    = 0xFFFFFFFFu;
+    // A stack entry and `cur` hold the wide-node index in bits 0-27 and, in bits 28-29, how many entries directly below it on
+    // the stack were pushed by the same node step (0-3). Those bits are free: the builder rejects meshes with 2^28 or more
+    // wide nodes (mesh.cpp), and leaf references (bit 31) go to the leaf queue, never on the stack.
+    constexpr uint32_t kNodeIndexMask = 0x0FFFFFFFu;
+    constexpr int      kGroupShift    = 28;
+    // HPSDF_MESH_STATS: per-thread event counters in dynamic shared memory, [counter][threadIdx], added to words 42.. of
+    // the stats buffer when the block ends (fit_kernels.cuh: printMeshStats)
+    enum MeshStat { kStatNodeVisit, kStatStalePop, kStatGroupDrop, kStatLeafTest, kStatLeafPruned, kStatWarpNodeIter, kStatWarpTriIter, kMeshStatCount };
+    constexpr int kMeshStatWord = 42;
 
     __device__ __forceinline__ unsigned long long stackEntry(uint32_t node, float bound)
     {
@@ -43,8 +56,12 @@ namespace hpsdf
                      const RootMap map, const FitTablesDev tab, double* __restrict__ samples, unsigned long long* __restrict__ counter,
                      const unsigned grab, const int triThreshold,   // (triThreshold: see launchOne)
                      const int handOver,                            // 1 = tail phase on (0: diagnostics, HPSDF_MESH_NO_HANDOVER)
-                     unsigned long long* __restrict__ stats)        // diagnostics (HPSDF_MESH_STATS): histogram of node steps per query, or nullptr
+                     unsigned long long* __restrict__ stats)        // diagnostics (HPSDF_MESH_STATS): histogram of node steps per query and event
+                                                                    // counts (kMeshStatCount x blockDim.x words of dynamic shared memory), or nullptr
     {
+        // the leaf queues of the block, [slot][thread]: conflict-free, and out of the local memory that holds the stacks
+        __shared__ unsigned long long sQueue[kMeshQueue][256];
+        extern __shared__ unsigned sStat[];
         const float4* __restrict__ wide = (const float4*)mesh->wide;           // 8 float4 per 4-wide node (meshWideKernel)
         const float4* __restrict__ tv = (const float4*)mesh->triVerts;
         const double* __restrict__ roots = tab.roots[D];
@@ -55,19 +72,26 @@ namespace hpsdf
         long long sid = -1;                       // sample index, -1 = idle
         F3 p = f3(0.0f, 0.0f, 0.0f);
         MeshHit h;
-        unsigned long long stack[kMeshStack];             // node | bound bits << 32
+        unsigned long long stack[kMeshStack];             // node | group << 28 | bound bits << 32
         int sp = 0;
-        uint32_t cur = kNoNode; float curD = 0.0f;       // wide node (or leaf reference, bit 31) to process and its bound
-        uint32_t qLeaf[kMeshQueue]; float qD[kMeshQueue];        // circular: head qh, count qn; entry = leaf reference
+        uint32_t cur = kNoNode; float curD = 0.0f;       // wide node (| group << 28) to process and its bound
+        unsigned long long* const queue = &sQueue[0][threadIdx.x];  // circular, slot s at queue[s * 256]: head qh, count qn; entry = leaf reference | bound bits << 32
         int qh = 0, qn = 0;
         unsigned steps = 0;                                      // node steps of the lane's current query
         // warp-uniform work cursor
         unsigned long long cursor = 0, grabEnd = 0;
         bool exhausted = false;
 
+        auto count = [&](const MeshStat c) { if (stats) ++sStat[c * blockDim.x + threadIdx.x]; };
+        if (stats) for (int c = 0; c < kMeshStatCount; ++c) sStat[c * blockDim.x + threadIdx.x] = 0u;
+        auto flushStats = [&]()
+        {
+            if (stats) for (int c = 0; c < kMeshStatCount; ++c) atomicAdd(stats + kMeshStatWord + c, (unsigned long long)sStat[c * blockDim.x + threadIdx.x]);
+        };
+
         // One entry per call: a stale entry (its bound no longer beats the lane's best) is recognised by the next node step,
-        // which then pops again — a divergent "skip the stale ones" loop here ran with 2-4 active lanes and drew 29 % of the
-        // kernel's stall samples on its dependent local-memory loads.
+        // which drops it with its group and pops again — a divergent "skip the stale ones" loop here ran with 2-4 active lanes
+        // and drew 29 % of the kernel's stall samples on its dependent local-memory loads.
         auto pop = [&]()
         {
             if (sp > 0) { --sp; const unsigned long long e = stack[sp]; cur = (uint32_t)e; curD = __uint_as_float((uint32_t)(e >> 32)); }
@@ -79,31 +103,35 @@ namespace hpsdf
         // farther than which can win (the lane's own best; in the tail phase the best of all lanes working on the same sample).
         auto step = [&](const bool active, const float bound)
         {
-            const bool wantNode = active && cur != kNoNode && qn < kMeshQueue;
+            const bool wantNode = active && cur != kNoNode && qn <= kMeshQueue - 4;      // room for all four children being leaves
             const unsigned nodeMask = __ballot_sync(0xFFFFFFFFu, wantNode);
             const unsigned triMask = __ballot_sync(0xFFFFFFFFu, qn > 0);
+            if (lane == 0 && (nodeMask == 0u || __popc(triMask) >= triThreshold) && triMask != 0u) count(kStatWarpTriIter);
             if (nodeMask != 0u && __popc(triMask) < triThreshold)
             {
+                if (lane == 0) count(kStatWarpNodeIter);
                 if (wantNode)
                 {
                     ++steps;
-                    if (curD > bound * 1.000001f) pop();                         // went stale on the stack
-                    else if (cur & 0x80000000u)
+                    const float lim = bound * 1.000001f;
+                    if (curD > lim)
                     {
-                        const int slot = (qh + qn) & (kMeshQueue - 1);
-                        qLeaf[slot] = cur;                                       // 0x80000000 | count << 28 | first triangle slot
-                        qD[slot] = curD;
-                        ++qn;
+                        // went stale on the stack; so did the entries below it from the same node step (its farther siblings):
+                        // drop them with it, no loads
+                        const int group = (int)(cur >> kGroupShift);
+                        sp -= group;
+                        count(kStatStalePop);
+                        if (stats) sStat[kStatGroupDrop * blockDim.x + threadIdx.x] += (unsigned)group;
                         pop();
                     }
                     else
                     {
+                        count(kStatNodeVisit);
                         // one cache line per step: the four child references, frame codes and boxes of the node, all requested at once
-                        const float4* __restrict__ w = wide + 8 * (size_t)cur;
+                        const float4* __restrict__ w = wide + 8 * (size_t)(cur & kNodeIndexMask);
                         const float4 hdr = __ldg(w), code = __ldg(w + 1), cu = __ldg(w + 2), cv = __ldg(w + 3), cn = __ldg(w + 4),
                                      hu = __ldg(w + 5), hv = __ldg(w + 6), hn = __ldg(w + 7);
                         const uint32_t ref[4] = { __float_as_uint(hdr.x), __float_as_uint(hdr.y), __float_as_uint(hdr.z), __float_as_uint(hdr.w) };
-                        const float lim = bound * 1.000001f;
                         float cd[4];
                         #pragma unroll
                         for (int k = 0; k < 4; ++k)
@@ -115,27 +143,42 @@ namespace hpsdf
                                                      make_float4(v.x, v.y, v.z, at(hn)), make_float4(nrm.x, nrm.y, nrm.z, 0.0f), p);
                             cd[k] = (ref[k] != kNoNode && d <= lim) ? d : 3.402823466e+38f;          // FLT_MAX = "do not visit" (lim < FLT_MAX once a triangle was seen; before that every real child passes)
                         }
-                        // visit order: nearest first; the others go on the stack farthest first so that the nearest of them is popped next
-                        uint32_t r0 = ref[0], r1 = ref[1], r2 = ref[2], r3 = ref[3];
-                        float d0 = cd[0], d1 = cd[1], d2 = cd[2], d3 = cd[3];
-                        #define HPSDF_CSWAP(da, ra, db, rb) if (db < da) { const float td = da; da = db; db = td; const uint32_t tr = ra; ra = rb; rb = tr; }
-                        HPSDF_CSWAP(d0, r0, d1, r1) HPSDF_CSWAP(d2, r2, d3, r3) HPSDF_CSWAP(d0, r0, d2, r2) HPSDF_CSWAP(d1, r1, d3, r3) HPSDF_CSWAP(d1, r1, d2, r2)
+                        // visit order: nearest first
+                        uint32_t r[4] = { ref[0], ref[1], ref[2], ref[3] };
+                        #define HPSDF_CSWAP(a, b) if (cd[b] < cd[a]) { const float td = cd[a]; cd[a] = cd[b]; cd[b] = td; const uint32_t tr = r[a]; r[a] = r[b]; r[b] = tr; }
+                        HPSDF_CSWAP(0, 1) HPSDF_CSWAP(2, 3) HPSDF_CSWAP(0, 2) HPSDF_CSWAP(1, 3) HPSDF_CSWAP(1, 2)
                         #undef HPSDF_CSWAP
-                        const bool v0 = d0 < 3.0e38f;
-                        if (d3 < 3.0e38f && sp < kMeshStack) stack[sp++] = stackEntry(r3, d3);
-                        if (d2 < 3.0e38f && sp < kMeshStack) stack[sp++] = stackEntry(r2, d2);
-                        if (d1 < 3.0e38f && sp < kMeshStack) stack[sp++] = stackEntry(r1, d1);
-                        if (v0) { cur = r0; curD = d0; }
+                        // leaves go straight to the queue, nearest first (wantNode left room for four)
+                        #pragma unroll
+                        for (int k = 0; k < 4; ++k)
+                            if (cd[k] < 3.0e38f && (r[k] & 0x80000000u))
+                            {
+                                queue[((qh + qn) & (kMeshQueue - 1)) * 256] = stackEntry(r[k], cd[k]);   // 0x80000000 | count << 28 | first triangle slot
+                                ++qn;
+                            }
+                        // inner children: the nearest becomes cur, the others go on the stack farthest first so that the nearest of
+                        // them is popped next; each records how many of its farther siblings lie below it
+                        uint32_t next = kNoNode, group = 0u;
+                        float nextD = 0.0f;
+                        #pragma unroll
+                        for (int k = 3; k >= 0; --k)
+                            if (cd[k] < 3.0e38f && !(r[k] & 0x80000000u))
+                            {
+                                if (next != kNoNode && sp < kMeshStack) { stack[sp++] = stackEntry(next | group << kGroupShift, nextD); ++group; }
+                                next = r[k]; nextD = cd[k];
+                            }
+                        if (next != kNoNode) { cur = next | group << kGroupShift; curD = nextD; }
                         else pop();
                     }
                 }
             }
             else if (qn > 0)
             {
-                const uint32_t e = qLeaf[qh];
-                const uint32_t first = e & 0x0FFFFFFFu, cnt = (e >> 28) & 7u;
-                if (qD[qh] <= bound * 1.000001f)                               // else: pruned while it waited
+                const unsigned long long e = queue[qh * 256];
+                const uint32_t first = (uint32_t)e & 0x0FFFFFFFu, cnt = ((uint32_t)e >> 28) & 7u;
+                if (__uint_as_float((uint32_t)(e >> 32)) <= bound * 1.000001f)    // else: pruned while it waited
                 {
+                    count(kStatLeafTest);
                     // the whole leaf in one iteration (3-4 triangles): the scheduler's ballots are paid once per leaf
                     #pragma unroll 1
                     for (uint32_t t = 0; t < cnt; ++t)
@@ -149,8 +192,19 @@ namespace hpsdf
                         if (d2 < h.best || (d2 == h.best && tri < h.tri)) { h.best = d2; h.tri = tri; h.simplex = s; h.id = id; h.pt = cp; }
                     }
                 }
+                else count(kStatLeafPruned);
                 qh = (qh + 1) & (kMeshQueue - 1);
                 --qn;
+                // leaves the new best has pruned leave the queue now (shared-memory reads only), so that they neither take a
+                // triangle iteration of their own nor count towards triThreshold. h.best is a distance this lane reached for
+                // the same point, so it bounds the answer in the tail phase too.
+                const float after = fminf(bound, h.best) * 1.000001f;
+                while (qn > 0 && __uint_as_float((uint32_t)(queue[qh * 256] >> 32)) > after)
+                {
+                    count(kStatLeafPruned);
+                    qh = (qh + 1) & (kMeshQueue - 1);
+                    --qn;
+                }
             }
         };
 
@@ -204,7 +258,7 @@ namespace hpsdf
                 cursor += want < avail ? want : avail;
                 idle = __ballot_sync(0xFFFFFFFFu, sid < 0);
             }
-            if (idle == 0xFFFFFFFFu) return;                                  // nothing in flight and nothing left to take
+            if (idle == 0xFFFFFFFFu) { flushStats(); return; }                // nothing in flight and nothing left to take
             if (idle && handOver) break;                                      // no samples left and some lanes have nothing to do: tail phase
             step(true, h.best);
         }
@@ -251,11 +305,12 @@ namespace hpsdf
             }
             if (sid >= 0 && cur == kNoNode && qn == 0 && helpers == 0) retire();
             const unsigned idle = __ballot_sync(0xFFFFFFFFu, sid < 0 && owner < 0);
-            if (idle == 0xFFFFFFFFu) return;
+            if (idle == 0xFFFFFFFFu) { flushStats(); return; }
             if (idle)
             {
                 // the i-th lane without work takes the top stack entry of the i-th lane that has one to spare (only from lanes that
-                // have seen a triangle: before that nothing can be pruned and a helper would walk its whole sub-tree)
+                // have seen a triangle: before that nothing can be pruned and a helper would walk its whole sub-tree); queued
+                // leaves are not handed over
                 const bool canGive = (sid >= 0 || owner >= 0) && sp > 0 && cur != kNoNode && h.best < 3.0e38f;
                 const unsigned donors = __ballot_sync(0xFFFFFFFFu, canGive);
                 if (donors)
@@ -265,7 +320,12 @@ namespace hpsdf
                     const bool give = canGive && (int)__popc(donors & ltMask) < nPairs;
                     const int src = take ? (int)__fns(donors, 0u, __popc(idle & ltMask) + 1) : (int)lane;
                     uint32_t gN = kNoNode; float gD = 0.0f;
-                    if (give) { --sp; const unsigned long long e = stack[sp]; gN = (uint32_t)e; gD = __uint_as_float((uint32_t)(e >> 32)); ++helpers; }
+                    if (give)
+                    {
+                        --sp; const unsigned long long e = stack[sp]; gN = (uint32_t)e & kNodeIndexMask; gD = __uint_as_float((uint32_t)(e >> 32)); ++helpers;
+                        // the helper's stack starts empty (gN without group); if the entry was one of cur's siblings, cur's group lost it
+                        if (cur >> kGroupShift) cur -= 1u << kGroupShift;
+                    }
                     const uint32_t tN = __shfl_sync(0xFFFFFFFFu, gN, src);
                     const float tD = __shfl_sync(0xFFFFFFFFu, gD, src);
                     const int tRoot = __shfl_sync(0xFFFFFFFFu, root, src);
