@@ -127,7 +127,7 @@ EXPORTS = [
     "hpsdf_get_root_aabb", "hpsdf_destroy", "hpsdf_get_build_stats", "hpsdf_get_decision_log", "hpsdf_get_apply_log", "hpsdf_fit_batch",
     "hpsdf_bench_frontier", "hpsdf_measure_fp64_peak", "hpsdf_comm_get_unique_id", "hpsdf_comm_init",
     "hpsdf_comm_destroy", "hpsdf_shard_range", "hpsdf_set_jit", "hpsdf_jit_compile_check", "hpsdf_query_ray",
-    "hpsdf_get_config", "hpsdf_get_device", "hpsdf_uniform_points_device",
+    "hpsdf_get_config", "hpsdf_get_device", "hpsdf_uniform_points_device", "hpsdf_extract_isosurface",
 ]
 
 _lib = None
@@ -169,6 +169,7 @@ def lib():
     L.hpsdf_query_device.argtypes = [vp, vp, sz, vp, vp]
     L.hpsdf_query_with_gradient.argtypes = [vp, vp, sz, vp, vp]
     L.hpsdf_query_ray.argtypes = [vp, vp, vp, sz, dbl, vp, vp]
+    L.hpsdf_extract_isosurface.argtypes = [vp, vp, vp, vp, dbl, C.POINTER(sz), C.POINTER(vp), C.POINTER(sz), C.POINTER(vp)]
     L.hpsdf_to_memory_block.argtypes = [vp, C.POINTER(sz), C.POINTER(vp)]
     L.hpsdf_from_memory_block.argtypes = [vp, sz, i32, C.POINTER(vp)]
     L.hpsdf_clone.argtypes = [vp, C.POINTER(vp)]
@@ -397,6 +398,28 @@ class Octree:
                 for i in range(n - 1, -1, -1):                      # BMP rows are stored bottom-up; channels as B, G, R
                     f.write(img[i, :, ::-1].tobytes() + pad)
         return vals, img
+
+    def ExtractIsosurface(self, resolution, iso=0.0, box=None):
+        """The level set F = iso as a triangle mesh (hpsdf_extract_isosurface): marching tetrahedra over a uniform grid of
+        `resolution` cells per axis (an int or 3 ints, each 1..1024) spanning box = (min xyz, max xyz), or the root box.
+        Returns (vertices (n,3) float32, triangles (m,3) uint32), counter-clockwise seen from the side where F >= iso; closed
+        when the surface stays inside the box. hp.Mesh(vertices, triangles) takes it as it is."""
+        res = [int(resolution)] * 3 if np.ndim(resolution) == 0 else [int(r) for r in resolution]
+        if len(res) != 3 or not all(0 <= r <= 0xFFFFFFFF for r in res):
+            raise HpsdfError(ERR_INVALID_ARG, "resolution must be one or three counts in [1, 1024]")
+        lo = hi = None
+        if box is not None:
+            lo, hi = ((C.c_double * 3)(*[float(x) for x in b]) for b in box)
+        nv, nt, pv, pt = C.c_size_t(), C.c_size_t(), C.c_void_p(), C.c_void_p()
+        _check(lib().hpsdf_extract_isosurface(self._h, (C.c_uint32 * 3)(*res), lo, hi, float(iso), C.byref(nv), C.byref(pv),
+                                              C.byref(nt), C.byref(pt)))
+        try:
+            v = np.ctypeslib.as_array((C.c_float * (3 * nv.value)).from_address(pv.value)).reshape(-1, 3).copy() if nv.value else np.empty((0, 3), np.float32)
+            t = np.ctypeslib.as_array((C.c_uint32 * (3 * nt.value)).from_address(pt.value)).reshape(-1, 3).copy() if nt.value else np.empty((0, 3), np.uint32)
+        finally:
+            MemoryBlock._libc.free(pv)
+            MemoryBlock._libc.free(pt)
+        return v, t
 
     # -- serialisation (Octree.cpp:403-456) ----------------------------------------------------------------------------
     def ToMemoryBlock(self):

@@ -1,5 +1,6 @@
 // capi.cpp — the extern "C" surface declared in include/hpsdf.h.
 #include <cmath>
+#include <cstdio>
 #include <cstdlib>
 #include <cstring>
 #include <mutex>
@@ -203,6 +204,91 @@ extern "C"
         if (e == cudaSuccess) e = cudaMemcpy(t, dT, n * 8, cudaMemcpyDeviceToHost);
         cudaFree(dO); cudaFree(dD); cudaFree(dT); cudaFree(dH);
         if (e != cudaSuccess) return failCuda(e, "hpsdf_query_ray");
+        return HPSDF_OK;
+    }
+
+    HPSDF_API hpsdf_status hpsdf_extract_isosurface(const hpsdf_octree* tree, const uint32_t resolution[3], const double box_min[3],
+                                                    const double box_max[3], double iso, size_t* n_vertices, float** vertices,
+                                                    size_t* n_triangles, uint32_t** tri_indices)
+    {
+        if (hpsdf_device_count() == 0) { setLastError("no CUDA device available: this library has no CPU path"); return HPSDF_ERR_NO_DEVICE; }
+        if (!tree || !resolution || !n_vertices || !vertices || !n_triangles || !tri_indices) { setLastError("null pointer"); return HPSDF_ERR_INVALID_ARG; }
+        *n_vertices = 0; *vertices = nullptr; *n_triangles = 0; *tri_indices = nullptr;
+        if (!box_min != !box_max) { setLastError("hpsdf_extract_isosurface: give both box corners or neither"); return HPSDF_ERR_INVALID_ARG; }
+        IsoGrid g;
+        g.iso = iso;
+        for (int a = 0; a < 3; ++a)
+        {
+            if (resolution[a] < 1 || resolution[a] > 1024) { setLastError("hpsdf_extract_isosurface: resolution outside [1, 1024]"); return HPSDF_ERR_INVALID_ARG; }
+            const double lo = box_min ? box_min[a] : (double)tree->cfg.root_min[a], hi = box_max ? box_max[a] : (double)tree->cfg.root_max[a];
+            if (!(lo < hi) || !std::isfinite(lo) || !std::isfinite(hi)) { setLastError("hpsdf_extract_isosurface: the box needs finite min < max"); return HPSDF_ERR_INVALID_ARG; }
+            g.n[a] = resolution[a];
+            g.lo[a] = lo;
+            g.h[a] = (hi - lo) / (double)resolution[a];
+        }
+        const uint32_t nPoints = (g.n[0] + 1) * (g.n[1] + 1) * (g.n[2] + 1);        // <= 1025^3 < 2^32
+        HPSDF_CUDA(cudaSetDevice(tree->device));
+        // HPSDF_ISO_TIMES: device time of the phases on stderr (grid, count + scans, emit, copy)
+        const bool timed = getenv("HPSDF_ISO_TIMES") != nullptr;
+        cudaStream_t stream = nullptr;
+        cudaEvent_t ev[6] = { nullptr, nullptr, nullptr, nullptr, nullptr, nullptr };
+        void* scratch = nullptr;
+        char* dOut = nullptr;
+        float* hV = nullptr;
+        uint32_t* hT = nullptr;
+        unsigned long long totals[2] = { 0, 0 };
+        hpsdf_status st = HPSDF_OK;
+        cudaError_t e = cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking);
+        for (int i = 0; i < 6 && timed && e == cudaSuccess; ++i) e = cudaEventCreate(&ev[i]);
+        auto mark = [&](int i) { if (timed && e == cudaSuccess) e = cudaEventRecord(ev[i], stream); };
+        if (e == cudaSuccess) e = cudaMalloc(&scratch, isoScratchBytes(nPoints));
+        IsoScratch s{};
+        if (e == cudaSuccess) s = carveIsoScratch(scratch, nPoints);
+        mark(0);
+        if (e == cudaSuccess) e = launchIsoGrid(tree->view, g, s, tree->ctx->smCount, stream);
+        mark(1);
+        if (e == cudaSuccess) e = launchIsoCount(g, s, tree->ctx->smCount, totals, stream);
+        mark(2);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(stream);
+        const size_t nv = (size_t)totals[0], nt = (size_t)totals[1];
+        if (e == cudaSuccess && (totals[0] > 0xFFFFFFFFull || totals[1] > 0xFFFFFFFFull))
+        {
+            setLastError("hpsdf_extract_isosurface: " + std::to_string(totals[0]) + " vertices and " + std::to_string(totals[1]) +
+                         " triangles: a count above 2^32 - 1 does not fit the uint32 indices");
+            st = HPSDF_ERR_UNSUPPORTED;
+        }
+        const size_t vBytes = (nv * 12 + 255) & ~(size_t)255;
+        if (e == cudaSuccess && st == HPSDF_OK && nv)
+        {
+            e = cudaMalloc((void**)&dOut, vBytes + nt * 12);
+            hV = (float*)malloc(nv * 12);
+            hT = (uint32_t*)malloc(nt * 12);
+            if (e == cudaSuccess && (!hV || !hT)) { setLastError("hpsdf_extract_isosurface: host allocation failed"); st = HPSDF_ERR_OOM; }
+            mark(3);
+            if (e == cudaSuccess && st == HPSDF_OK) e = launchIsoEmit(g, s, (float*)dOut, (uint32_t*)(dOut + vBytes), stream);
+            mark(4);
+            if (e == cudaSuccess && st == HPSDF_OK) e = cudaMemcpyAsync(hV, dOut, nv * 12, cudaMemcpyDeviceToHost, stream);
+            if (e == cudaSuccess && st == HPSDF_OK) e = cudaMemcpyAsync(hT, dOut + vBytes, nt * 12, cudaMemcpyDeviceToHost, stream);
+            mark(5);
+            if (e == cudaSuccess) e = cudaStreamSynchronize(stream);
+        }
+        if (timed && e == cudaSuccess && st == HPSDF_OK)
+        {
+            float ms[4] = { 0, 0, 0, 0 };
+            cudaEventElapsedTime(&ms[0], ev[0], ev[1]);
+            cudaEventElapsedTime(&ms[1], ev[1], ev[2]);
+            if (nv) { cudaEventElapsedTime(&ms[2], ev[3], ev[4]); cudaEventElapsedTime(&ms[3], ev[4], ev[5]); }
+            fprintf(stderr, "hpsdf_extract_isosurface: %u x %u x %u cells, %zu vertices, %zu triangles; grid %.3f ms, count+scan %.3f ms, emit %.3f ms, copy %.3f ms\n",
+                    g.n[0], g.n[1], g.n[2], nv, nt, ms[0], ms[1], ms[2], ms[3]);
+        }
+        if (stream) cudaStreamSynchronize(stream);
+        for (int i = 0; i < 6; ++i) if (ev[i]) cudaEventDestroy(ev[i]);
+        if (stream) cudaStreamDestroy(stream);
+        cudaFree(scratch);
+        cudaFree(dOut);
+        if (e != cudaSuccess) st = failCuda(e, "hpsdf_extract_isosurface");
+        if (st != HPSDF_OK) { free(hV); free(hT); return st; }
+        *n_vertices = nv; *vertices = hV; *n_triangles = nt; *tri_indices = hT;
         return HPSDF_OK;
     }
 

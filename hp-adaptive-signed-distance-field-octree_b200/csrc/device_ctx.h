@@ -130,6 +130,30 @@ namespace hpsdf
     cudaError_t launchQueryRay(const DeviceTreeView& view, const double* dOrigins, const double* dDirs, size_t n, double tMax,
                                unsigned char* dHit, double* dT, cudaStream_t stream);
     cudaError_t launchQueryGradient(const DeviceTreeView& view, const double* dXyz, size_t n, double* dOut, double* dGrad, cudaStream_t stream);
+    // hpsdf_extract_isosurface (isosurface_kernels.cuh): a grid of (n0+1)(n1+1)(n2+1) < 2^32 points
+    struct IsoGrid
+    {
+        double   lo[3], h[3];     // point (i,j,k) = lo + idx * h per axis
+        double   iso;
+        uint32_t n[3];            // cells per axis
+    };
+    struct IsoScratch             // about 18 bytes per grid point
+    {
+        double*   vals;
+        uint8_t*  mask;           // crossing owned edges, bit d-1 = direction d
+        uint8_t*  label;          // inside bits of the cell whose lowest corner the point is (0 for points that are none)
+        uint32_t* vbase;          // exclusive scans: first vertex / triangle of the point
+        uint32_t* tbase;
+        unsigned long long* totals;   // vertices, triangles (64-bit)
+        void*     cubTmp;
+        size_t    cubTmpBytes;
+    };
+    size_t      isoScratchBytes(uint32_t nPoints);
+    IsoScratch  carveIsoScratch(void* mem, uint32_t nPoints);
+    cudaError_t launchIsoGrid(const DeviceTreeView& view, const IsoGrid& g, const IsoScratch& s, int smCount, cudaStream_t stream);
+    // masks, labels, the two scans; hostTotals[0..1] hold the vertex and triangle totals once the stream has drained
+    cudaError_t launchIsoCount(const IsoGrid& g, const IsoScratch& s, int smCount, unsigned long long* hostTotals, cudaStream_t stream);
+    cudaError_t launchIsoEmit(const IsoGrid& g, const IsoScratch& s, float* dVerts, uint32_t* dTris, cudaStream_t stream);
     // continuity (continuity_kernels.cuh)
     cudaError_t launchFaceEmit(const FaceJobDev* dFaces, uint32_t nFaces, const DeviceCtx& ctx, uint64_t* keys, double* vals, uint32_t n, cudaStream_t stream);
     size_t      faceEnumTempBytes(uint32_t nNodes);

@@ -23,6 +23,7 @@ namespace hpsdf
 #include "sched_kernels.cuh"
 #include "finish_kernels.cuh"
 #include "mesh_build.cuh"
+#include "isosurface_kernels.cuh"
 
 namespace hpsdf
 {
@@ -44,6 +45,12 @@ namespace hpsdf
         }
         cudaMemcpyToSymbol(c_lp1, lp1, sizeof(lp1));
         cudaMemcpyToSymbol(c_lm1, lm1, sizeof(lm1));
+        IsoTetCase tet[6][16];
+        uint8_t chain[6][4], cellTris[256];
+        isoBuildTables(tet, chain, cellTris);
+        cudaMemcpyToSymbol(c_isoTet, tet, sizeof(tet));
+        cudaMemcpyToSymbol(c_isoChain, chain, sizeof(chain));
+        cudaMemcpyToSymbol(c_isoCellTris, cellTris, sizeof(cellTris));
     }
 
     static const uint32_t* g_bidxDev[16] = { nullptr };
@@ -478,6 +485,81 @@ namespace hpsdf
     {
         if (!n) return cudaSuccess;
         meshDistanceKernel<<<(unsigned)((n + 127) / 128), 128, 0, stream>>>(dView, dXyz, n, dOut);
+        return cudaGetLastError();
+    }
+
+    // ---- hpsdf_extract_isosurface (isosurface_kernels.cuh) -------------------------------------------------------------------
+    using IsoVertexCounts = thrust::transform_iterator<IsoPopc, const uint8_t*, uint32_t>;
+    using IsoTriCounts = thrust::transform_iterator<IsoCellTriCount, const uint8_t*, uint32_t>;
+
+    static size_t isoScanTempBytes(uint32_t nPoints)
+    {
+        size_t a = 0, b = 0;
+        cub::DeviceScan::ExclusiveSum(nullptr, a, IsoVertexCounts(nullptr, IsoPopc()), (uint32_t*)nullptr, (int)nPoints, (cudaStream_t)0);
+        cub::DeviceScan::ExclusiveSum(nullptr, b, IsoTriCounts(nullptr, IsoCellTriCount()), (uint32_t*)nullptr, (int)nPoints, (cudaStream_t)0);
+        return std::max(a, b);
+    }
+
+    size_t isoScratchBytes(uint32_t nPoints)
+    {
+        auto al = [](size_t b) { return (b + 255) & ~(size_t)255; };
+        const size_t n = nPoints;
+        return al(n * 8) + 2 * al(n) + 2 * al(n * 4) + 256 + al(isoScanTempBytes(nPoints));
+    }
+
+    IsoScratch carveIsoScratch(void* mem, uint32_t nPoints)
+    {
+        auto al = [](size_t b) { return (b + 255) & ~(size_t)255; };
+        const size_t n = nPoints;
+        char* p = (char*)mem;
+        auto take = [&](size_t bytes) { char* at = p; p += al(bytes); return at; };
+        IsoScratch s;
+        s.vals = (double*)take(n * 8);
+        s.mask = (uint8_t*)take(n);
+        s.label = (uint8_t*)take(n);
+        s.vbase = (uint32_t*)take(n * 4);
+        s.tbase = (uint32_t*)take(n * 4);
+        s.totals = (unsigned long long*)take(256);
+        s.cubTmpBytes = isoScanTempBytes(nPoints);
+        s.cubTmp = take(s.cubTmpBytes);
+        return s;
+    }
+
+    static uint32_t isoPoints(const IsoGrid& g) { return (g.n[0] + 1) * (g.n[1] + 1) * (g.n[2] + 1); }
+
+    cudaError_t launchIsoGrid(const DeviceTreeView& view, const IsoGrid& g, const IsoScratch& s, int smCount, cudaStream_t stream)
+    {
+        const size_t groups = ((size_t)isoPoints(g) + 31) / 32;
+        size_t grid = (size_t)(smCount > 0 ? smCount : 148) * kQueryBlocksPerSm;
+        if (grid > (groups + 7) / 8) grid = (groups + 7) / 8;
+        int dev = 0;
+        cudaGetDevice(&dev);
+        isoGridKernel<<<(unsigned)grid, kQueryThreads, 0, stream>>>(view, g, s.vals, g_bidxDev[dev & 15]);
+        return cudaGetLastError();
+    }
+
+    cudaError_t launchIsoCount(const IsoGrid& g, const IsoScratch& s, int smCount, unsigned long long* hostTotals, cudaStream_t stream)
+    {
+        const uint32_t n = isoPoints(g);
+        cudaError_t e = cudaMemsetAsync(s.totals, 0, 16, stream);
+        if (e != cudaSuccess) return e;
+        size_t grid = (size_t)(smCount > 0 ? smCount : 148) * 8;
+        if (grid > ((size_t)n + 255) / 256) grid = ((size_t)n + 255) / 256;
+        isoCountKernel<<<(unsigned)grid, 256, 0, stream>>>(g, s.vals, s.mask, s.label, s.totals);
+        if ((e = cudaGetLastError()) != cudaSuccess) return e;
+        size_t tb = s.cubTmpBytes;
+        e = cub::DeviceScan::ExclusiveSum(s.cubTmp, tb, IsoVertexCounts(s.mask, IsoPopc()), s.vbase, (int)n, stream);
+        tb = s.cubTmpBytes;
+        if (e == cudaSuccess) e = cub::DeviceScan::ExclusiveSum(s.cubTmp, tb, IsoTriCounts(s.label, IsoCellTriCount()), s.tbase, (int)n, stream);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(hostTotals, s.totals, 16, cudaMemcpyDeviceToHost, stream);
+        return e;
+    }
+
+    cudaError_t launchIsoEmit(const IsoGrid& g, const IsoScratch& s, float* dVerts, uint32_t* dTris, cudaStream_t stream)
+    {
+        const uint32_t n = isoPoints(g), blocks = (uint32_t)(((size_t)n + 255) / 256);
+        isoEmitKernel<<<blocks, 256, 0, stream>>>(g, s.vals, s.mask, s.vbase, dVerts);
+        isoTriKernel<<<blocks, 256, 0, stream>>>(g, s.label, s.mask, s.vbase, s.tbase, dTris);
         return cudaGetLastError();
     }
 }

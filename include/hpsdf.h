@@ -229,6 +229,25 @@ HPSDF_API hpsdf_status hpsdf_query_with_gradient(const hpsdf_octree* tree, const
 HPSDF_API hpsdf_status hpsdf_query_ray(const hpsdf_octree* tree, const double* origins, const double* directions, size_t n, double t_max,
                                        unsigned char* hit, double* t);
 
+/* The level set F = iso of the tree as a triangle mesh: marching tetrahedra over a uniform grid of
+ * resolution[0] x resolution[1] x resolution[2] cells spanning [box_min, box_max] (both NULL = the root box).
+ * Grid values are Query values (DBL_MAX outside the root). Vertices: n_vertices x 3 float32, triangles:
+ * n_triangles x 3 uint32, counter-clockwise seen from the side where F >= iso. Both arrays are malloc()ed;
+ * the CALLER free()s them (as hpsdf_to_memory_block). An empty result gives 0, 0 and NULL pointers.
+ * Blocks the calling thread; runs on the tree's device.
+ *
+ * Grid point (i,j,k) is box_min + idx * h per axis, h = (box_max - box_min) / resolution, each operation rounded in f64;
+ * a corner is inside when its value is below iso. Every cell is cut into the six Kuhn tetrahedra along its 0-7 diagonal.
+ * Vertices are ordered by the grid point that owns their edge (its lower end), then by edge direction; triangles by cell,
+ * tetrahedron and position (DESIGN.md §11 has the full contract). When no grid point on the box's boundary faces is
+ * inside, the mesh is a closed, oriented 2-manifold with every vertex used (hpsdf_mesh_create accepts it); a surface that
+ * crosses the box leaves the mesh open there. A grid value exactly equal to iso puts vertices on that grid point, so
+ * zero-area triangles can appear. Resolutions are 1..1024; HPSDF_ERR_UNSUPPORTED when either count exceeds 2^32 - 1. */
+HPSDF_API hpsdf_status hpsdf_extract_isosurface(const hpsdf_octree* tree, const uint32_t resolution[3],
+                                                const double box_min[3], const double box_max[3], double iso,
+                                                size_t* n_vertices, float** vertices,
+                                                size_t* n_triangles, uint32_t** tri_indices);
+
 /* Octree::ToMemoryBlock (Octree.cpp:424-456): *ptr is malloc()ed, the CALLER free()s it. LP64 layout. */
 HPSDF_API hpsdf_status hpsdf_to_memory_block(const hpsdf_octree* tree, size_t* size, void** ptr);
 /* Octree::FromMemoryBlock (Octree.cpp:403-421): copies; the caller keeps ownership of the block. */

@@ -4,7 +4,8 @@
 //     SDF::Config                 Include/HP/Config.h:12-43        (same members, same 80-byte LP64 image)
 //     SDF::Octree                 Include/HP/Octree.h:36-86        Create / Query / QueryWithGradient / QueryRay / UnionSDF /
 //                                                                  SubtractSDF / IntersectSDF / Clear / FromMemoryBlock /
-//                                                                  ToMemoryBlock / GetRootAABB, copy + move
+//                                                                  ToMemoryBlock / GetRootAABB, copy + move; plus
+//                                                                  ExtractIsosurface (no counterpart in the reference)
 //     MemoryBlock                 Include/Utility/MemoryBlock.h:5-9
 //
 // Differences, all forced by the device: (1) Create takes an SDF::Program (closed-form primitives / meshes / trees
@@ -19,6 +20,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <functional>
+#include <memory>
 #include <stdexcept>
 #include <string>
 #include <thread>
@@ -214,6 +216,22 @@ namespace SDF
         void QueryRay(const double* origins_, const double* directions_, size_t n_, double tMax_, unsigned char* hit_, double* t_) const
         {
             check(hpsdf_query_ray(need(), origins_, directions_, n_, tMax_, hit_, t_));
+        }
+
+        /// The level set F = iso_ as a triangle mesh (hpsdf_extract_isosurface): marching tetrahedra over resolution_ cells per axis
+        /// spanning [boxMin_, boxMax_] (both nullptr = the root box). vertices_ gets 3 floats per vertex, triIndices_ 3 indices per
+        /// triangle, counter-clockwise seen from the side where F >= iso_: what Meshing::Mesh::Create takes.
+        void ExtractIsosurface(const uint32_t resolution_[3], double iso_, std::vector<float>& vertices_, std::vector<uint32_t>& triIndices_,
+                               const double* boxMin_ = nullptr, const double* boxMax_ = nullptr) const
+        {
+            size_t nv = 0, nt = 0;
+            float* v = nullptr;
+            uint32_t* t = nullptr;
+            check(hpsdf_extract_isosurface(need(), resolution_, boxMin_, boxMax_, iso_, &nv, &v, &nt, &t));
+            std::unique_ptr<float, void (*)(void*)> ownV(v, std::free);
+            std::unique_ptr<uint32_t, void (*)(void*)> ownT(t, std::free);
+            vertices_.assign(v, v + 3 * nv);
+            triIndices_.assign(t, t + 3 * nt);
         }
 
         /// The aabb of the root node (Octree.cpp:106-109)
