@@ -60,6 +60,7 @@ namespace hpsdf
         DeviceBuf<uint32_t>  segs;
         DeviceBuf<double>    samples;     // F at the Gauss-Legendre points of a chunk of fits (mesh / octree programs only)
         DeviceBuf<unsigned long long> sampleCounter;   // work counter of meshSampleKernel
+        DeviceBuf<float4>    meshCut;     // per-fit cuts of the mesh BVH next to the sample scratch (mesh_sample_kernel.cuh: meshCutKernel)
         PinnedBuf<FitTask>   hTasks;
         DeviceBuf<JobDesc>   jobs;
         PinnedBuf<JobDesc>   hJobs;

@@ -82,6 +82,10 @@ namespace hpsdf
                 c[kStatLeafTest] / q, c[kStatLeafPruned] / q,
                 c[kStatWarpNodeIter] ? (double)(c[kStatNodeVisit] + c[kStatStalePop]) / c[kStatWarpNodeIter] : 0.0,
                 c[kStatWarpTriIter] ? (double)(c[kStatLeafTest] + c[kStatLeafPruned]) / c[kStatWarpTriIter] : 0.0);
+        const unsigned long long* k = h + kCutStatWord;
+        if (k[3])
+            fprintf(stderr, "meshCutKernel: %llu fits, mean %.2f cut entries, max %llu; %.1f %% of the cuts are still the root's children\n",
+                    k[3], (double)k[0] / k[3], k[1], 100.0 * k[2] / k[3]);
     }
 
     // HPSDF_DEBUG_ROUNDS=3: events around the sample and fit kernels of every degree group (diagnostics only)
@@ -110,8 +114,8 @@ namespace hpsdf
 
     template <int D, bool EXT>
     static cudaError_t launchOne(const FitTask* dTasks, int n, double* pool, FitRecord* recs, const SdfProgramDev& prog,
-                                 const RootMap& map, const FitTablesDev& tab, double* samples, size_t sampleCap, unsigned long long* counter,
-                                 int smCount, cudaStream_t stream)
+                                 const RootMap& map, const FitTablesDev& tab, double* samples, size_t sampleCap, float4* cut,
+                                 unsigned long long* counter, int smCount, cudaStream_t stream)
     {
         constexpr size_t smem = fitSmemDoubles(D) * sizeof(double);
         static bool attrSet[16] = { false };
@@ -131,8 +135,9 @@ namespace hpsdf
         else
         {
             constexpr size_t n3 = (size_t)fitRule(D) * fitRule(D) * fitRule(D);
-            const size_t chunk = sampleCap / n3;
-            if (!samples || !chunk) return cudaErrorInvalidValue;
+            // the cut records of a chunk are indexed in bits 0-27 of a stack entry (mesh_sample_kernel.cuh)
+            const size_t chunk = std::min(sampleCap / n3, ((size_t)1 << 28) / kCutStride - 1);
+            if (!samples || !cut || !chunk) return cudaErrorInvalidValue;
             for (size_t b = 0; b < (size_t)n; b += chunk)
             {
                 const size_t m = std::min(chunk, (size_t)n - b);
@@ -159,8 +164,12 @@ namespace hpsdf
                     constexpr int triThreshold = 16;
                     unsigned long long* stats = meshStatsBuffer();
                     const size_t statSmem = stats ? (size_t)kMeshStatCount * 256 * sizeof(unsigned) : 0;
-                    meshSampleKernel<<<(unsigned)std::min(want, sms * 4), 256, statSmem, stream>>>(dTasks + b, total, D, (const DeviceMeshView*)prog.instr[0].handle,
-                                                                                                 map, tab, samples, counter, grab, triThreshold, getenv("HPSDF_MESH_NO_HANDOVER") ? 0 : 1, stats);
+                    const DeviceMeshView* mesh = (const DeviceMeshView*)prog.instr[0].handle;
+                    // every sample of a fit starts from the fit's cut of the tree (HPSDF_MESH_NO_CUT: from the root, for A/B runs)
+                    const bool useCut = getenv("HPSDF_MESH_NO_CUT") == nullptr;
+                    if (useCut) meshCutKernel<<<(unsigned)((m + 3) / 4), 128, 0, stream>>>(dTasks + b, (unsigned)m, D, mesh, map, tab, cut, stats);
+                    meshSampleKernel<<<(unsigned)std::min(want, sms * 4), 256, statSmem, stream>>>(dTasks + b, total, D, mesh, map, tab, samples, counter, grab, triThreshold,
+                                                                                                 getenv("HPSDF_MESH_NO_HANDOVER") ? 0 : 1, useCut ? cut : nullptr, stats);
                 }
                 else
                 {
@@ -184,13 +193,13 @@ namespace hpsdf
 
     template <bool EXT>
     static cudaError_t launchFitKernelT(int degree, const FitTask* dTasks, int n, double* pool, FitRecord* recs, const SdfProgramDev& prog,
-                                        const RootMap& map, const FitTablesDev& tab, double* samples, size_t sampleCap, unsigned long long* counter,
-                                        int smCount, cudaStream_t stream)
+                                        const RootMap& map, const FitTablesDev& tab, double* samples, size_t sampleCap, float4* cut,
+                                        unsigned long long* counter, int smCount, cudaStream_t stream)
     {
         if (n <= 0) return cudaSuccess;
         switch (degree)
         {
-#define HPSDF_FIT_CASE(d) case d: return launchOne<d, EXT>(dTasks, n, pool, recs, prog, map, tab, samples, sampleCap, counter, smCount, stream);
+#define HPSDF_FIT_CASE(d) case d: return launchOne<d, EXT>(dTasks, n, pool, recs, prog, map, tab, samples, sampleCap, cut, counter, smCount, stream);
             HPSDF_FIT_CASE(1) HPSDF_FIT_CASE(2) HPSDF_FIT_CASE(3) HPSDF_FIT_CASE(4) HPSDF_FIT_CASE(5) HPSDF_FIT_CASE(6)
             HPSDF_FIT_CASE(7) HPSDF_FIT_CASE(8) HPSDF_FIT_CASE(9) HPSDF_FIT_CASE(10) HPSDF_FIT_CASE(11)
 #undef HPSDF_FIT_CASE
@@ -198,14 +207,21 @@ namespace hpsdf
         }
     }
 
-    // Sample scratch of mesh / octree programs: grow-only, sized by the caller BEFORE a round whose degree groups run
-    // concurrently (a reallocation inside the round would pull the buffer from under the launches in flight).
+    // cut records (meshCutKernel) that go with `doubles` of sample scratch: a slice at sample offset o owns the records from
+    // cutOffset(o) on, and no chunk of it has more fits than the slice has multiples of the smallest fit's sample count
+    static size_t cutFloat4s(size_t doubles) { return (doubles / kCutSamplesPerFit + 1) * kCutStride * 8; }
+    static size_t cutOffset(size_t sampleOffset) { return sampleOffset / kCutSamplesPerFit * kCutStride * 8; }
+
+    // Sample scratch of mesh / octree programs and the cut records next to it: grow-only, sized by the caller BEFORE a round
+    // whose degree groups run concurrently (a reallocation inside the round would pull the buffers from under the launches in
+    // flight).
     cudaError_t reserveSampleScratch(DeviceCtx& ctx, size_t doubles, cudaStream_t stream)
     {
-        if (ctx.ws.samples.cap < doubles)
+        if (ctx.ws.samples.cap < doubles || ctx.ws.meshCut.cap < cutFloat4s(doubles))
         {
             cudaError_t e = cudaStreamSynchronize(stream);
             if (e == cudaSuccess) e = ctx.ws.samples.reserve(doubles);
+            if (e == cudaSuccess) e = ctx.ws.meshCut.reserve(cutFloat4s(doubles));
             if (e != cudaSuccess) return e;
         }
         if (!ctx.ws.sampleCounter.p) return ctx.ws.sampleCounter.reserve(32);
@@ -220,13 +236,13 @@ namespace hpsdf
                                 const SdfProgramDev& prog, const RootMap& map, DeviceCtx& ctx, cudaStream_t stream,
                                 size_t sliceOffset, size_t sliceDoubles, int counterIdx)
     {
-        if (!programHasExt(prog)) return launchFitKernelT<false>(degree, dTasks, n, pool, recs, prog, map, ctx.fitTab, nullptr, 0, nullptr, ctx.smCount, stream);
+        if (!programHasExt(prog)) return launchFitKernelT<false>(degree, dTasks, n, pool, recs, prog, map, ctx.fitTab, nullptr, 0, nullptr, nullptr, ctx.smCount, stream);
         const size_t n3 = (size_t)fitRule(degree) * fitRule(degree) * fitRule(degree);
         if (sliceDoubles)
         {
             if (sliceDoubles < (size_t)std::max(n, 1) * n3 || sliceOffset + sliceDoubles > ctx.ws.samples.cap || !ctx.ws.sampleCounter.p) return cudaErrorInvalidValue;
             return launchFitKernelT<true>(degree, dTasks, n, pool, recs, prog, map, ctx.fitTab, ctx.ws.samples.p + sliceOffset, sliceDoubles,
-                                          ctx.ws.sampleCounter.p + counterIdx, ctx.smCount, stream);
+                                          ctx.ws.meshCut.p + cutOffset(sliceOffset), ctx.ws.sampleCounter.p + counterIdx, ctx.smCount, stream);
         }
         // chunk size limit; HPSDF_SAMPLE_CAP (doubles, read per call) lets the tests force the multi-chunk path on small inputs
         size_t limit = kSampleScratchDoubles;
@@ -236,7 +252,7 @@ namespace hpsdf
         const cudaError_t e = reserveSampleScratch(ctx, want, stream);
         if (e != cudaSuccess) return e;
         return launchFitKernelT<true>(degree, dTasks, n, pool, recs, prog, map, ctx.fitTab, ctx.ws.samples.p, std::min(ctx.ws.samples.cap, limit),
-                                      ctx.ws.sampleCounter.p, ctx.smCount, stream);
+                                      ctx.ws.meshCut.p, ctx.ws.sampleCounter.p, ctx.smCount, stream);
     }
 
     // ---- job records -> fit tasks ------------------------------------------------------------------------------------

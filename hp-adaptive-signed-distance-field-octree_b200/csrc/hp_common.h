@@ -184,6 +184,7 @@ namespace hpsdf
         const void*     triVerts;     // 3 float4 per triangle SLOT (BVH order): a, b, c; .w of a = original triangle index (bits)
         const float*    pseudo;       // 21 floats per ORIGINAL triangle: face normal, 3 edge normals (AB, BC, CA), 3 vertex normals (A, B, C)
         uint32_t        nTris, nNodes;
+        float           inflate;      // absolute margin of the boxes against f32 rounding: 1e-5 of the mesh's size (mesh.cpp)
     };
 
     // Device SDF program (hpsdf_sdf_program with handles resolved to device pointers). Passed by value as a kernel parameter.

@@ -198,6 +198,7 @@ extern "C"
         }
         // float32 projection error on the device is ~1e-7 |p|; query points live in a root box of about the mesh's size
         const double inflate = 1e-5 * std::max(std::sqrt(diag2), maxAbs);
+        m->view.inflate = (float)inflate;
         e = meshBuildBoxes(M, T, order, nNodes, inflate, m->view.nodes, (float*)m->view.obb, (float*)m->view.wide, (float4*)m->view.triVerts, stream);
         if (e == cudaSuccess) e = cudaMemcpyAsync(m->dView, &m->view, sizeof(DeviceMeshView), cudaMemcpyHostToDevice, stream);
         if (e == cudaSuccess) e = cudaStreamSynchronize(stream);
