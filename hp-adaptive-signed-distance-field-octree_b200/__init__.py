@@ -128,6 +128,7 @@ EXPORTS = [
     "hpsdf_bench_frontier", "hpsdf_measure_fp64_peak", "hpsdf_comm_get_unique_id", "hpsdf_comm_init",
     "hpsdf_comm_destroy", "hpsdf_shard_range", "hpsdf_set_jit", "hpsdf_jit_compile_check", "hpsdf_query_ray",
     "hpsdf_get_config", "hpsdf_get_device", "hpsdf_uniform_points_device", "hpsdf_extract_isosurface",
+    "hpsdf_raycast", "hpsdf_raycast_device",
 ]
 
 _lib = None
@@ -169,6 +170,8 @@ def lib():
     L.hpsdf_query_device.argtypes = [vp, vp, sz, vp, vp]
     L.hpsdf_query_with_gradient.argtypes = [vp, vp, sz, vp, vp]
     L.hpsdf_query_ray.argtypes = [vp, vp, vp, sz, dbl, vp, vp]
+    L.hpsdf_raycast.argtypes = [vp, vp, vp, sz, dbl, dbl, dbl, vp, vp]
+    L.hpsdf_raycast_device.argtypes = [vp, vp, vp, sz, dbl, dbl, dbl, vp, vp, vp]
     L.hpsdf_extract_isosurface.argtypes = [vp, vp, vp, vp, dbl, C.POINTER(sz), C.POINTER(vp), C.POINTER(sz), C.POINTER(vp)]
     L.hpsdf_to_memory_block.argtypes = [vp, C.POINTER(sz), C.POINTER(vp)]
     L.hpsdf_from_memory_block.argtypes = [vp, sz, i32, C.POINTER(vp)]
@@ -358,6 +361,25 @@ class Octree:
         t = np.zeros(len(o), np.float64)
         _check(lib().hpsdf_query_ray(self._h, o.ctypes.data, d.ctypes.data, len(o), float(t_max), hit.ctypes.data, t.ctypes.data))
         return hit.astype(bool), t
+
+    def Raycast(self, origins, directions, t_min=0.0, t_max=np.inf, iso=0.0):
+        """First crossing of F = iso along rays o + t d, t in [t_min, t_max] (hpsdf_raycast; d need not be unit, t is in units
+        of d) -> (t (n,) f64, +inf for a miss; normals (n,3) f64, unit gradients of the hit leaf's polynomial, 0 on a miss).
+        Exact per leaf (DESIGN §12); the ray query to use, where QueryRay mirrors the reference."""
+        o = np.ascontiguousarray(origins, np.float64).reshape(-1, 3)
+        d = np.ascontiguousarray(directions, np.float64).reshape(-1, 3)
+        if len(o) != len(d):
+            raise HpsdfError(ERR_INVALID_ARG, "origins and directions differ in length")
+        t = np.empty(len(o), np.float64)
+        nrm = np.empty((len(o), 3), np.float64)
+        _check(lib().hpsdf_raycast(self._h, o.ctypes.data, d.ctypes.data, len(o), float(t_min), float(t_max), float(iso),
+                                   t.ctypes.data, nrm.ctypes.data))
+        return t, nrm
+
+    def RaycastDevice(self, d_origins, d_directions, n, d_t, d_normals=None, t_min=0.0, t_max=np.inf, iso=0.0, stream=None):
+        """Raycast with device pointers (e.g. torch tensors' data_ptr()), asynchronous on `stream` (cudaStream_t as int)."""
+        _check(lib().hpsdf_raycast_device(self._h, d_origins, d_directions, n, float(t_min), float(t_max), float(iso), d_t, d_normals,
+                                          stream))
 
     def OutputFunctionSlice(self, fname, c, view_min, view_max, n_samples=2048):
         """Octree::OutputFunctionSlice (Octree.cpp:1132-1205): the z = c slice of the field over viewArea as an n x n grid of

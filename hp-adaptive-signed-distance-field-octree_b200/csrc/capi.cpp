@@ -207,6 +207,50 @@ extern "C"
         return HPSDF_OK;
     }
 
+    static hpsdf_status raycastArgs(const hpsdf_octree* tree, const void* origins, const void* directions, size_t n, double t_min,
+                                    double t_max, double iso, const void* t_hit, const char* fn)
+    {
+        if (hpsdf_device_count() == 0) { setLastError("no CUDA device available: this library has no CPU path"); return HPSDF_ERR_NO_DEVICE; }
+        if (!tree || (n && (!origins || !directions || !t_hit))) { setLastError("null pointer"); return HPSDF_ERR_INVALID_ARG; }
+        if (!std::isfinite(t_min) || !std::isfinite(iso) || !(t_max >= t_min))
+        { setLastError(std::string(fn) + ": t_min and iso must be finite and t_max >= t_min"); return HPSDF_ERR_INVALID_ARG; }
+        return HPSDF_OK;
+    }
+
+    HPSDF_API hpsdf_status hpsdf_raycast(const hpsdf_octree* tree, const double* origins, const double* directions, size_t n, double t_min,
+                                         double t_max, double iso, double* t_hit, double* normals)
+    {
+        hpsdf_status st = raycastArgs(tree, origins, directions, n, t_min, t_max, iso, t_hit, "hpsdf_raycast");
+        if (st != HPSDF_OK || !n) return st;
+        HPSDF_CUDA(cudaSetDevice(tree->device));
+        double *dO = nullptr, *dD = nullptr, *dT = nullptr, *dN = nullptr;
+        HPSDF_CUDA(cudaMalloc((void**)&dO, n * 24));
+        cudaError_t e = cudaMalloc((void**)&dD, n * 24);
+        if (e == cudaSuccess) e = cudaMalloc((void**)&dT, n * 8);
+        if (e == cudaSuccess && normals) e = cudaMalloc((void**)&dN, n * 24);
+        if (e == cudaSuccess) e = cudaMemcpy(dO, origins, n * 24, cudaMemcpyHostToDevice);
+        if (e == cudaSuccess) e = cudaMemcpy(dD, directions, n * 24, cudaMemcpyHostToDevice);
+        if (e == cudaSuccess) e = launchRaycast(tree->view, dO, dD, n, t_min, t_max, iso, dT, dN, tree->ctx->smCount, nullptr);
+        if (e == cudaSuccess) e = cudaMemcpy(t_hit, dT, n * 8, cudaMemcpyDeviceToHost);
+        if (e == cudaSuccess && normals) e = cudaMemcpy(normals, dN, n * 24, cudaMemcpyDeviceToHost);
+        cudaFree(dO); cudaFree(dD); cudaFree(dT); cudaFree(dN);
+        if (e != cudaSuccess) return failCuda(e, "hpsdf_raycast");
+        return HPSDF_OK;
+    }
+
+    HPSDF_API hpsdf_status hpsdf_raycast_device(const hpsdf_octree* tree, const double* d_origins, const double* d_directions, size_t n,
+                                                double t_min, double t_max, double iso, double* d_t_hit, double* d_normals, void* stream)
+    {
+        hpsdf_status st = raycastArgs(tree, d_origins, d_directions, n, t_min, t_max, iso, d_t_hit, "hpsdf_raycast_device");
+        if (st != HPSDF_OK) return st;
+        int cur = -1;
+        if (cudaGetDevice(&cur) != cudaSuccess || cur != tree->device)
+        { setLastError("hpsdf_raycast_device: the current CUDA device is not the tree's device"); return HPSDF_ERR_INVALID_ARG; }
+        HPSDF_CUDA(launchRaycast(tree->view, d_origins, d_directions, n, t_min, t_max, iso, d_t_hit, d_normals, tree->ctx->smCount,
+                                 (cudaStream_t)stream));
+        return HPSDF_OK;
+    }
+
     HPSDF_API hpsdf_status hpsdf_extract_isosurface(const hpsdf_octree* tree, const uint32_t resolution[3], const double box_min[3],
                                                     const double box_max[3], double iso, size_t* n_vertices, float** vertices,
                                                     size_t* n_triangles, uint32_t** tri_indices)

@@ -130,6 +130,9 @@ namespace hpsdf
     cudaError_t launchQuery(const DeviceTreeView& view, const double* dXyz, size_t n, double* dOut, int smCount, cudaStream_t stream);
     cudaError_t launchQueryRay(const DeviceTreeView& view, const double* dOrigins, const double* dDirs, size_t n, double tMax,
                                unsigned char* dHit, double* dT, cudaStream_t stream);
+    // hpsdf_raycast (raycast_kernels.cuh): first crossing of F = iso per ray; dNormals may be nullptr
+    cudaError_t launchRaycast(const DeviceTreeView& view, const double* dOrigins, const double* dDirs, size_t n, double tMin, double tMax,
+                              double iso, double* dT, double* dNormals, int smCount, cudaStream_t stream);
     cudaError_t launchQueryGradient(const DeviceTreeView& view, const double* dXyz, size_t n, double* dOut, double* dGrad, cudaStream_t stream);
     // hpsdf_extract_isosurface (isosurface_kernels.cuh): a grid of (n0+1)(n1+1)(n2+1) < 2^32 points
     struct IsoGrid

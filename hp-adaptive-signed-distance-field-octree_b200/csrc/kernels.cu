@@ -24,6 +24,7 @@ namespace hpsdf
 #include "finish_kernels.cuh"
 #include "mesh_build.cuh"
 #include "isosurface_kernels.cuh"
+#include "raycast_kernels.cuh"
 
 namespace hpsdf
 {
@@ -51,6 +52,10 @@ namespace hpsdf
         cudaMemcpyToSymbol(c_isoTet, tet, sizeof(tet));
         cudaMemcpyToSymbol(c_isoChain, chain, sizeof(chain));
         cudaMemcpyToSymbol(c_isoCellTris, cellTris, sizeof(cellTris));
+        static double rayNodes[rayNodeOffset(kMaxDegree + 1)], rayBern[rayBernOffset(kMaxDegree + 1)];
+        rayBuildTables(rayNodes, rayBern);
+        cudaMemcpyToSymbol(c_rayNodes, rayNodes, sizeof(rayNodes));
+        cudaMemcpyToSymbol(c_rayBern, rayBern, sizeof(rayBern));
     }
 
     static const uint32_t* g_bidxDev[16] = { nullptr };
@@ -83,6 +88,20 @@ namespace hpsdf
     {
         if (!n) return cudaSuccess;
         queryRayKernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(view, dOrigins, dDirs, n, tMax, dHit, dT);
+        return cudaGetLastError();
+    }
+
+    cudaError_t launchRaycast(const DeviceTreeView& view, const double* dOrigins, const double* dDirs, size_t n, double tMin, double tMax,
+                              double iso, double* dT, double* dNormals, int smCount, cudaStream_t stream)
+    {
+        if (!n) return cudaSuccess;
+        const size_t groups = (n + 31) / 32;
+        size_t grid = (size_t)(smCount > 0 ? smCount : 148) * 2;
+        if (grid > (groups + 7) / 8) grid = (groups + 7) / 8;
+        int dev = 0;
+        cudaGetDevice(&dev);
+        raycastKernel<<<(unsigned)grid, kQueryThreads, 0, stream>>>(view, dOrigins, dDirs, n, RayArgs{ tMin, tMax, iso }, dT, dNormals,
+                                                                     g_bidxDev[dev & 15]);
         return cudaGetLastError();
     }
 

@@ -229,6 +229,22 @@ HPSDF_API hpsdf_status hpsdf_query_with_gradient(const hpsdf_octree* tree, const
 HPSDF_API hpsdf_status hpsdf_query_ray(const hpsdf_octree* tree, const double* origins, const double* directions, size_t n, double t_max,
                                        unsigned char* hit, double* t);
 
+/* First crossing of the level set F = iso along n rays x(t) = o + t*d, t in [t_min, t_max] (user space, d need not be
+ * unit; t is in units of d). F is the tree's own piecewise polynomial field: Query's leaves and coefficients, DBL_MAX
+ * outside the root box. t_hit[i] = the smallest t at which F <= iso, or +INFINITY for a miss. normals (may be NULL):
+ * the unit gradient of the hit leaf's polynomial at t_hit in user space, pointing to increasing F; (0,0,0) on a miss
+ * or a vanishing gradient. Each leaf's polynomial along the ray is solved exactly (DESIGN.md §12): no step size, no
+ * Lipschitz assumption, thin parts and jumps across leaf faces are found; any root box works. This, not
+ * hpsdf_query_ray (the reference's mirror), is the ray query to use.
+ * HPSDF_ERR_INVALID_ARG: null pointers when n > 0 (normals may be NULL), non-finite t_min or iso, t_max < t_min or NaN
+ * (t_max = +inf is allowed). A zero or non-finite direction or a non-finite origin is a miss. Blocks the calling thread. */
+HPSDF_API hpsdf_status hpsdf_raycast(const hpsdf_octree* tree, const double* origins, const double* directions, size_t n,
+                                     double t_min, double t_max, double iso, double* t_hit, double* normals);
+/* Same with DEVICE pointers, asynchronous on `stream`; the current device must be the tree's (as hpsdf_query_device). */
+HPSDF_API hpsdf_status hpsdf_raycast_device(const hpsdf_octree* tree, const double* d_origins, const double* d_directions,
+                                            size_t n, double t_min, double t_max, double iso, double* d_t_hit,
+                                            double* d_normals, void* stream);
+
 /* The level set F = iso of the tree as a triangle mesh: marching tetrahedra over a uniform grid of
  * resolution[0] x resolution[1] x resolution[2] cells spanning [box_min, box_max] (both NULL = the root box).
  * Grid values are Query values (DBL_MAX outside the root). Vertices: n_vertices x 3 float32, triangles:

@@ -5,7 +5,8 @@
 //     SDF::Octree                 Include/HP/Octree.h:36-86        Create / Query / QueryWithGradient / QueryRay / UnionSDF /
 //                                                                  SubtractSDF / IntersectSDF / Clear / FromMemoryBlock /
 //                                                                  ToMemoryBlock / GetRootAABB, copy + move; plus
-//                                                                  ExtractIsosurface (no counterpart in the reference)
+//                                                                  ExtractIsosurface / Raycast / RaycastDevice (no
+//                                                                  counterpart in the reference)
 //     MemoryBlock                 Include/Utility/MemoryBlock.h:5-9
 //
 // Differences, all forced by the device: (1) Create takes an SDF::Program (closed-form primitives / meshes / trees
@@ -216,6 +217,21 @@ namespace SDF
         void QueryRay(const double* origins_, const double* directions_, size_t n_, double tMax_, unsigned char* hit_, double* t_) const
         {
             check(hpsdf_query_ray(need(), origins_, directions_, n_, tMax_, hit_, t_));
+        }
+
+        /// First crossing of F = iso_ along n_ rays o + t d, t in [tMin_, tMax_] (hpsdf_raycast): tHit_ gets t or +INFINITY for a
+        /// miss, normals_ (3 per ray, may be nullptr) the unit gradient of the hit leaf's polynomial. The ray query to use.
+        void Raycast(const double* origins_, const double* directions_, size_t n_, double tMin_, double tMax_, double iso_, double* tHit_,
+                     double* normals_ = nullptr) const
+        {
+            check(hpsdf_raycast(need(), origins_, directions_, n_, tMin_, tMax_, iso_, tHit_, normals_));
+        }
+
+        /// Raycast with device pointers, asynchronous on stream_ (hpsdf_raycast_device).
+        void RaycastDevice(const double* dOrigins_, const double* dDirections_, size_t n_, double tMin_, double tMax_, double iso_,
+                           double* dTHit_, double* dNormals_, void* stream_) const
+        {
+            check(hpsdf_raycast_device(need(), dOrigins_, dDirections_, n_, tMin_, tMax_, iso_, dTHit_, dNormals_, stream_));
         }
 
         /// The level set F = iso_ as a triangle mesh (hpsdf_extract_isosurface): marching tetrahedra over resolution_ cells per axis
