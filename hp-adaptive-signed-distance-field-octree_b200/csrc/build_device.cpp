@@ -518,8 +518,7 @@ namespace hpsdf
             const double tFin0 = nowMs();
             HPSDF_CUDA(launchPadCoefficients(S, nN, w.cstartOf, w.padOf, t_.dCoeffs, t_.dCoeffsPad, stream_));
             HPSDF_CUDA(cudaMemcpyAsync(t_.dTop, w.tTop, 4096 * 4, cudaMemcpyDeviceToDevice, stream_));
-            t_.view.nodes = t_.dNodes; t_.view.coeffs = t_.dCoeffsPad; t_.view.top = t_.dTop; t_.view.map = t_.map; t_.view.nNodes = nN;
-            HPSDF_CUDA(cudaMemcpyAsync(t_.dView, &t_.view, sizeof(DeviceTreeView), cudaMemcpyHostToDevice, stream_));
+            HPSDF_CUDA(uploadTreeView(t_, t_.dTop, stream_));
             t_.stats.kernel_launches++;
             HPSDF_CUDA(cudaStreamSynchronize(stream_));
             t_.stats.finalize_ms = nowMs() - tFin0;

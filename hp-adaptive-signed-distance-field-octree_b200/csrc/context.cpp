@@ -7,8 +7,6 @@
 
 namespace hpsdf
 {
-    void setBidxDev(int device, const uint32_t* p);     // kernels.cu
-
     namespace
     {
         thread_local std::string g_lastError;
@@ -139,7 +137,6 @@ namespace hpsdf
         }
         ctx->fitTab.bidx = (const uint32_t*)(base + bidxOff);
         ctx->glRoots = base + glOff; ctx->glWeights = base + glOff + 2080;
-        setBidxDev(device, ctx->fitTab.bidx);
         cudaDeviceGetAttribute(&ctx->smCount, cudaDevAttrMultiProcessorCount, device);
         uploadConstants();
         ctx->wsMutex = new std::mutex();

@@ -217,6 +217,7 @@ namespace hpsdf
         const QNode*    nodes;
         const double*   coeffs;      // padded store: every leaf starts at an even index
         const uint32_t* top;         // 4096 entries: node reached at depth <= 4 for each cell of the 16^3 grid (x + 16 y + 256 z)
+        const uint32_t* bidx;        // BasisIndexValues of the tree's device (FitTablesDev::bidx)
         RootMap         map;
         uint32_t        nNodes;
     };

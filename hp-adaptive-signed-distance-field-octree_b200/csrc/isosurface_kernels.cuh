@@ -109,16 +109,10 @@ namespace hpsdf
     // A warp takes 32 consecutive points (mostly one x row, so neighbouring lanes mostly share a leaf); the coordinates are
     // made in registers. Persistent grid with the top table staged once per CTA, as queryKernel.
     __global__ void __launch_bounds__(kQueryThreads, kQueryBlocksPerSm)
-    isoGridKernel(const DeviceTreeView view, const IsoGrid g, double* __restrict__ vals, const uint32_t* __restrict__ bidx)
+    isoGridKernel(const DeviceTreeView view, const IsoGrid g, double* __restrict__ vals)
     {
         __shared__ uint32_t sTop[4096];
-        const bool useTop = view.top != nullptr;
-        if (useTop)
-        {
-            for (int i = threadIdx.x; i < 1024; i += kQueryThreads)
-                reinterpret_cast<uint4*>(sTop)[i] = __ldg(reinterpret_cast<const uint4*>(view.top) + i);
-            __syncthreads();
-        }
+        const bool useTop = stageTop(sTop, view.top);
         const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
         const uint32_t px = g.n[0] + 1, py = g.n[1] + 1, n = px * py * (g.n[2] + 1);
         const uint32_t nGroups = (n + 31) / 32, warpsTotal = gridDim.x * (kQueryThreads / 32);
@@ -126,13 +120,12 @@ namespace hpsdf
         {
             const uint32_t p = grp * 32 + lane;
             LeafHit h;
-            h.coeffs = view.coeffs; h.ux = h.uy = h.uz = 0.0; h.degree = -1; h.depth = 0;
             if (p < n)
             {
                 const uint32_t i = p % px, r = p / px, j = r % py, k = r / py;
-                h = findLeaf(view.nodes, view.coeffs, useTop ? sTop : nullptr, view.map, isoCoord(g, 0, i), isoCoord(g, 1, j), isoCoord(g, 2, k));
+                h = findLeaf(view, useTop ? sTop : nullptr, isoCoord(g, 0, i), isoCoord(g, 1, j), isoCoord(g, 2, k));
             }
-            const double v = evalWarp(h, bidx);
+            const double v = evalWarp(h, view.bidx);
             if (p < n) __stcs(vals + p, v);
         }
     }

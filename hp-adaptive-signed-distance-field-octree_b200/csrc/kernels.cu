@@ -58,28 +58,23 @@ namespace hpsdf
         cudaMemcpyToSymbol(c_rayBern, rayBern, sizeof(rayBern));
     }
 
-    static const uint32_t* g_bidxDev[16] = { nullptr };
-    void setBidxDev(int device, const uint32_t* p) { g_bidxDev[device & 15] = p; }
+    // Persistent grid of 256-thread CTAs: ctasPerSm on every SM, fewer when n items fill fewer CTAs
+    static unsigned persistentGrid(size_t n, int ctasPerSm, int smCount)
+    {
+        return (unsigned)std::min((size_t)(smCount > 0 ? smCount : 148) * ctasPerSm, (n + 255) / 256);
+    }
 
     cudaError_t launchQuery(const DeviceTreeView& view, const double* dXyz, size_t n, double* dOut, int smCount, cudaStream_t stream)
     {
         if (!n) return cudaSuccess;
-        const size_t tiles = (n + kQueryThreads - 1) / kQueryThreads;
-        // persistent grid: as many CTAs of 256 threads per SM as the register budget allows, fewer if the batch is small
-        size_t grid = (size_t)(smCount > 0 ? smCount : 148) * kQueryBlocksPerSm;
-        if (grid > tiles) grid = tiles;
-        int dev = 0;
-        cudaGetDevice(&dev);
-        queryKernel<<<(unsigned)grid, kQueryThreads, 0, stream>>>(view, dXyz, n, dOut, g_bidxDev[dev & 15], ((uintptr_t)dXyz & 15u) == 0 ? 1 : 0);
+        queryKernel<<<persistentGrid(n, kQueryBlocksPerSm, smCount), kQueryThreads, 0, stream>>>(view, dXyz, n, dOut, ((uintptr_t)dXyz & 15u) == 0 ? 1 : 0);
         return cudaGetLastError();
     }
 
     cudaError_t launchQueryGradient(const DeviceTreeView& view, const double* dXyz, size_t n, double* dOut, double* dGrad, cudaStream_t stream)
     {
         if (!n) return cudaSuccess;
-        int dev = 0;
-        cudaGetDevice(&dev);
-        queryGradientKernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(view, dXyz, n, dOut, dGrad, g_bidxDev[dev & 15]);
+        queryGradientKernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(view, dXyz, n, dOut, dGrad);
         return cudaGetLastError();
     }
 
@@ -95,13 +90,7 @@ namespace hpsdf
                               double iso, double* dT, double* dNormals, int smCount, cudaStream_t stream)
     {
         if (!n) return cudaSuccess;
-        const size_t groups = (n + 31) / 32;
-        size_t grid = (size_t)(smCount > 0 ? smCount : 148) * 2;
-        if (grid > (groups + 7) / 8) grid = (groups + 7) / 8;
-        int dev = 0;
-        cudaGetDevice(&dev);
-        raycastKernel<<<(unsigned)grid, kQueryThreads, 0, stream>>>(view, dOrigins, dDirs, n, RayArgs{ tMin, tMax, iso }, dT, dNormals,
-                                                                     g_bidxDev[dev & 15]);
+        raycastKernel<<<persistentGrid(n, 2, smCount), kQueryThreads, 0, stream>>>(view, dOrigins, dDirs, n, RayArgs{ tMin, tMax, iso }, dT, dNormals);
         return cudaGetLastError();
     }
 
@@ -548,12 +537,7 @@ namespace hpsdf
 
     cudaError_t launchIsoGrid(const DeviceTreeView& view, const IsoGrid& g, const IsoScratch& s, int smCount, cudaStream_t stream)
     {
-        const size_t groups = ((size_t)isoPoints(g) + 31) / 32;
-        size_t grid = (size_t)(smCount > 0 ? smCount : 148) * kQueryBlocksPerSm;
-        if (grid > (groups + 7) / 8) grid = (groups + 7) / 8;
-        int dev = 0;
-        cudaGetDevice(&dev);
-        isoGridKernel<<<(unsigned)grid, kQueryThreads, 0, stream>>>(view, g, s.vals, g_bidxDev[dev & 15]);
+        isoGridKernel<<<persistentGrid(isoPoints(g), kQueryBlocksPerSm, smCount), kQueryThreads, 0, stream>>>(view, g, s.vals);
         return cudaGetLastError();
     }
 
@@ -562,9 +546,7 @@ namespace hpsdf
         const uint32_t n = isoPoints(g);
         cudaError_t e = cudaMemsetAsync(s.totals, 0, 16, stream);
         if (e != cudaSuccess) return e;
-        size_t grid = (size_t)(smCount > 0 ? smCount : 148) * 8;
-        if (grid > ((size_t)n + 255) / 256) grid = ((size_t)n + 255) / 256;
-        isoCountKernel<<<(unsigned)grid, 256, 0, stream>>>(g, s.vals, s.mask, s.label, s.totals);
+        isoCountKernel<<<persistentGrid(n, 8, smCount), 256, 0, stream>>>(g, s.vals, s.mask, s.label, s.totals);
         if ((e = cudaGetLastError()) != cudaSuccess) return e;
         size_t tb = s.cubTmpBytes;
         e = cub::DeviceScan::ExclusiveSum(s.cubTmp, tb, IsoVertexCounts(s.mask, IsoPopc()), s.vbase, (int)n, stream);

@@ -95,6 +95,8 @@ namespace hpsdf
     void          ensureApplyLog(hpsdf_octree& t);
     // Build QNodes, the padded coefficient store and the top table from nodes + dCoeffs.
     hpsdf_status  finalizeQueryStructures(hpsdf_octree& t, cudaStream_t stream);
+    // Fill t.view from the tree's device arrays (top: the depth-4 table, or nullptr) and copy it to t.dView on `stream`.
+    cudaError_t   uploadTreeView(hpsdf_octree& t, const uint32_t* top, cudaStream_t stream);
     // SDF program with handles resolved to device views; fails on malformed programs.
     hpsdf_status  resolveProgram(const hpsdf_sdf_program* prog, int device, SdfProgramDev& out);
     // Octree::Create on the device (build.cpp)

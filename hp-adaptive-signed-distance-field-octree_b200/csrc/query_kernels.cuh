@@ -16,19 +16,26 @@ namespace hpsdf
 #endif
     constexpr int kQueryBlocksPerSm = HPSDF_QUERY_MINBLOCKS;
 
+    // Stage the 4096-entry top table of the tree into shared memory once per CTA of a persistent kernel (all threads must
+    // call this); false when the tree has none. The only block-wide barrier: the table is read-only afterwards. Callers
+    // pick sTop or nullptr where they descend: a returned table pointer stays live across their loops and made queryKernel
+    // and isoGridKernel spill more.
+    __device__ __forceinline__ bool stageTop(uint32_t (&sTop)[4096], const uint32_t* top)
+    {
+        if (!top) return false;
+        for (int i = threadIdx.x; i < 1024; i += kQueryThreads)
+            reinterpret_cast<uint4*>(sTop)[i] = __ldg(reinterpret_cast<const uint4*>(top) + i);
+        __syncthreads();
+        return true;
+    }
+
     __global__ void __launch_bounds__(kQueryThreads, kQueryBlocksPerSm)
     queryKernel(const DeviceTreeView view, const double* __restrict__ xyz, size_t n, double* __restrict__ out,
-                const uint32_t* __restrict__ bidx, const int aligned /* xyz starts on a 16-byte boundary */)
+                const int aligned /* xyz starts on a 16-byte boundary */)
     {
         __shared__ uint32_t sTop[4096];
         __shared__ __align__(16) double sPts[kQueryThreads / 32][96];          // per warp: 32 points x 3 doubles
-        const bool useTop = view.top != nullptr;
-        if (useTop)
-        {
-            for (int i = threadIdx.x; i < 1024; i += kQueryThreads)
-                reinterpret_cast<uint4*>(sTop)[i] = __ldg(reinterpret_cast<const uint4*>(view.top) + i);
-            __syncthreads();                        // the only block-wide barrier: the table is read-only afterwards
-        }
+        const bool useTop = stageTop(sTop, view.top);
         const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
         const size_t nGroups = (n + 31) / 32;                                   // a warp handles 32 consecutive points
         const size_t warpsTotal = (size_t)gridDim.x * (kQueryThreads / 32);
@@ -47,10 +54,9 @@ namespace hpsdf
                 for (size_t v = lane; v < 3 * cnt; v += 32) sp[v] = src[v];
             __syncwarp();
             LeafHit h;
-            h.coeffs = view.coeffs; h.ux = h.uy = h.uz = 0.0; h.degree = -1; h.depth = 0;
-            if ((size_t)lane < cnt) h = findLeaf(view.nodes, view.coeffs, useTop ? sTop : nullptr, view.map, sp[3 * lane], sp[3 * lane + 1], sp[3 * lane + 2]);
+            if ((size_t)lane < cnt) h = findLeaf(view, useTop ? sTop : nullptr, sp[3 * lane], sp[3 * lane + 1], sp[3 * lane + 2]);
             __syncwarp();                           // sp is overwritten by the next group
-            const double v = evalWarp(h, bidx);
+            const double v = evalWarp(h, view.bidx);
             if ((size_t)lane < cnt) __stcs(out + base + lane, v);
         }
     }
@@ -59,34 +65,20 @@ namespace hpsdf
     // in the leaf's local coordinate, gradient normalised. One thread per point, generic-degree loops (not a hot path).
     __global__ void __launch_bounds__(256)
     queryGradientKernel(const DeviceTreeView view, const double* __restrict__ xyz, size_t n, double* __restrict__ out,
-                        double* __restrict__ grad, const uint32_t* __restrict__ bidx)
+                        double* __restrict__ grad)
     {
         const size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
         if (t >= n) return;
-        const RootMap& map = view.map;
-        const double px = (xyz[3 * t] - map.centre[0]) * map.invSizes[0];
-        const double py = (xyz[3 * t + 1] - map.centre[1]) * map.invSizes[1];
-        const double pz = (xyz[3 * t + 2] - map.centre[2]) * map.invSizes[2];
-        const float fx = (float)px, fy = (float)py, fz = (float)pz;
-        if (!(fx >= -0.5f && fx <= 0.5f && fy >= -0.5f && fy <= 0.5f && fz >= -0.5f && fz <= 0.5f)) { out[t] = DBL_MAX; return; }
-        double c[3] = { 0.0, 0.0, 0.0 }, q = 0.25;
-        const double p[3] = { px, py, pz };
-        uint4 raw = __ldg(reinterpret_cast<const uint4*>(view.nodes));
-        while (raw.z == kInternalTag)
-        {
-            uint32_t b[3];
-            for (int a = 0; a < 3; ++a) { b[a] = p[a] >= c[a]; c[a] += b[a] ? q : -q; }
-            q *= 0.5;
-            raw = __ldg(reinterpret_cast<const uint4*>(view.nodes) + raw.x + b[0] + (b[1] << 1) + (b[2] << 2));
-        }
-        const int depth = (int)raw.w, degree = (int)raw.z;
-        const double* coeffs = view.coeffs + raw.y;
-        const double scale = (double)(2u << depth), eps = 0.0001;
+        const LeafHit h = findLeaf(view, view.top, xyz[3 * t], xyz[3 * t + 1], xyz[3 * t + 2]);
+        if (h.degree < 0) { out[t] = DBL_MAX; return; }
+        const int depth = h.depth, degree = h.degree;
+        const double* coeffs = h.coeffs;
+        const uint32_t* bidx = view.bidx;
+        const double eps = 0.0001, u[3] = { h.ux, h.uy, h.uz };
         double lut[kMaxDegree + 1][3][3];
         for (int a = 0; a < 3; ++a)
         {
-            const double u = (p[a] - c[a]) * scale;
-            const double us[3] = { u, u + eps, u - eps };
+            const double us[3] = { u[a], u[a] + eps, u[a] - eps };
             for (int v = 0; v < 3; ++v)
             {
                 lut[0][a][v] = c_nl[0][depth];
@@ -189,7 +181,7 @@ namespace hpsdf
             double d = 0.0;
             for (unsigned s = 0; s < MAX_STEPS; ++s)
             {
-                const double v = queryPoint(view.nodes, view.coeffs, view.top, map, intMin[0] + d * dir[0], intMin[1] + d * dir[1], intMin[2] + d * dir[2]);
+                const double v = treeQuery(view, intMin[0] + d * dir[0], intMin[1] + d * dir[1], intMin[2] + d * dir[2]);
                 if (v < eps) { t = v; h = 1; break; }                                           // :731-736
                 d += v * 0.95 + minStep;                                                        // :739
                 if (d > tMax) break;                                                            // :741-744

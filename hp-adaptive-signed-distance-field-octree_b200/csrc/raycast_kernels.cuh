@@ -233,16 +233,10 @@ namespace hpsdf
     // One ray per lane, a warp per 32 consecutive rays, persistent grid. The top table is staged as in queryKernel.
     __global__ void __launch_bounds__(kQueryThreads, 2)
     raycastKernel(const DeviceTreeView view, const double* __restrict__ origins, const double* __restrict__ dirs, size_t n,
-                  const RayArgs args, double* __restrict__ tHit, double* __restrict__ normals, const uint32_t* __restrict__ bidx)
+                  const RayArgs args, double* __restrict__ tHit, double* __restrict__ normals)
     {
         __shared__ uint32_t sTop[4096];
-        const bool useTop = view.top != nullptr;
-        if (useTop)
-        {
-            for (int i = threadIdx.x; i < 1024; i += kQueryThreads)
-                reinterpret_cast<uint4*>(sTop)[i] = __ldg(reinterpret_cast<const uint4*>(view.top) + i);
-            __syncthreads();
-        }
+        const bool useTop = stageTop(sTop, view.top);
         const RootMap& map = view.map;
         const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
         const size_t nGroups = (n + 31) / 32, warpsTotal = (size_t)gridDim.x * (kQueryThreads / 32);
@@ -329,19 +323,19 @@ namespace hpsdf
                 double tau;
                 switch (m)
                 {
-                    case 0:  tau = rayLeafFirstCrossing<0>(coeffs, degree, depth, ua, ub, args.iso, pointOnly, bidx); break;
-                    case 1:  tau = rayLeafFirstCrossing<1>(coeffs, degree, depth, ua, ub, args.iso, pointOnly, bidx); break;
-                    case 2:  tau = rayLeafFirstCrossing<2>(coeffs, degree, depth, ua, ub, args.iso, pointOnly, bidx); break;
-                    case 3:  tau = rayLeafFirstCrossing<3>(coeffs, degree, depth, ua, ub, args.iso, pointOnly, bidx); break;
-                    case 4:  tau = rayLeafFirstCrossing<4>(coeffs, degree, depth, ua, ub, args.iso, pointOnly, bidx); break;
-                    case 5:  tau = rayLeafFirstCrossing<5>(coeffs, degree, depth, ua, ub, args.iso, pointOnly, bidx); break;
-                    case 6:  tau = rayLeafFirstCrossing<6>(coeffs, degree, depth, ua, ub, args.iso, pointOnly, bidx); break;
-                    case 7:  tau = rayLeafFirstCrossingHigh<7>(coeffs, degree, depth, ua, ub, args.iso, pointOnly, bidx); break;
-                    case 8:  tau = rayLeafFirstCrossingHigh<8>(coeffs, degree, depth, ua, ub, args.iso, pointOnly, bidx); break;
-                    case 9:  tau = rayLeafFirstCrossingHigh<9>(coeffs, degree, depth, ua, ub, args.iso, pointOnly, bidx); break;
-                    case 10: tau = rayLeafFirstCrossingHigh<10>(coeffs, degree, depth, ua, ub, args.iso, pointOnly, bidx); break;
-                    case 11: tau = rayLeafFirstCrossingHigh<11>(coeffs, degree, depth, ua, ub, args.iso, pointOnly, bidx); break;
-                    default: tau = rayLeafFirstCrossingHigh<12>(coeffs, degree, depth, ua, ub, args.iso, pointOnly, bidx); break;
+                    case 0:  tau = rayLeafFirstCrossing<0>(coeffs, degree, depth, ua, ub, args.iso, pointOnly, view.bidx); break;
+                    case 1:  tau = rayLeafFirstCrossing<1>(coeffs, degree, depth, ua, ub, args.iso, pointOnly, view.bidx); break;
+                    case 2:  tau = rayLeafFirstCrossing<2>(coeffs, degree, depth, ua, ub, args.iso, pointOnly, view.bidx); break;
+                    case 3:  tau = rayLeafFirstCrossing<3>(coeffs, degree, depth, ua, ub, args.iso, pointOnly, view.bidx); break;
+                    case 4:  tau = rayLeafFirstCrossing<4>(coeffs, degree, depth, ua, ub, args.iso, pointOnly, view.bidx); break;
+                    case 5:  tau = rayLeafFirstCrossing<5>(coeffs, degree, depth, ua, ub, args.iso, pointOnly, view.bidx); break;
+                    case 6:  tau = rayLeafFirstCrossing<6>(coeffs, degree, depth, ua, ub, args.iso, pointOnly, view.bidx); break;
+                    case 7:  tau = rayLeafFirstCrossingHigh<7>(coeffs, degree, depth, ua, ub, args.iso, pointOnly, view.bidx); break;
+                    case 8:  tau = rayLeafFirstCrossingHigh<8>(coeffs, degree, depth, ua, ub, args.iso, pointOnly, view.bidx); break;
+                    case 9:  tau = rayLeafFirstCrossingHigh<9>(coeffs, degree, depth, ua, ub, args.iso, pointOnly, view.bidx); break;
+                    case 10: tau = rayLeafFirstCrossingHigh<10>(coeffs, degree, depth, ua, ub, args.iso, pointOnly, view.bidx); break;
+                    case 11: tau = rayLeafFirstCrossingHigh<11>(coeffs, degree, depth, ua, ub, args.iso, pointOnly, view.bidx); break;
+                    default: tau = rayLeafFirstCrossingHigh<12>(coeffs, degree, depth, ua, ub, args.iso, pointOnly, view.bidx); break;
                 }
                 if (!active) continue;
                 if (tau >= 0.0)
@@ -370,7 +364,7 @@ namespace hpsdf
                 if (normals)
                 {
                     double nv[3] = { 0.0, 0.0, 0.0 };
-                    if (hitCoeffs) rayNormal(hitCoeffs, hitDeg, hitDepth, hitU, map, bidx, nv);
+                    if (hitCoeffs) rayNormal(hitCoeffs, hitDeg, hitDepth, hitU, map, view.bidx, nv);
                     for (int a = 0; a < 3; ++a) normals[3 * ray + a] = nv[a];
                 }
             }

@@ -107,10 +107,16 @@ namespace hpsdf
         HPSDF_CUDA(cudaMemsetAsync(t.dCoeffsPad, 0, std::max<size_t>(padCur, 2) * 8, stream));
         HPSDF_CUDA(launchGatherSegments(t.dCoeffs, t.dCoeffsPad, ws.segs.p, ws.segs.p + nLeaves, ws.segs.p + 2 * nLeaves, (uint32_t)nLeaves, stream));
         t.stats.kernel_launches++;
-        t.view.nodes = t.dNodes; t.view.coeffs = t.dCoeffsPad; t.view.top = topOk ? t.dTop : nullptr; t.view.map = t.map; t.view.nNodes = (uint32_t)nNodes;
-        HPSDF_CUDA(cudaMemcpyAsync(t.dView, &t.view, sizeof(DeviceTreeView), cudaMemcpyHostToDevice, stream));
+        HPSDF_CUDA(uploadTreeView(t, topOk ? t.dTop : nullptr, stream));
         HPSDF_CUDA(cudaStreamSynchronize(stream));
         return HPSDF_OK;
+    }
+
+    cudaError_t uploadTreeView(hpsdf_octree& t, const uint32_t* top, cudaStream_t stream)
+    {
+        t.view.nodes = t.dNodes; t.view.coeffs = t.dCoeffsPad; t.view.top = top; t.view.bidx = t.ctx->fitTab.bidx;
+        t.view.map = t.map; t.view.nNodes = (uint32_t)t.nNodes;
+        return cudaMemcpyAsync(t.dView, &t.view, sizeof(DeviceTreeView), cudaMemcpyHostToDevice, stream);
     }
 
     hpsdf_status resolveProgram(const hpsdf_sdf_program* prog, int device, SdfProgramDev& out)
