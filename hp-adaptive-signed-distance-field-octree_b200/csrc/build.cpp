@@ -40,6 +40,9 @@ namespace hpsdf
             double   hErr[8] = { 0 }, pErr = 0.0, hImp = 0.0, pImp = 0.0;
         };
 
+        // JobDesc slots behind a round's job records that carry its RoundLayout to the device in the same copy
+        constexpr size_t kLayoutSlots = (sizeof(RoundLayout) + sizeof(JobDesc) - 1) / sizeof(JobDesc);
+
         // Octree.h:95-102: max-heap on the error only
         struct QueuePredicate
         {
@@ -121,10 +124,9 @@ namespace hpsdf
             long double exactSum_ = 0.0L;
             long        unfitted_ = 0;
             int         rank_ = 0, world_ = 1;
-            double      sdfFlops_ = 0.0;
             double      launchMs_ = 0.0;           // host time spent in upload / launch calls (diagnostics)
             size_t      strictSteps_ = 0, levelCalls_ = 0;   // diagnostics: strictly sequential pops; guaranteed-level computations
-            bool        progHasExt_ = false;       // the program samples a mesh or another octree
+            ProgramSummary progSummary_;
             hpsdf_decision_log_entry lastApplied_{};      // last job applied before the termination cut
             double      lastTotal_ = 0.0, totalBeforeLast_ = 0.0;
 
@@ -224,13 +226,13 @@ namespace hpsdf
             // pass A: select, create the jobs, count fits per degree
             const size_t firstJob = jobs_.size();
             evaluated_.clear();
-            size_t cnt[kMaxDegree + 2] = { 0 };
+            uint32_t cnt[kMaxDegree + 2] = { 0 };
             // Everything at or above the level is needed work. If that is only a handful of jobs the round would cost a full
             // upload / launch / synchronise / replay cycle for them (10 of the 18 rounds of a C2 build selected fewer than 20
             // jobs), so the round is topped up to `min_round_jobs` with the next-largest pending errors: the greedy loop is
             // about to reach them anyway and their results stay cached until it does.
             // (not for mesh / octree programs by default: there a fit costs 10^3-10^4 BVH queries and speculation measured 25-35 % slower)
-            const size_t minJobs = o_.min_round_jobs ? o_.min_round_jobs : (progHasExt_ ? 1u : 512u);
+            const size_t minJobs = o_.min_round_jobs ? o_.min_round_jobs : (progSummary_.samplesExt ? 1u : 512u);
             const size_t pendBefore = pendCount_;
             auto select = [&](uint64_t idx) { evaluated_.push_back(idx); };
             const int levelBucket = bucketOf(level);
@@ -253,14 +255,12 @@ namespace hpsdf
             }
             while (pendTop_ > 0 && pendB_[pendTop_].empty()) --pendTop_;
             if (pendCount_) for (uint64_t idx : pendB_[pendTop_]) pendingMax_ = std::max(pendingMax_, errOf_[idx]);
-            // Several GPUs evaluate contiguous shards of each degree group. Selection order is spatially coherent (far and near
-            // cells of a mesh cluster, and their fits differ 10x in cost), so the jobs of a round are dealt out by a fixed
-            // stride permutation first: every shard gets the same mix. (Only node numbering depends on the order.)
+            // several GPUs: every shard of a degree group gets the same mix of jobs (dealStride; only node numbering depends on
+            // the order)
             if (world_ > 1 && evaluated_.size() > 2)
             {
                 const size_t n = evaluated_.size();
-                size_t stride = 7919;
-                for (const size_t cand : { (size_t)7919, (size_t)7907, (size_t)7901, (size_t)7883 }) if (n % cand != 0) { stride = cand; break; }
+                const size_t stride = dealStride((uint32_t)n);
                 std::vector<uint64_t> perm(n);
                 for (size_t k = 0; k < n; ++k) perm[k] = evaluated_[(k * stride) % n];
                 evaluated_.swap(perm);
@@ -285,35 +285,28 @@ namespace hpsdf
             if (dbgRounds) fprintf(stderr, "round %llu: pending %zu -> %zu, jobs %zu, heap %zu, level %.3e, passA %.3f ms\n", (unsigned long long)t_.stats.rounds,
                                    pendBefore, pendCount_, evaluated_.size(), queue_.entries().size(), level, nowMs() - tTask0);
 
-            // Tasks in degree order; task index == record index; slots allocated in task order (contiguous per degree,
-            // so a rank's shard of a degree group is one contiguous pool range).
-            size_t nTasks = 0, poolNeed = poolUsed_;
-            size_t groupBegin[kMaxDegree + 2] = { 0 }, groupPool[kMaxDegree + 2] = { 0 }, cursor[kMaxDegree + 2] = { 0 };
-            for (int d = 1; d <= kMaxDegree; ++d)
-            {
-                groupBegin[d] = cursor[d] = nTasks; groupPool[d] = poolNeed;
-                nTasks += cnt[d]; poolNeed += cnt[d] * (size_t)coeffCount(d);
-            }
-            groupBegin[kMaxDegree + 1] = nTasks;
+            // task index == record index
+            RoundLayout lay;
+            uint64_t poolNeed = 0;
+            const uint32_t nTasks = layoutRound(cnt, (uint32_t)poolUsed_, lay.groupBegin, lay.groupPool, poolNeed);
             if (poolNeed >= 0xFFFFFFF0ull) { setLastError("coefficient pool exceeds 2^32 doubles"); return HPSDF_ERR_OOM; }
+            const size_t nJobs = evaluated_.size();
+            HPSDF_CUDA(hJobs_.reserve(nJobs + kLayoutSlots));       // (pass B writes the records of a round without fits too)
             if (nTasks)
             {
                 HPSDF_CUDA(pool_.reserve(poolNeed + 1024, stream_, poolUsed_));
                 HPSDF_CUDA(dTasks_.reserve(nTasks));
                 HPSDF_CUDA(dRecs_.reserve(nTasks));
                 HPSDF_CUDA(hRecs_.reserve(nTasks));
-                HPSDF_CUDA(dJobs_.reserve(evaluated_.size()));
-                HPSDF_CUDA(hJobs_.reserve(evaluated_.size()));
+                HPSDF_CUDA(dJobs_.reserve(nJobs + kLayoutSlots));
             }
-            // pass B: one 32-byte job record per job straight into pinned memory; expandJobsKernel derives the fit tasks on
+            // pass B: one 32-byte job record per job straight into pinned memory; expandJobsDevKernel derives the fit tasks on
             // the device (the host used to write all 9 descriptors of a job: 75 k x 32 B per C2 build, a quarter of its time).
-            // Task index == record index; slots are allocated in task order (contiguous per degree, so a rank's shard of a
-            // degree group is one contiguous pool range).
-            RoundLayout lay;
-            for (int d = 0; d <= kMaxDegree + 1; ++d) { lay.groupBegin[d] = (uint32_t)groupBegin[d]; lay.groupPool[d] = (uint32_t)groupPool[d]; }
-            auto slotOf = [&](int d, size_t pos) { return (uint32_t)(groupPool[d] + (pos - groupBegin[d]) * (size_t)coeffCount(d)); };
+            uint32_t cursor[kMaxDegree + 2];
+            for (int d = 0; d <= kMaxDegree + 1; ++d) cursor[d] = lay.groupBegin[d];
+            auto slotOf = [&](int d, uint32_t pos) { return lay.groupPool[d] + (pos - lay.groupBegin[d]) * (uint32_t)coeffCount(d); };
             JobDesc* J = hJobs_.p;
-            for (size_t k = 0; k < evaluated_.size(); ++k)
+            for (size_t k = 0; k < nJobs; ++k)
             {
                 const uint64_t idx = evaluated_[k];
                 const HostNode& n = nodes_[idx];
@@ -325,100 +318,36 @@ namespace hpsdf
                 if (j.coarse)                                                                    // Octree.cpp:840
                 {
                     o.flags = 4u;
-                    j.pPos = o.pPos = (uint32_t)cursor[kCoarseDegree]++;
+                    j.pPos = o.pPos = cursor[kCoarseDegree]++;
                     j.pSlot = slotOf(kCoarseDegree, j.pPos);
                     continue;
                 }
                 o.flags = (j.doH ? 1u : 0u) | (j.doP ? 2u : 0u);
                 if (j.doH)                                                                       // Octree.cpp:820
                 {
-                    j.hPos = o.hPos = (uint32_t)cursor[n.degree];
+                    j.hPos = o.hPos = cursor[n.degree];
                     cursor[n.degree] += 8;
                     j.hSlot0 = slotOf(n.degree, j.hPos);
                 }
                 if (j.doP)                                                                       // Octree.cpp:846-851
                 {
-                    j.pPos = o.pPos = (uint32_t)cursor[n.degree + 1]++;
+                    j.pPos = o.pPos = cursor[n.degree + 1]++;
                     j.pSlot = slotOf(n.degree + 1, j.pPos);
                 }
             }
             poolUsed_ = poolNeed;
-            double roundFlops = 0.0; uint64_t roundEvals = 0;
             t_.stats.host_tasks_ms += nowMs() - tTask0;
 
-            // ---- 2. upload, launch one kernel per degree present (this rank's shard), gather across ranks ----------
-            // Sharding a round costs one grouped broadcast per (degree group, rank) and its latency. It pays when fits are
-            // expensive (mesh / octree programs: 10^3-10^4 BVH queries each) or the round is large; a small round of closed-form
-            // fits (tens of microseconds of kernel time) is cheaper to evaluate redundantly on every rank — identical
-            // kernels on identical hardware give identical bits, so the replicas stay in lock-step without an exchange.
-            const bool shard = world_ > 1 && (progHasExt_ || nTasks >= (size_t)1 << 18);
+            // ---- 2. upload the job records with the layout behind them, expand, launch, read the fit records back ------------
             const double tLaunch0 = nowMs();
             if (nTasks)
             {
-                HPSDF_CUDA(cudaMemcpyAsync(dJobs_.p, hJobs_.p, evaluated_.size() * sizeof(JobDesc), cudaMemcpyHostToDevice, stream_));
-                HPSDF_CUDA(launchExpandJobs(dJobs_.p, (uint32_t)evaluated_.size(), lay, dTasks_.p, stream_));
+                memcpy(hJobs_.p + nJobs, &lay, sizeof(lay));
+                HPSDF_CUDA(cudaMemcpyAsync(dJobs_.p, hJobs_.p, nJobs * sizeof(JobDesc) + sizeof(lay), cudaMemcpyHostToDevice, stream_));
+                HPSDF_CUDA(launchExpandJobsDev(dJobs_.p, (uint32_t)nJobs, (const RoundLayout*)(dJobs_.p + nJobs), dTasks_.p, stream_));
                 t_.stats.kernel_launches++;
-                HPSDF_CUDA(cudaEventRecord(ev0_, stream_));
-                // The launches of a round (one per degree present) are independent and individually too small to fill 148 SMs:
-                // closed-form programs fan them out over four auxiliary streams and join again (mesh / octree programs share
-                // one sample scratch buffer and stay on the build stream).
-                int groups = 0;
-                for (int d = 1; d <= kMaxDegree; ++d) groups += cnt[d] != 0;
-                const bool fan = !progHasExt_ && groups > 1;
-                if (fan) HPSDF_CUDA(cudaEventRecord(ws_.evFork, stream_));
-                int g = 0;
-                bool used[4] = { false, false, false, false };
-                for (int d = kMaxDegree; d >= 1; --d)                 // highest degree first: the longest kernels start earliest
-                {
-                    const size_t n = cnt[d];
-                    if (!n) continue;
-                    size_t b = 0, e = n;
-                    if (shard) hpsdf_shard_range(n, rank_, world_, &b, &e);
-                    if (e > b)
-                    {
-                        cudaStream_t s = stream_;
-                        if (fan)
-                        {
-                            s = ws_.aux[g & 3];
-                            if (!used[g & 3]) { HPSDF_CUDA(cudaStreamWaitEvent(s, ws_.evFork, 0)); used[g & 3] = true; }
-                            ++g;
-                        }
-                        const hpsdf_status ls = launchFit(o_.jit, d, dTasks_.p + groupBegin[d] + b, (int)(e - b), pool_.p, dRecs_.p, prog_, t_.map, *t_.ctx, s);
-                        if (ls != HPSDF_OK) return ls;
-                        t_.stats.kernel_launches++;
-                    }
-                    t_.stats.fits_evaluated += n;
-                    roundFlops += (double)n * (fitFlops(d) + sdfFlops_ * fitRule(d) * fitRule(d) * fitRule(d));
-                    roundEvals += (uint64_t)n * fitRule(d) * fitRule(d) * fitRule(d);
-                }
-                if (fan)
-                    for (int i = 0; i < 4; ++i)
-                        if (used[i])
-                        {
-                            HPSDF_CUDA(cudaEventRecord(ws_.evJoin[i], ws_.aux[i]));
-                            HPSDF_CUDA(cudaStreamWaitEvent(stream_, ws_.evJoin[i], 0));
-                        }
-                HPSDF_CUDA(cudaEventRecord(ev1_, stream_));
-                if (shard)
-                {
-                    // every rank receives every other rank's shard: coefficients and records (replicated pool, identical replay)
-                    std::vector<CommSegment> segs;
-                    for (int d = 1; d <= kMaxDegree; ++d)
-                    {
-                        const size_t n = cnt[d];
-                        if (!n) continue;
-                        for (int r = 0; r < world_; ++r)
-                        {
-                            size_t b, e;
-                            hpsdf_shard_range(n, r, world_, &b, &e);
-                            if (e <= b) continue;
-                            segs.push_back({ pool_.p + groupPool[d] + b * (size_t)coeffCount(d), (e - b) * (size_t)coeffCount(d), r });
-                            segs.push_back({ (double*)(dRecs_.p + groupBegin[d] + b), (e - b) * 2, r });
-                        }
-                    }
-                    hpsdf_status cs = commBroadcastSegments(o_.comm, segs, stream_);
-                    if (cs != HPSDF_OK) return cs;
-                }
+                const hpsdf_status ls = launchRoundFits(t_, o_, prog_, progSummary_, stream_, cnt, lay, nTasks, rank_, world_, ev0_, ev1_);
+                if (ls != HPSDF_OK) return ls;
                 HPSDF_CUDA(cudaMemcpyAsync(hRecs_.p, dRecs_.p, nTasks * sizeof(FitRecord), cudaMemcpyDeviceToHost, stream_));
                 const double tWait0 = nowMs();
                 launchMs_ += tWait0 - tLaunch0;
@@ -427,9 +356,6 @@ namespace hpsdf
                 float ms = 0.0f;
                 cudaEventElapsedTime(&ms, ev0_, ev1_);
                 t_.stats.fit_kernel_ms += ms;
-                t_.stats.algorithmic_flops += roundFlops;
-                t_.stats.sdf_evals += roundEvals;
-                t_.stats.rounds++;
             }
             t_.stats.jobs_evaluated += jobs_.size() - firstJob;
 
@@ -437,7 +363,7 @@ namespace hpsdf
             const double tRec0 = nowMs();
             const bool weighted = cfg_.nearness_type != HPSDF_NEARNESS_NONE;
             const FitRecord* R = hRecs_.p;
-            for (size_t k = 0; k < evaluated_.size() && nTasks; ++k)
+            for (size_t k = 0; k < nJobs && nTasks; ++k)
             {
                 Job& j = jobs_[firstJob + k];
                 const uint32_t depth = nodes_[evaluated_[k]].depth;
@@ -694,13 +620,8 @@ namespace hpsdf
             stream_ = o_.stream ? (cudaStream_t)o_.stream : ws_.stream;
             ev0_ = ws_.ev0; ev1_ = ws_.ev1;
             if (o_.comm) { rank_ = commRank(o_.comm); world_ = commWorld(o_.comm); }
-            sdfFlops_ = 6.0;
-            for (uint32_t i = 0; i < prog_.n; ++i)
-            {
-                sdfFlops_ += sdfOpFlops(prog_.instr[i].op);
-                progHasExt_ |= prog_.instr[i].op == HPSDF_PRIM_MESH || prog_.instr[i].op == HPSDF_PRIM_OCTREE;
-            }
-            t_.stats.sdf_flops_per_eval = sdfFlops_;
+            progSummary_ = summarizeProgram(prog_);
+            t_.stats.sdf_flops_per_eval = progSummary_.flopsPerEval;
 
             hpsdf_status st = HPSDF_OK;
             const double tSetup0 = nowMs();

@@ -1,11 +1,106 @@
-// build_common.cpp — ReallocCoeffs and the cut-tie log, shared by the two schedulers of Octree::Create.
+// build_common.cpp — round launches, ReallocCoeffs and the cut-tie log, shared by the two schedulers of Octree::Create.
 #include <algorithm>
 #include <cmath>
+#include <cstdlib>
 #include <cstring>
 #include "build_common.h"
+#include "comm.h"
 
 namespace hpsdf
 {
+    hpsdf_status launchRoundFits(hpsdf_octree& t, const hpsdf_build_opts& o, const SdfProgramDev& prog, const ProgramSummary& ps,
+                                 cudaStream_t stream, const uint32_t* cnt, const RoundLayout& lay, uint32_t nTasks, int rank, int world,
+                                 cudaEvent_t evBegin, cudaEvent_t evEnd)
+    {
+        BuildWorkspace& ws = t.ctx->ws;
+        // Sharding a round costs one grouped broadcast per (degree group, rank) and its latency. It pays when fits are
+        // expensive (mesh / octree programs: 10^3-10^4 BVH queries each) or the round is large; a small round of closed-form
+        // fits (tens of microseconds of kernel time) is cheaper to evaluate redundantly on every rank — identical kernels on
+        // identical hardware give identical bits, so the replicas stay in lock-step without an exchange.
+        const bool shard = world > 1 && (ps.samplesExt || nTasks >= (1u << 18));
+        HPSDF_CUDA(cudaEventRecord(evBegin, stream));
+        int groups = 0;
+        for (int d = 1; d <= kMaxDegree; ++d) groups += cnt[d] != 0;
+        // The launches of a round (one per degree present) are independent: they fan out over four auxiliary streams and join
+        // again. Mesh / octree programs sample into a scratch buffer: their groups run concurrently when every group gets its own
+        // slice of it (a mesh query is a chain of ~50-300 dependent L2 round trips, so a launch lasts at least 0.1-0.4 ms however
+        // few samples it has: back to back, the groups of a small round — all of them, on 8 GPUs — just queue those latencies up).
+        size_t slice[kMaxDegree + 2] = { 0 }, sliceOff[kMaxDegree + 2] = { 0 }, sliceTotal = 0;
+        if (ps.samplesExt && groups > 1)
+            for (int d = 1; d <= kMaxDegree; ++d)
+            {
+                size_t b = 0, e = cnt[d];
+                if (shard) hpsdf_shard_range(cnt[d], rank, world, &b, &e);
+                slice[d] = (e - b) * (size_t)fitRule(d) * fitRule(d) * fitRule(d);
+                sliceOff[d] = sliceTotal;
+                sliceTotal += (slice[d] + 31) & ~(size_t)31;
+            }
+        const bool sliced = ps.samplesExt && groups > 1 && sliceTotal <= ((size_t)1 << 28) && !getenv("HPSDF_SAMPLE_CAP");
+        if (sliced) HPSDF_CUDA(reserveSampleScratch(*t.ctx, sliceTotal, stream));
+        const bool fan = groups > 1 && (!ps.samplesExt || sliced);
+        if (fan) HPSDF_CUDA(cudaEventRecord(ws.evFork, stream));
+        int g = 0;
+        bool used[4] = { false, false, false, false };
+        double flops = 0.0; uint64_t evals = 0;
+        for (int d = kMaxDegree; d >= 1; --d)                 // highest degree first: the longest kernels start earliest
+        {
+            const size_t n = cnt[d];
+            if (!n) continue;
+            size_t b = 0, e = n;
+            if (shard) hpsdf_shard_range(n, rank, world, &b, &e);
+            if (e > b)
+            {
+                cudaStream_t s = stream;
+                if (fan)
+                {
+                    s = ws.aux[g & 3];
+                    if (!used[g & 3]) { HPSDF_CUDA(cudaStreamWaitEvent(s, ws.evFork, 0)); used[g & 3] = true; }
+                    ++g;
+                }
+                const hpsdf_status ls = launchFit(o.jit, d, ws.tasks.p + lay.groupBegin[d] + b, (int)(e - b), ws.pool.p, ws.recs.p, prog, t.map, *t.ctx, s,
+                                                  sliced ? sliceOff[d] : 0, sliced ? slice[d] : 0, sliced ? d : 0);
+                if (ls != HPSDF_OK) return ls;
+                t.stats.kernel_launches++;
+            }
+            const double n3 = (double)fitRule(d) * fitRule(d) * fitRule(d);
+            flops += (double)n * (fitFlops(d) + ps.flopsPerEval * n3);
+            evals += (uint64_t)n * (uint64_t)n3;
+        }
+        if (fan)
+            for (int i = 0; i < 4; ++i)
+                if (used[i])
+                {
+                    HPSDF_CUDA(cudaEventRecord(ws.evJoin[i], ws.aux[i]));
+                    HPSDF_CUDA(cudaStreamWaitEvent(stream, ws.evJoin[i], 0));
+                }
+        HPSDF_CUDA(cudaEventRecord(evEnd, stream));
+        if (shard)
+        {
+            // every rank receives every other rank's shard: coefficients and records (replicated pool, identical replay)
+            std::vector<CommSegment> segs;
+            for (int d = 1; d <= kMaxDegree; ++d)
+            {
+                const size_t n = cnt[d];
+                if (!n) continue;
+                for (int r = 0; r < world; ++r)
+                {
+                    size_t b, e;
+                    hpsdf_shard_range(n, r, world, &b, &e);
+                    if (e <= b) continue;
+                    segs.push_back({ ws.pool.p + lay.groupPool[d] + b * (size_t)coeffCount(d), (e - b) * (size_t)coeffCount(d), r });
+                    segs.push_back({ (double*)(ws.recs.p + lay.groupBegin[d] + b), (e - b) * 2, r });
+                }
+            }
+            const hpsdf_status cs = commBroadcastSegments(o.comm, segs, stream);
+            if (cs != HPSDF_OK) return cs;
+        }
+        t.stats.algorithmic_flops += flops;
+        t.stats.sdf_evals += evals;
+        t.stats.fits_evaluated += nTasks;
+        t.stats.rounds++;
+        return HPSDF_OK;
+    }
+
     hpsdf_status packCoefficients(hpsdf_octree& t, const double* pool, cudaStream_t stream)
     {
         std::vector<HostNode>& nodes = t.nodes;

@@ -16,6 +16,15 @@ namespace hpsdf
     // errOf: current error per node; levelLogStart: first apply-log entry of the last batch of applied jobs.
     void logCutTieGroup(hpsdf_octree& t, const std::vector<double>& errOf, size_t levelLogStart, bool queueEmpty);
 
+    // The fit launches of one round, for both schedulers (ps = summarizeProgram(prog), worked out once per build): cnt[d]
+    // fits of degree d at the task positions and pool slots of `lay`, already expanded into t.ctx->ws.tasks
+    // (launchExpandJobsDev) with the pool reserved. One kernel per degree present (this rank's shard), highest degree first,
+    // fanned out over the workspace's four auxiliary streams; evBegin / evEnd bracket the launches on `stream`. A sharded
+    // round ends with one grouped broadcast per (degree group, rank).
+    hpsdf_status launchRoundFits(hpsdf_octree& t, const hpsdf_build_opts& o, const SdfProgramDev& prog, const ProgramSummary& ps,
+                                 cudaStream_t stream, const uint32_t* cnt, const RoundLayout& lay, uint32_t nTasks, int rank, int world,
+                                 cudaEvent_t evBegin, cudaEvent_t evEnd);
+
     hpsdf_status buildOctreeHost(hpsdf_octree& t, const hpsdf_build_opts& opts, const SdfProgramDev& prog);
     hpsdf_status buildOctreeDevice(hpsdf_octree& t, const hpsdf_build_opts& opts, const SdfProgramDev& prog, bool& fallBack);
 }

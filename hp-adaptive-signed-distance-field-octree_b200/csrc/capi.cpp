@@ -576,8 +576,7 @@ extern "C"
         out->jobs = jobs; out->fits = nH + nP;
         const uint64_t nh = fitRule((int)degree), np = fitRule((int)degree + 1);
         out->sdf_evals = nH * nh * nh * nh + nP * np * np * np;
-        double cF = 6.0;
-        for (uint32_t i = 0; i < dp.n; ++i) cF += sdfOpFlops(dp.instr[i].op);
+        const double cF = summarizeProgram(dp).flopsPerEval;
         out->sdf_flops_per_eval = cF;
         out->algorithmic_flops = (double)nH * fitFlops((int)degree) + (double)nP * fitFlops((int)degree + 1) + cF * (double)out->sdf_evals;
         for (const FitRecord& r : recs) out->checksum += r.rawErr;

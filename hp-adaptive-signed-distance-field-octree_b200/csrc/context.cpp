@@ -153,7 +153,7 @@ namespace hpsdf
         // a first pool of 32 M doubles (256 MB) and pinned staging for 128 K fits: a README-sized build never reallocates
         ctx->ws.pool.reserve((size_t)32 << 20);
         ctx->ws.tasks.reserve((size_t)1 << 17); ctx->ws.recs.reserve((size_t)1 << 17);
-        ctx->ws.hTasks.reserve((size_t)1 << 17); ctx->ws.hRecs.reserve((size_t)1 << 17);
+        ctx->ws.hRecs.reserve((size_t)1 << 17);
         if ((e = cudaDeviceSynchronize()) != cudaSuccess) { err = cudaGetErrorString(e); delete ctx; cudaFree(mem); return nullptr; }
         g_ctx[device] = ctx;
         return ctx;

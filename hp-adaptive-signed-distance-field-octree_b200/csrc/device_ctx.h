@@ -61,7 +61,6 @@ namespace hpsdf
         DeviceBuf<double>    samples;     // F at the Gauss-Legendre points of a chunk of fits (mesh / octree programs only)
         DeviceBuf<unsigned long long> sampleCounter;   // work counter of meshSampleKernel
         DeviceBuf<float4>    meshCut;     // per-fit cuts of the mesh BVH next to the sample scratch (mesh_sample_kernel.cuh: meshCutKernel)
-        PinnedBuf<FitTask>   hTasks;
         DeviceBuf<JobDesc>   jobs;
         PinnedBuf<JobDesc>   hJobs;
         PinnedBuf<FitRecord> hRecs;
@@ -112,7 +111,7 @@ namespace hpsdf
     void        uploadConstants();
     constexpr size_t kSampleScratchDoubles = (size_t)1 << 26;      // 512 MB of samples per chunk at most
     cudaError_t launchFitKernel(int degree, const FitTask* dTasks, int n, double* pool, FitRecord* recs,
-                                const SdfProgramDev& prog, const RootMap& map, DeviceCtx& ctx, cudaStream_t stream,
+                                const SdfProgramDev& prog, bool samplesExt, const RootMap& map, DeviceCtx& ctx, cudaStream_t stream,
                                 size_t sliceOffset = 0, size_t sliceDoubles = 0, int counterIdx = 0);
     cudaError_t reserveSampleScratch(DeviceCtx& ctx, size_t doubles, cudaStream_t stream);
     void        printFitTimeline(int rank);      // HPSDF_DEBUG_ROUNDS=3
@@ -123,7 +122,8 @@ namespace hpsdf
     bool        jitCompileCheck(const SdfProgramDev& prog, int degree, std::string* source, size_t* cubinBytes, std::string& why);
     void        setJitDefault(bool on);
     bool        jitDefault();
-    cudaError_t launchExpandJobs(const JobDesc* dJobs, uint32_t nJobs, const RoundLayout& layout, FitTask* dTasks, cudaStream_t stream);
+    // the fit tasks of a round's job records, at the task positions of the layout in device memory (fit_kernels.cuh)
+    cudaError_t launchExpandJobsDev(const JobDesc* dJobs, uint32_t nJobs, const RoundLayout* dLayout, FitTask* dTasks, cudaStream_t stream);
     cudaError_t launchSdfEval(const SdfProgramDev& prog, const double* dXyz, size_t n, double* dOut, cudaStream_t stream);
     cudaError_t launchDfmaPeak(double* dOut, int blocks, cudaStream_t stream);
     cudaError_t launchUniformPoints(uint64_t seed, uint64_t first, size_t n, const double lo[3], const double hi[3], double* dXyz, cudaStream_t stream);

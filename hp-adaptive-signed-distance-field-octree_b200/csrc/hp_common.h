@@ -132,8 +132,8 @@ namespace hpsdf
     };
     constexpr uint32_t kNoSrc = 0xFFFFFFFFu;
 
-    // One refinement job of a round as the host writes it (32 bytes instead of 9 FitTasks): expandJobsKernel turns it into
-    // the 8 child fits @degree at task positions hPos..hPos+7 of that degree's group and the p-fit @degree+1 at pPos.
+    // One refinement job of a round as a scheduler writes it (32 bytes instead of 9 FitTasks): expandJobsDevKernel turns it
+    // into the 8 child fits @degree at task positions hPos..hPos+7 of that degree's group and the p-fit @degree+1 at pPos.
     struct JobDesc
     {
         float    cx, cy, cz, half;   // the parent cell
@@ -149,6 +149,37 @@ namespace hpsdf
         uint32_t groupBegin[kMaxDegree + 2];
         uint32_t groupPool[kMaxDegree + 2];
     };
+
+    // The layout of a round with cnt[d] fits of degree d (d = 1..kMaxDegree): tasks in degree order, output slots handed out
+    // in task order from pool offset poolUsed, so a degree group (and a rank's shard of it) is one contiguous range of tasks
+    // and one of the pool. Returns the number of tasks; poolEnd = the pool offset after the round (callers refuse a round
+    // that takes it past 2^32 doubles).
+    HPSDF_HD inline uint32_t layoutRound(const uint32_t* cnt, uint32_t poolUsed, uint32_t* groupBegin, uint32_t* groupPool, uint64_t& poolEnd)
+    {
+        uint32_t nTasks = 0;
+        uint64_t pool = poolUsed;
+        groupBegin[0] = 0; groupPool[0] = poolUsed;
+        for (int d = 1; d <= kMaxDegree; ++d)
+        {
+            groupBegin[d] = nTasks; groupPool[d] = (uint32_t)pool;
+            nTasks += cnt[d]; pool += (uint64_t)cnt[d] * (uint64_t)coeffCount(d);
+        }
+        groupBegin[kMaxDegree + 1] = nTasks; groupPool[kMaxDegree + 1] = (uint32_t)pool;
+        poolEnd = pool;
+        return nTasks;
+    }
+
+    // Several GPUs evaluate contiguous shards of each degree group of a round, and selection order is spatially coherent (far
+    // and near cells of a mesh cluster, and their fits differ 10x in cost), so the n > 2 jobs of a sharded round are dealt
+    // out along the permutation k -> k * stride mod n: every shard gets the same mix. The stride is a prime that does not
+    // divide n (n < 2^32 cannot be a multiple of all four).
+    HPSDF_HD inline uint32_t dealStride(uint32_t n)
+    {
+        const uint32_t primes[4] = { 7919u, 7907u, 7901u, 7883u };
+        for (int i = 0; i < 4; ++i)
+            if (n % primes[i] != 0u) return primes[i];
+        return 1u;
+    }
 
     // What the host replay needs from a fit: the raw top-shell energy (Octree.cpp:1062-1069) and coeffs[0]
     // (the cell mean of the approximant up to NL[0][depth]^3, for the nearness weight).
@@ -202,6 +233,25 @@ namespace hpsdf
         uint32_t    pad;
         SdfInstrDev instr[HPSDF_PROGRAM_MAX_INSTR];
     };
+#ifndef __CUDACC_RTC__
+    // What launching a program's fits depends on: whether it samples a mesh or another octree (those fits sample F in a
+    // kernel of its own, into scratch: fit_kernels.cuh) and its FLOPs per evaluation (6 for the root map + the operators).
+    struct ProgramSummary
+    {
+        bool   samplesExt = false;
+        double flopsPerEval = 6.0;
+    };
+    inline ProgramSummary summarizeProgram(const SdfProgramDev& prog)
+    {
+        ProgramSummary s;
+        for (uint32_t i = 0; i < prog.n; ++i)
+        {
+            s.flopsPerEval += sdfOpFlops(prog.instr[i].op);
+            s.samplesExt |= prog.instr[i].op == HPSDF_PRIM_MESH || prog.instr[i].op == HPSDF_PRIM_OCTREE;
+        }
+        return s;
+    }
+#endif
 
     // Leaf/internal node as the Query kernel reads it: 16 bytes, one LDG.128.
     struct QNode

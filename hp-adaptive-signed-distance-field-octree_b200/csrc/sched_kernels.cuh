@@ -1021,30 +1021,19 @@ namespace hpsdf
                 if (job0 + nSel > S.capJobs) { if (tid == 0) sh.done = 2u; nSel = 0; }
                 __syncthreads();
                 for (int d = 1; d <= kMaxDegree; ++d) cnt[d] = nSel ? sh.degCnt[d] : 0u;
-                // layout: tasks in degree order, slots allocated in task order (contiguous per degree: a rank's shard of a degree
-                // group is one contiguous pool range)
                 uint32_t groupBegin[kMaxDegree + 2], groupPool[kMaxDegree + 2];
-                uint32_t nTasks = 0;
-                unsigned long long poolNeed = sh.poolUsed;
-                groupBegin[0] = 0; groupPool[0] = sh.poolUsed;
-                for (int d = 1; d <= kMaxDegree; ++d)
-                {
-                    groupBegin[d] = nTasks; groupPool[d] = (uint32_t)poolNeed;
-                    nTasks += cnt[d]; poolNeed += (unsigned long long)cnt[d] * (unsigned long long)coeffCount(d);
-                }
-                groupBegin[kMaxDegree + 1] = nTasks; groupPool[kMaxDegree + 1] = (uint32_t)poolNeed;
+                uint64_t poolNeed = 0;
+                layoutRound(cnt, sh.poolUsed, groupBegin, groupPool, poolNeed);
                 if (poolNeed >= 0xFFFFFFF0ull) { if (tid == 0) sh.done = 2u; nSel = 0; }
                 for (int d = 0; d <= kMaxDegree + 1; ++d) { lay2Begin[d] = groupBegin[d]; lay2Pool[d] = groupPool[d]; }
                 __syncthreads();
-                // positions of every job's fits inside its groups, in job order; job records for expandJobsKernel
+                // positions of every job's fits inside its groups, in job order; job records for expandJobsDevKernel
                 uint32_t cursor[kMaxDegree + 2];
                 for (int d = 0; d <= kMaxDegree + 1; ++d) cursor[d] = groupBegin[d];
-                // Several GPUs evaluate contiguous shards of each degree group, and list order is spatially coherent (far and near cells
-                // of a mesh cluster; their fits differ 10x in cost): task positions are handed out along a fixed stride permutation of the
-                // round's jobs, so every shard gets the same mix. (Only pool slots and record positions depend on it.)
-                uint32_t dealStride = 1u;
-                if (S.dealJobs && nSel > 2u)
-                    for (const uint32_t cand : { 7919u, 7907u, 7901u, 7883u }) if (nSel % cand != 0u) { dealStride = cand; break; }
+                // several GPUs: task positions are handed out along the deal permutation of the round's jobs (dealStride; only pool
+                // slots and record positions depend on it)
+                uint32_t stride = 1u;
+                if (S.dealJobs && nSel > 2u) stride = dealStride(nSel);
                 for (uint32_t base = 0; base < nSel; base += kSchedThreads * 4u)
                 {
                     uint32_t node[4], p[4], hPos[4], pPos[4];
@@ -1054,7 +1043,7 @@ namespace hpsdf
                     {
                         const uint32_t k = base + tid * 4u + r;
                         node[r] = 0; p[r] = 0; flags[r] = 0; hPos[r] = 0; pPos[r] = 0;
-                        if (k < nSel) { const uint32_t j = job0 + (uint32_t)(((unsigned long long)k * dealStride) % nSel); node[r] = S.jobNode[j]; p[r] = S.degree[node[r]]; flags[r] = S.jobFlags[j]; }
+                        if (k < nSel) { const uint32_t j = job0 + (uint32_t)(((unsigned long long)k * stride) % nSel); node[r] = S.jobNode[j]; p[r] = S.degree[node[r]]; flags[r] = S.jobFlags[j]; }
                     }
                     for (int d = 1; d <= kMaxDegree; ++d)
                     {
@@ -1078,7 +1067,7 @@ namespace hpsdf
                     {
                         const uint32_t k = base + tid * 4u + r;
                         if (k >= nSel) continue;
-                        const uint32_t j = job0 + (uint32_t)(((unsigned long long)k * dealStride) % nSel), pp = p[r];
+                        const uint32_t j = job0 + (uint32_t)(((unsigned long long)k * stride) % nSel), pp = p[r];
                         const uint32_t depth = S.depth[node[r]];
                         S.jobHPos[j] = hPos[r]; S.jobPPos[j] = pPos[r];
                         S.jobHSlot[j] = (flags[r] & 1u) ? groupPool[pp] + (hPos[r] - groupBegin[pp]) * (uint32_t)coeffCount((int)pp) : 0u;
@@ -1239,15 +1228,8 @@ namespace hpsdf
             __syncthreads();
             const uint32_t nSel = sTotal[1];
             uint32_t groupBegin[kMaxDegree + 2], groupPool[kMaxDegree + 2];
-            uint32_t nTasks = 0;
-            unsigned long long poolNeed = poolUsed0;
-            groupBegin[0] = 0; groupPool[0] = poolUsed0;
-            for (int d = 1; d <= kMaxDegree; ++d)
-            {
-                groupBegin[d] = nTasks; groupPool[d] = (uint32_t)poolNeed;
-                nTasks += sTotal[2 + d]; poolNeed += (unsigned long long)sTotal[2 + d] * (unsigned long long)coeffCount(d);
-            }
-            groupBegin[kMaxDegree + 1] = nTasks; groupPool[kMaxDegree + 1] = (uint32_t)poolNeed;
+            uint64_t poolNeed = 0;
+            const uint32_t nTasks = layoutRound(sTotal + 2, poolUsed0, groupBegin, groupPool, poolNeed);
             const bool overflow = job0 + nSel > S.capJobs || poolNeed >= 0xFFFFFFF0ull;
             const uint32_t doneCode = overflow ? 2u : (nSel == 0u ? 4u : 0u);
             if (chunk == 0 && tid == 0)
