@@ -128,7 +128,7 @@ EXPORTS = [
     "hpsdf_bench_frontier", "hpsdf_measure_fp64_peak", "hpsdf_comm_get_unique_id", "hpsdf_comm_init",
     "hpsdf_comm_destroy", "hpsdf_shard_range", "hpsdf_set_jit", "hpsdf_jit_compile_check", "hpsdf_query_ray",
     "hpsdf_get_config", "hpsdf_get_device", "hpsdf_uniform_points_device", "hpsdf_extract_isosurface",
-    "hpsdf_raycast", "hpsdf_raycast_device",
+    "hpsdf_raycast", "hpsdf_raycast_device", "hpsdf_query_derivatives", "hpsdf_query_derivatives_device",
 ]
 
 _lib = None
@@ -172,6 +172,8 @@ def lib():
     L.hpsdf_query_ray.argtypes = [vp, vp, vp, sz, dbl, vp, vp]
     L.hpsdf_raycast.argtypes = [vp, vp, vp, sz, dbl, dbl, dbl, vp, vp]
     L.hpsdf_raycast_device.argtypes = [vp, vp, vp, sz, dbl, dbl, dbl, vp, vp, vp]
+    L.hpsdf_query_derivatives.argtypes = [vp, vp, sz, vp, vp, vp]
+    L.hpsdf_query_derivatives_device.argtypes = [vp, vp, sz, vp, vp, vp, vp]
     L.hpsdf_extract_isosurface.argtypes = [vp, vp, vp, vp, dbl, C.POINTER(sz), C.POINTER(vp), C.POINTER(sz), C.POINTER(vp)]
     L.hpsdf_to_memory_block.argtypes = [vp, C.POINTER(sz), C.POINTER(vp)]
     L.hpsdf_from_memory_block.argtypes = [vp, sz, i32, C.POINTER(vp)]
@@ -350,6 +352,42 @@ class Octree:
         g = np.empty((len(a), 3), np.float64)
         _check(lib().hpsdf_query_with_gradient(self._h, a.ctypes.data, len(a), out.ctypes.data, g.ctypes.data))
         return out, g
+
+    def QueryDerivatives(self, pts, hessian=False):
+        """Query's values with the exact gradients and, with hessian=True, Hessians of the hit leaves' polynomials in user
+        space (hpsdf_query_derivatives, DESIGN §13) -> (values (n,), grads (n,3)[, hess (n,6): xx, xy, xz, yy, yz, zz]).
+        Gradients are not normalised; outside the root the value is DBL_MAX and the derivatives are 0."""
+        a = np.ascontiguousarray(pts, np.float64).reshape(-1, 3)
+        v = np.empty(len(a), np.float64)
+        g = np.empty((len(a), 3), np.float64)
+        h = np.empty((len(a), 6), np.float64) if hessian else None
+        _check(lib().hpsdf_query_derivatives(self._h, a.ctypes.data, len(a), v.ctypes.data, g.ctypes.data,
+                                             h.ctypes.data if hessian else None))
+        return (v, g, h) if hessian else (v, g)
+
+    def QueryDerivativesDevice(self, d_xyz, n, d_value, d_grad, d_hess=None, stream=None):
+        """QueryDerivatives with device pointers (e.g. torch tensors' data_ptr()), asynchronous on `stream` (cudaStream_t as
+        int); d_hess = None skips the Hessians."""
+        _check(lib().hpsdf_query_derivatives_device(self._h, d_xyz, n, d_value, d_grad, d_hess, stream))
+
+    def QueryTorch(self, x):
+        """Query as a differentiable torch function: x is a contiguous CUDA float64 (n,3) tensor on the tree's device, the
+        result (n,) float64, computed on the current stream of that device. Autograd gets the exact gradient from the
+        forward launch, and the exact Hessian on a second differentiation (create_graph=True); a third raises. Nothing is
+        copied: another dtype, device, shape or layout raises."""
+        import torch
+        self._need()
+        if not isinstance(x, torch.Tensor) or x.dtype != torch.float64:
+            raise TypeError("QueryTorch needs a float64 torch tensor")
+        dev = C.c_int()
+        _check(lib().hpsdf_get_device(self._h, C.byref(dev)))
+        if x.device.type != "cuda" or x.device.index != dev.value:
+            raise ValueError("QueryTorch needs a tensor on cuda:%d, the tree's device (got %s)" % (dev.value, x.device))
+        if x.dim() != 2 or x.shape[1] != 3 or not x.is_contiguous():
+            raise ValueError("QueryTorch needs a contiguous (n, 3) tensor (got shape %s)" % (tuple(x.shape),))
+        if x.requires_grad and torch.is_grad_enabled():
+            return _torch_query()[0].apply(x, self)
+        return _torch_launch(self, x, 0)[0]
 
     def QueryRay(self, origins, directions, t_max):
         """Octree::QueryRay (Octree.cpp:705-746) for a batch of rays -> (hit flags, t). Mirrors the reference statement by statement."""
@@ -553,6 +591,88 @@ class Octree:
             self.Clear()
         except Exception:
             pass
+
+
+def _torch_launch(tree, x, order):
+    """Query (order 0) or the derivatives (order 1, 2) of a checked CUDA tensor x, on the current stream of its device."""
+    import torch
+    n = x.shape[0]
+    v = torch.empty(n, dtype=torch.float64, device=x.device)
+    g = torch.empty((n, 3), dtype=torch.float64, device=x.device) if order >= 1 else None
+    h = torch.empty((n, 6), dtype=torch.float64, device=x.device) if order == 2 else None
+    with torch.cuda.device(x.device):
+        stream = torch.cuda.current_stream(x.device).cuda_stream
+        if order == 0:
+            _check(lib().hpsdf_query_device(tree._h, x.data_ptr(), n, v.data_ptr(), stream))
+        else:
+            _check(lib().hpsdf_query_derivatives_device(tree._h, x.data_ptr(), n, v.data_ptr(), g.data_ptr(),
+                                                        h.data_ptr() if h is not None else None, stream))
+    return v, g, h
+
+
+_TORCH_QUERY = None
+
+
+def _torch_query():
+    """The autograd functions behind Octree.QueryTorch, defined on first use so that importing this package needs no torch."""
+    global _TORCH_QUERY
+    if _TORCH_QUERY is not None:
+        return _TORCH_QUERY
+    import torch
+
+    class QueryFn(torch.autograd.Function):
+        """F(x): one ORDER-1 launch gives the value and keeps the gradient for backward."""
+
+        @staticmethod
+        def forward(ctx, x, tree):
+            v, g, _ = _torch_launch(tree, x, 1)
+            ctx.tree = tree
+            ctx.save_for_backward(x, g)
+            return v
+
+        @staticmethod
+        def backward(ctx, gv):
+            x, g = ctx.saved_tensors
+            return GradFn.apply(x, gv, g, ctx.tree), None
+
+    class GradFn(torch.autograd.Function):
+        """gv[:, None] * grad F(x); its backward is the Hessian-vector product from one ORDER-2 launch."""
+
+        @staticmethod
+        def forward(ctx, x, gv, g, tree):
+            ctx.tree = tree
+            ctx.save_for_backward(x, gv, g)
+            return gv[:, None] * g
+
+        @staticmethod
+        def backward(ctx, w):
+            x, gv, g = ctx.saved_tensors
+            gx = ggv = None
+            if ctx.needs_input_grad[0]:
+                H = _torch_launch(ctx.tree, x.detach(), 2)[2]
+                Hw = torch.stack([H[:, 0] * w[:, 0] + H[:, 1] * w[:, 1] + H[:, 2] * w[:, 2],
+                                  H[:, 1] * w[:, 0] + H[:, 3] * w[:, 1] + H[:, 4] * w[:, 2],
+                                  H[:, 2] * w[:, 0] + H[:, 4] * w[:, 1] + H[:, 5] * w[:, 2]], 1)
+                gx = gv[:, None] * Hw
+            if ctx.needs_input_grad[1]:
+                ggv = (g * w).sum(1)
+            if torch.is_grad_enabled():
+                gx, ggv = NoThirdOrder.apply(x, gx, ggv)
+            return gx, ggv, None, None
+
+    class NoThirdOrder(torch.autograd.Function):
+        """Passes the second derivatives through; differentiating them (a third derivative of F) raises."""
+
+        @staticmethod
+        def forward(ctx, x, gx, ggv):
+            return (None if gx is None else gx.clone()), (None if ggv is None else ggv.clone())
+
+        @staticmethod
+        def backward(ctx, *_):
+            raise RuntimeError("Octree.QueryTorch is differentiable twice: a third derivative of the field is not available")
+
+    _TORCH_QUERY = (QueryFn, GradFn)
+    return _TORCH_QUERY
 
 
 def fit_batch(config, F, cells, depth, degree, device=-1):

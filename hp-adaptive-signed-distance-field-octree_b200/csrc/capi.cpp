@@ -185,6 +185,46 @@ extern "C"
         return HPSDF_OK;
     }
 
+    static hpsdf_status derivativesArgs(const hpsdf_octree* tree, const void* xyz, size_t n, const void* value, const void* grad)
+    {
+        if (hpsdf_device_count() == 0) { setLastError("no CUDA device available: this library has no CPU path"); return HPSDF_ERR_NO_DEVICE; }
+        if (!tree || (n && (!xyz || !value || !grad))) { setLastError("null pointer"); return HPSDF_ERR_INVALID_ARG; }
+        return HPSDF_OK;
+    }
+
+    HPSDF_API hpsdf_status hpsdf_query_derivatives(const hpsdf_octree* tree, const double* xyz, size_t n, double* value, double* grad,
+                                                   double* hess)
+    {
+        hpsdf_status st = derivativesArgs(tree, xyz, n, value, grad);
+        if (st != HPSDF_OK || !n) return st;
+        HPSDF_CUDA(cudaSetDevice(tree->device));
+        double *dIn = nullptr, *dV = nullptr, *dG = nullptr, *dH = nullptr;
+        HPSDF_CUDA(cudaMalloc((void**)&dIn, n * 24));
+        cudaError_t e = cudaMalloc((void**)&dV, n * 8);
+        if (e == cudaSuccess) e = cudaMalloc((void**)&dG, n * 24);
+        if (e == cudaSuccess && hess) e = cudaMalloc((void**)&dH, n * 48);
+        if (e == cudaSuccess) e = cudaMemcpy(dIn, xyz, n * 24, cudaMemcpyHostToDevice);
+        if (e == cudaSuccess) e = launchQueryDerivatives(tree->view, dIn, n, dV, dG, dH, tree->ctx->smCount, nullptr);
+        if (e == cudaSuccess) e = cudaMemcpy(value, dV, n * 8, cudaMemcpyDeviceToHost);
+        if (e == cudaSuccess) e = cudaMemcpy(grad, dG, n * 24, cudaMemcpyDeviceToHost);
+        if (e == cudaSuccess && hess) e = cudaMemcpy(hess, dH, n * 48, cudaMemcpyDeviceToHost);
+        cudaFree(dIn); cudaFree(dV); cudaFree(dG); cudaFree(dH);
+        if (e != cudaSuccess) return failCuda(e, "hpsdf_query_derivatives");
+        return HPSDF_OK;
+    }
+
+    HPSDF_API hpsdf_status hpsdf_query_derivatives_device(const hpsdf_octree* tree, const double* d_xyz, size_t n, double* d_value,
+                                                          double* d_grad, double* d_hess, void* stream)
+    {
+        hpsdf_status st = derivativesArgs(tree, d_xyz, n, d_value, d_grad);
+        if (st != HPSDF_OK) return st;
+        int cur = -1;
+        if (cudaGetDevice(&cur) != cudaSuccess || cur != tree->device)
+        { setLastError("hpsdf_query_derivatives_device: the current CUDA device is not the tree's device"); return HPSDF_ERR_INVALID_ARG; }
+        HPSDF_CUDA(launchQueryDerivatives(tree->view, d_xyz, n, d_value, d_grad, d_hess, tree->ctx->smCount, (cudaStream_t)stream));
+        return HPSDF_OK;
+    }
+
     HPSDF_API hpsdf_status hpsdf_query_ray(const hpsdf_octree* tree, const double* origins, const double* directions, size_t n, double t_max,
                                            unsigned char* hit, double* t)
     {

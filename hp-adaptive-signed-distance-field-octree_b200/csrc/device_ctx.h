@@ -134,6 +134,9 @@ namespace hpsdf
     cudaError_t launchRaycast(const DeviceTreeView& view, const double* dOrigins, const double* dDirs, size_t n, double tMin, double tMax,
                               double iso, double* dT, double* dNormals, int smCount, cudaStream_t stream);
     cudaError_t launchQueryGradient(const DeviceTreeView& view, const double* dXyz, size_t n, double* dOut, double* dGrad, cudaStream_t stream);
+    // hpsdf_query_derivatives (query_kernels.cuh): value, gradient, and the Hessian when dHess is not nullptr
+    cudaError_t launchQueryDerivatives(const DeviceTreeView& view, const double* dXyz, size_t n, double* dValue, double* dGrad,
+                                       double* dHess, int smCount, cudaStream_t stream);
     // hpsdf_extract_isosurface (isosurface_kernels.cuh): a grid of (n0+1)(n1+1)(n2+1) < 2^32 points
     struct IsoGrid
     {

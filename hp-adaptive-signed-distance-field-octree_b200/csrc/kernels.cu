@@ -71,6 +71,20 @@ namespace hpsdf
         return cudaGetLastError();
     }
 
+    cudaError_t launchQueryDerivatives(const DeviceTreeView& view, const double* dXyz, size_t n, double* dValue, double* dGrad,
+                                       double* dHess, int smCount, cudaStream_t stream)
+    {
+        if (!n) return cudaSuccess;
+        const int aligned = ((uintptr_t)dXyz & 15u) == 0 ? 1 : 0;
+        if (dHess)
+            queryDerivativesKernel<2><<<persistentGrid(n, derivBlocksPerSm(2), smCount), kQueryThreads, 0, stream>>>(view, dXyz, n, dValue,
+                                                                                                                   dGrad, dHess, aligned);
+        else
+            queryDerivativesKernel<1><<<persistentGrid(n, derivBlocksPerSm(1), smCount), kQueryThreads, 0, stream>>>(view, dXyz, n, dValue,
+                                                                                                                   dGrad, nullptr, aligned);
+        return cudaGetLastError();
+    }
+
     cudaError_t launchQueryGradient(const DeviceTreeView& view, const double* dXyz, size_t n, double* dOut, double* dGrad, cudaStream_t stream)
     {
         if (!n) return cudaSuccess;

@@ -18,21 +18,51 @@
 
 namespace hpsdf
 {
+    // Derivatives of a leaf polynomial with respect to its local coordinate u: gradient, and Hessian in the order
+    // xx, xy, xz, yy, yz, zz (filled for ORDER 2 only).
+    struct LeafDerivs
+    {
+        double g[3] = { 0.0, 0.0, 0.0 };
+        double h[6] = { 0.0, 0.0, 0.0, 0.0, 0.0, 0.0 };
+    };
+
     // Warp-uniform evaluation: all lanes run the instantiation of the warp's LARGEST leaf degree and switch whole shells
     // off with a predicate (p <= myDeg), so lanes whose leaves have different degrees do not serialise (ncu showed 17 of
     // 32 lanes active per instruction when each lane branched to its own degree). Lanes without a leaf pass myDeg = -1.
-    template <int DEG>
-    __device__ __forceinline__ double evalLeafMasked(const double* __restrict__ coeffs, int myDeg, double ux, double uy, double uz, int depth)
+    // ORDER 1 / 2 also accumulate the derivatives into *dv, from the derivatives of the Legendre recurrence
+    // (P'_j = r0 (P_j-1 + u P'_j-1) - r1 P'_j-2, P''_j = r0 (2 P'_j-1 + u P''_j-1) - r1 P''_j-2). The value keeps ORDER 0's
+    // products and order, and no product of it gets another use, so it is Query's to the bit.
+    template <int DEG, int ORDER = 0>
+    __device__ __forceinline__ double evalLeafMasked(const double* __restrict__ coeffs, int myDeg, double ux, double uy, double uz, int depth,
+                                                     LeafDerivs* dv = nullptr)
     {
+        constexpr int N1 = ORDER >= 1 ? DEG + 1 : 1, N2 = ORDER >= 2 ? DEG + 1 : 1;
         double lx[DEG + 1], ly[DEG + 1], lz[DEG + 1];
+        double dlx[N1], dly[N1], dlz[N1], ddlx[N2], ddly[N2], ddlz[N2];
         {
             const double nl0 = c_nl[0][depth];
             lx[0] = nl0; ly[0] = nl0; lz[0] = nl0;
+            if constexpr (ORDER >= 1) { dlx[0] = 0.0; dly[0] = 0.0; dlz[0] = 0.0; }
+            if constexpr (ORDER >= 2) { ddlx[0] = 0.0; ddly[0] = 0.0; ddlz[0] = 0.0; }
             double ax2 = 0.0, ax1 = 1.0, ay2 = 0.0, ay1 = 1.0, az2 = 0.0, az1 = 1.0;
+            double bx2 = 0.0, bx1 = 0.0, by2 = 0.0, by1 = 0.0, bz2 = 0.0, bz1 = 0.0;      // P'
+            double cx2 = 0.0, cx1 = 0.0, cy2 = 0.0, cy1 = 0.0, cz2 = 0.0, cz1 = 0.0;      // P''
             #pragma unroll
             for (int j = 1; j <= DEG; ++j)
             {
                 const double r0 = c_rec[j][0], r1 = c_rec[j][1], nl = c_nl[j][depth];
+                if constexpr (ORDER >= 2)
+                {
+                    const double cx = r0 * (2.0 * bx1 + ux * cx1) - r1 * cx2; cx2 = cx1; cx1 = cx; ddlx[j] = cx * nl;
+                    const double cy = r0 * (2.0 * by1 + uy * cy1) - r1 * cy2; cy2 = cy1; cy1 = cy; ddly[j] = cy * nl;
+                    const double cz = r0 * (2.0 * bz1 + uz * cz1) - r1 * cz2; cz2 = cz1; cz1 = cz; ddlz[j] = cz * nl;
+                }
+                if constexpr (ORDER >= 1)
+                {
+                    const double bx = r0 * (ax1 + ux * bx1) - r1 * bx2; bx2 = bx1; bx1 = bx; dlx[j] = bx * nl;
+                    const double by = r0 * (ay1 + uy * by1) - r1 * by2; by2 = by1; by1 = by; dly[j] = by * nl;
+                    const double bz = r0 * (az1 + uz * bz1) - r1 * bz2; bz2 = bz1; bz1 = bz; dlz[j] = bz * nl;
+                }
                 const double ax = r0 * ux * ax1 - r1 * ax2; ax2 = ax1; ax1 = ax; lx[j] = ax * nl;      // Octree.cpp:879-883
                 const double ay = r0 * uy * ay1 - r1 * ay2; ay2 = ay1; ay1 = ay; ly[j] = ay * nl;
                 const double az = r0 * uz * az1 - r1 * az2; az2 = az1; az1 = az; lz[j] = az * nl;
@@ -58,6 +88,23 @@ namespace hpsdf
                     if ((idx & 1) == 0) { if (on) cur = __ldg(c2 + (idx >> 1)); }
                     const double cv = (idx & 1) ? cur.y : cur.x;
                     if (term) f = fma(cv, (lx[i] * ly[j]) * lz[k], f);                                  // Octree.cpp:891-897
+                    if constexpr (ORDER >= 1)
+                        if (term)
+                        {
+                            dv->g[0] = fma(cv, (dlx[i] * ly[j]) * lz[k], dv->g[0]);
+                            dv->g[1] = fma(cv, (lx[i] * dly[j]) * lz[k], dv->g[1]);
+                            dv->g[2] = fma(cv, (lx[i] * ly[j]) * dlz[k], dv->g[2]);
+                        }
+                    if constexpr (ORDER >= 2)
+                        if (term)
+                        {
+                            dv->h[0] = fma(cv, (ddlx[i] * ly[j]) * lz[k], dv->h[0]);
+                            dv->h[1] = fma(cv, (dlx[i] * dly[j]) * lz[k], dv->h[1]);
+                            dv->h[2] = fma(cv, (dlx[i] * ly[j]) * dlz[k], dv->h[2]);
+                            dv->h[3] = fma(cv, (lx[i] * ddly[j]) * lz[k], dv->h[3]);
+                            dv->h[4] = fma(cv, (lx[i] * dly[j]) * dlz[k], dv->h[4]);
+                            dv->h[5] = fma(cv, (lx[i] * ly[j]) * ddlz[k], dv->h[5]);
+                        }
                     ++idx;
                 }
             }
@@ -90,6 +137,54 @@ namespace hpsdf
             f = fma(coeffs[i], (l[0][abc & 0xFF] * l[1][(abc >> 8) & 0xFF]) * l[2][(abc >> 16) & 0xFF], f);
         }
         return f;
+    }
+
+    // Gradient and, for ORDER 2, Hessian of a leaf polynomial of any degree with respect to its local u: the basis-table loop
+    // over Legendre values and their derivatives in local memory. rayNormal is this routine (ORDER 1) plus normalisation.
+    template <int ORDER>
+    __device__ __noinline__ void leafDerivsGeneric(const double* __restrict__ coeffs, int degree, int depth, const double (&u)[3],
+                                                   const uint32_t* __restrict__ bidx, LeafDerivs& d)
+    {
+        constexpr int N2 = ORDER >= 2 ? kMaxDegree + 1 : 1;
+        double l[3][kMaxDegree + 1], dl[3][kMaxDegree + 1], ddl[3][N2];
+        for (int a = 0; a < 3; ++a)
+        {
+            l[a][0] = c_nl[0][depth]; dl[a][0] = 0.0;
+            if constexpr (ORDER >= 2) ddl[a][0] = 0.0;
+            double m2 = 0.0, m1 = 1.0, d2 = 0.0, d1 = 0.0, e2 = 0.0, e1 = 0.0;
+            for (int j = 1; j <= degree; ++j)
+            {
+                const double r0 = c_rec[j][0], r1 = c_rec[j][1];
+                if constexpr (ORDER >= 2)
+                {
+                    const double ev = r0 * (2.0 * d1 + u[a] * e1) - r1 * e2;
+                    e2 = e1; e1 = ev;
+                    ddl[a][j] = ev * c_nl[j][depth];
+                }
+                const double v = r0 * u[a] * m1 - r1 * m2, dv = r0 * (m1 + u[a] * d1) - r1 * d2;
+                m2 = m1; m1 = v; d2 = d1; d1 = dv;
+                l[a][j] = v * c_nl[j][depth]; dl[a][j] = dv * c_nl[j][depth];
+            }
+        }
+        const int nc = coeffCount(degree);
+        for (int i = 0; i < nc; ++i)
+        {
+            const uint32_t abc = __ldg(bidx + i);
+            const int x = abc & 0xFF, y = (abc >> 8) & 0xFF, z = (abc >> 16) & 0xFF;
+            const double c = __ldg(coeffs + i);
+            d.g[0] = fma(c, (dl[0][x] * l[1][y]) * l[2][z], d.g[0]);
+            d.g[1] = fma(c, (l[0][x] * dl[1][y]) * l[2][z], d.g[1]);
+            d.g[2] = fma(c, (l[0][x] * l[1][y]) * dl[2][z], d.g[2]);
+            if constexpr (ORDER >= 2)
+            {
+                d.h[0] = fma(c, (ddl[0][x] * l[1][y]) * l[2][z], d.h[0]);
+                d.h[1] = fma(c, (dl[0][x] * dl[1][y]) * l[2][z], d.h[1]);
+                d.h[2] = fma(c, (dl[0][x] * l[1][y]) * dl[2][z], d.h[2]);
+                d.h[3] = fma(c, (l[0][x] * ddl[1][y]) * l[2][z], d.h[3]);
+                d.h[4] = fma(c, (l[0][x] * dl[1][y]) * dl[2][z], d.h[4]);
+                d.h[5] = fma(c, (l[0][x] * l[1][y]) * ddl[2][z], d.h[5]);
+            }
+        }
     }
 
     struct LeafHit

@@ -61,6 +61,91 @@ namespace hpsdf
         }
     }
 
+#ifndef HPSDF_DERIV1_MINBLOCKS
+#define HPSDF_DERIV1_MINBLOCKS 3
+#endif
+#ifndef HPSDF_DERIV2_MINBLOCKS
+#define HPSDF_DERIV2_MINBLOCKS 2
+#endif
+    // CTAs per SM of queryDerivativesKernel<ORDER>: they set its register budget (DESIGN.md §13 has the ptxas lines)
+    constexpr int derivBlocksPerSm(int order) { return order == 1 ? HPSDF_DERIV1_MINBLOCKS : HPSDF_DERIV2_MINBLOCKS; }
+
+    // hpsdf_query_derivatives (DESIGN.md §13): Query's value and the exact gradient (ORDER 1) and Hessian (ORDER 2) of the
+    // hit leaf's polynomial in user space, d/dx_a = s_a d/du_a with s_a = 2^(depth+1) invSizes_a; 0 outside the root.
+    // queryKernel's structure: persistent grid, warp tiles of 32 points staged through shared memory, the top table in
+    // shared memory, warp-uniform degree dispatch. The value is evalLeafMasked's / evalLeafGeneric's, so Query's to the bit.
+    // The tile buffer also stages the gradients and Hessians, so every store of a warp is one contiguous run.
+    template <int ORDER>
+    __global__ void __launch_bounds__(kQueryThreads, derivBlocksPerSm(ORDER))
+    queryDerivativesKernel(const DeviceTreeView view, const double* __restrict__ xyz, size_t n, double* __restrict__ value,
+                           double* __restrict__ grad, double* __restrict__ hess, const int aligned /* xyz is 16-byte aligned */)
+    {
+        constexpr int kTile = ORDER == 2 ? 6 * 32 : 3 * 32;
+        __shared__ uint32_t sTop[4096];
+        __shared__ __align__(16) double sBuf[kQueryThreads / 32][kTile];
+        const bool useTop = stageTop(sTop, view.top);
+        const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+        const size_t nGroups = (n + 31) / 32;
+        const size_t warpsTotal = (size_t)gridDim.x * (kQueryThreads / 32);
+        double* sp = sBuf[warp];
+        for (size_t g = (size_t)blockIdx.x * (kQueryThreads / 32) + warp; g < nGroups; g += warpsTotal)
+        {
+            const size_t base = g * 32;
+            const size_t cnt = n - base < 32 ? n - base : 32;
+            const double* src = xyz + 3 * base;
+            if (cnt == 32 && aligned)
+            {
+                reinterpret_cast<double2*>(sp)[lane] = __ldcs(reinterpret_cast<const double2*>(src) + lane);
+                if (lane < 16) reinterpret_cast<double2*>(sp)[32 + lane] = __ldcs(reinterpret_cast<const double2*>(src) + 32 + lane);
+            }
+            else
+                for (size_t v = lane; v < 3 * cnt; v += 32) sp[v] = src[v];
+            __syncwarp();
+            LeafHit h;
+            if ((size_t)lane < cnt) h = findLeaf(view, useTop ? sTop : nullptr, sp[3 * lane], sp[3 * lane + 1], sp[3 * lane + 2]);
+            __syncwarp();                           // sp now takes this tile's results
+            LeafDerivs d;
+            double v;
+            switch ((int)__reduce_max_sync(0xFFFFFFFFu, (unsigned)(h.degree < 0 ? 0 : h.degree)))
+            {
+                case 0:  v = evalLeafMasked<0, ORDER>(h.coeffs, h.degree, h.ux, h.uy, h.uz, h.depth, &d); break;
+                case 1:  v = evalLeafMasked<1, ORDER>(h.coeffs, h.degree, h.ux, h.uy, h.uz, h.depth, &d); break;
+                case 2:  v = evalLeafMasked<2, ORDER>(h.coeffs, h.degree, h.ux, h.uy, h.uz, h.depth, &d); break;
+                case 3:  v = evalLeafMasked<3, ORDER>(h.coeffs, h.degree, h.ux, h.uy, h.uz, h.depth, &d); break;
+                case 4:  v = evalLeafMasked<4, ORDER>(h.coeffs, h.degree, h.ux, h.uy, h.uz, h.depth, &d); break;
+                case 5:  v = evalLeafMasked<5, ORDER>(h.coeffs, h.degree, h.ux, h.uy, h.uz, h.depth, &d); break;
+                case 6:  v = evalLeafMasked<6, ORDER>(h.coeffs, h.degree, h.ux, h.uy, h.uz, h.depth, &d); break;
+                default:
+                    v = 0.0;
+                    if (h.degree >= 0)
+                    {
+                        v = evalLeafGeneric(h.coeffs, h.degree, h.ux, h.uy, h.uz, h.depth, view.bidx);
+                        const double u[3] = { h.ux, h.uy, h.uz };
+                        leafDerivsGeneric<ORDER>(h.coeffs, h.degree, h.depth, u, view.bidx, d);
+                    }
+                    break;
+            }
+            const double scale = (double)(2u << h.depth);
+            const double s[3] = { scale * view.map.invSizes[0], scale * view.map.invSizes[1], scale * view.map.invSizes[2] };
+            const bool in = h.degree >= 0;                                          // outside the root: DBL_MAX, derivatives 0
+            if ((size_t)lane < cnt) __stcs(value + base + lane, in ? v : DBL_MAX);
+            #pragma unroll
+            for (int a = 0; a < 3; ++a) sp[3 * lane + a] = in ? d.g[a] * s[a] : 0.0;
+            __syncwarp();
+            for (size_t k = lane; k < 3 * cnt; k += 32) __stcs(grad + 3 * base + k, sp[k]);
+            if constexpr (ORDER == 2)
+            {
+                __syncwarp();
+                constexpr int ia[6] = { 0, 0, 0, 1, 1, 2 }, ib[6] = { 0, 1, 2, 1, 2, 2 };
+                #pragma unroll
+                for (int k = 0; k < 6; ++k) sp[6 * lane + k] = in ? d.h[k] * (s[ia[k]] * s[ib[k]]) : 0.0;
+                __syncwarp();
+                for (size_t k = lane; k < 6 * cnt; k += 32) __stcs(hess + 6 * base + k, sp[k]);
+            }
+            __syncwarp();                           // sp is overwritten by the next tile
+        }
+    }
+
     // Octree::QueryWithGradient (Octree.cpp:749-789) / FApproxWithGradient (:904-985): central differences with eps = 1e-4
     // in the leaf's local coordinate, gradient normalised. One thread per point, generic-degree loops (not a hot path).
     __global__ void __launch_bounds__(256)

@@ -198,30 +198,9 @@ namespace hpsdf
     __device__ __noinline__ void rayNormal(const double* __restrict__ coeffs, int degree, int depth, const double (&u)[3],
                                            const RootMap& map, const uint32_t* __restrict__ bidx, double (&nrm)[3])
     {
-        double l[3][kMaxDegree + 1], dl[3][kMaxDegree + 1];
-        for (int a = 0; a < 3; ++a)
-        {
-            l[a][0] = c_nl[0][depth]; dl[a][0] = 0.0;
-            double m2 = 0.0, m1 = 1.0, d2 = 0.0, d1 = 0.0;
-            for (int j = 1; j <= degree; ++j)
-            {
-                const double r0 = c_rec[j][0], r1 = c_rec[j][1];
-                const double v = r0 * u[a] * m1 - r1 * m2, dv = r0 * (m1 + u[a] * d1) - r1 * d2;
-                m2 = m1; m1 = v; d2 = d1; d1 = dv;
-                l[a][j] = v * c_nl[j][depth]; dl[a][j] = dv * c_nl[j][depth];
-            }
-        }
-        double g[3] = { 0.0, 0.0, 0.0 };
-        const int nc = coeffCount(degree);
-        for (int i = 0; i < nc; ++i)
-        {
-            const uint32_t abc = __ldg(bidx + i);
-            const int x = abc & 0xFF, y = (abc >> 8) & 0xFF, z = (abc >> 16) & 0xFF;
-            const double c = __ldg(coeffs + i);
-            g[0] = fma(c, (dl[0][x] * l[1][y]) * l[2][z], g[0]);
-            g[1] = fma(c, (l[0][x] * dl[1][y]) * l[2][z], g[1]);
-            g[2] = fma(c, (l[0][x] * l[1][y]) * dl[2][z], g[2]);
-        }
+        LeafDerivs d;
+        leafDerivsGeneric<1>(coeffs, degree, depth, u, bidx, d);
+        double (&g)[3] = d.g;
         const double scale = (double)(2u << depth);
         for (int a = 0; a < 3; ++a) g[a] *= scale * map.invSizes[a];
         const double n = sqrt(g[0] * g[0] + (g[1] * g[1] + g[2] * g[2]));

@@ -223,6 +223,22 @@ HPSDF_API hpsdf_status hpsdf_query_device(const hpsdf_octree* tree, const double
 /* Octree::QueryWithGradient (Octree.cpp:749-789, 904-985): value + unit central-difference gradient. */
 HPSDF_API hpsdf_status hpsdf_query_with_gradient(const hpsdf_octree* tree, const double* xyz, size_t n, double* out, double* unit_grad);
 
+/* Value and exact derivatives of the field hpsdf_query evaluates (DESIGN.md §13; no counterpart in the reference). For each
+ * point, Query's leaf and local coordinate u (same root map, f32 containment test and descent) give F(x) = P_leaf(u(x)),
+ * u_a = (p_a - c_a) 2^(depth+1), p_a = (x_a - centre_a) invSizes_a with Query's f32-rounded invSizes; s_a = 2^(depth+1) invSizes_a.
+ *   value[i]        = hpsdf_query's value, bit for bit (DBL_MAX outside the root);
+ *   grad[3i + a]    = dP/du_a s_a: the gradient in user space, NOT normalised;
+ *   hess[6i + k]    = d2P/du_a du_b s_a s_b in the order xx, xy, xz, yy, yz, zz; hess may be NULL (not computed).
+ * Outside the root grad and hess are 0. F is not continuous across leaf faces: at a point on a face the derivatives are
+ * those of the leaf Query picks (one-sided). xyz = n x 3 f64 (AoS), HOST pointers; blocks the calling thread.
+ * HPSDF_ERR_NO_DEVICE without a GPU; HPSDF_ERR_INVALID_ARG for a null tree, or a null xyz, value or grad when n > 0. */
+HPSDF_API hpsdf_status hpsdf_query_derivatives(const hpsdf_octree* tree, const double* xyz, size_t n, double* value, double* grad,
+                                               double* hess);
+/* Same with DEVICE pointers, asynchronous on `stream`; the current device must be the tree's (HPSDF_ERR_INVALID_ARG otherwise).
+ * d_xyz needs 8-byte alignment only. */
+HPSDF_API hpsdf_status hpsdf_query_derivatives_device(const hpsdf_octree* tree, const double* d_xyz, size_t n, double* d_value,
+                                                      double* d_grad, double* d_hess, void* stream);
+
 /* Octree::QueryRay (Octree.cpp:705-746, Ray.cpp:5-65) for n rays: origins / directions n x 3 f64, hit n bytes (1 = the march
  * reached a field value below 1e-4 within 200 steps and t_max), t n f64 (the reference stores the last field value there).
  * Statement-by-statement mirror of the reference, see query_kernels.cuh for what that implies outside the default root box. */

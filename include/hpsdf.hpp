@@ -5,7 +5,8 @@
 //     SDF::Octree                 Include/HP/Octree.h:36-86        Create / Query / QueryWithGradient / QueryRay / UnionSDF /
 //                                                                  SubtractSDF / IntersectSDF / Clear / FromMemoryBlock /
 //                                                                  ToMemoryBlock / GetRootAABB, copy + move; plus
-//                                                                  ExtractIsosurface / Raycast / RaycastDevice (no
+//                                                                  ExtractIsosurface / Raycast / RaycastDevice /
+//                                                                  QueryDerivatives / QueryDerivativesDevice (no
 //                                                                  counterpart in the reference)
 //     MemoryBlock                 Include/Utility/MemoryBlock.h:5-9
 //
@@ -232,6 +233,19 @@ namespace SDF
                            double* dTHit_, double* dNormals_, void* stream_) const
         {
             check(hpsdf_raycast_device(need(), dOrigins_, dDirections_, n_, tMin_, tMax_, iso_, dTHit_, dNormals_, stream_));
+        }
+
+        /// Query's value with the exact gradient and, when hess_ is not nullptr, Hessian (xx, xy, xz, yy, yz, zz) of the hit leaf's
+        /// polynomial in user space, not normalised; 0 outside the root (hpsdf_query_derivatives). Host pointers, n_ x 3 points.
+        void QueryDerivatives(const double* xyz_, size_t n_, double* value_, double* grad_, double* hess_ = nullptr) const
+        {
+            check(hpsdf_query_derivatives(need(), xyz_, n_, value_, grad_, hess_));
+        }
+
+        /// QueryDerivatives with device pointers, asynchronous on stream_ (hpsdf_query_derivatives_device).
+        void QueryDerivativesDevice(const double* dXyz_, size_t n_, double* dValue_, double* dGrad_, double* dHess_, void* stream_) const
+        {
+            check(hpsdf_query_derivatives_device(need(), dXyz_, n_, dValue_, dGrad_, dHess_, stream_));
         }
 
         /// The level set F = iso_ as a triangle mesh (hpsdf_extract_isosurface): marching tetrahedra over resolution_ cells per axis
