@@ -22,6 +22,22 @@ namespace
         return HPSDF_OK;
     }
 
+    hpsdf_status noDevice()
+    {
+        setLastError("no CUDA device available: this library has no CPU path");
+        return HPSDF_ERR_NO_DEVICE;
+    }
+
+    // The _device entry points launch with the tree's device pointers on the caller's stream, which belongs to the current
+    // device: that must be the tree's.
+    hpsdf_status onTreeDevice(const hpsdf_octree* tree, const char* fn)
+    {
+        int cur = -1;
+        if (cudaGetDevice(&cur) == cudaSuccess && cur == tree->device) return HPSDF_OK;
+        setLastError(std::string(fn) + ": the current CUDA device is not the tree's device");
+        return HPSDF_ERR_INVALID_ARG;
+    }
+
     hpsdf_build_opts normalisedOpts(const hpsdf_build_opts* in)
     {
         hpsdf_build_opts o;
@@ -117,16 +133,9 @@ extern "C"
         if (st != HPSDF_OK) return st;
         SdfProgramDev dp;
         if ((st = resolveProgram(prog, ctx->device, dp)) != HPSDF_OK) return st;
-        if (!n) return HPSDF_OK;
-        double *dIn = nullptr, *dOut = nullptr;
-        HPSDF_CUDA(cudaMalloc((void**)&dIn, n * 24));
-        cudaError_t e = cudaMalloc((void**)&dOut, n * 8);
-        if (e == cudaSuccess) e = cudaMemcpy(dIn, xyz, n * 24, cudaMemcpyHostToDevice);
-        if (e == cudaSuccess) e = launchSdfEval(dp, dIn, n, dOut, nullptr);
-        if (e == cudaSuccess) e = cudaMemcpy(out, dOut, n * 8, cudaMemcpyDeviceToHost);
-        cudaFree(dIn); cudaFree(dOut);
-        if (e != cudaSuccess) return failCuda(e, "hpsdf_sdf_eval");
-        return HPSDF_OK;
+        return stageHostBatch(*ctx, n, { { xyz, 24 } }, { { out, 8 } },
+                              [&](char* const* in, char* const* o, size_t m, cudaStream_t s)
+                              { return launchSdfEval(dp, (const double*)in[0], m, (double*)o[0], s); }, "hpsdf_sdf_eval");
     }
 
     HPSDF_API hpsdf_status hpsdf_create(const hpsdf_config* cfg, const hpsdf_build_opts* opts, const hpsdf_sdf_program* prog, hpsdf_octree** out)
@@ -152,16 +161,16 @@ extern "C"
     HPSDF_API hpsdf_status hpsdf_query(const hpsdf_octree* tree, const double* xyz, size_t n, double* out)
     {
         if (!tree || (n && (!xyz || !out))) { setLastError("null pointer"); return HPSDF_ERR_INVALID_ARG; }
-        return queryHost(*const_cast<hpsdf_octree*>(tree), xyz, n, out);
+        return stageHostBatch(*tree->ctx, n, { { xyz, 24 } }, { { out, 8 } },
+                              [&](char* const* in, char* const* o, size_t m, cudaStream_t s)
+                              { return launchQuery(tree->view, (const double*)in[0], m, (double*)o[0], tree->ctx->smCount, s); }, "hpsdf_query");
     }
 
     HPSDF_API hpsdf_status hpsdf_query_device(const hpsdf_octree* tree, const double* d_xyz, size_t n, double* d_out, void* stream)
     {
         if (!tree || (n && (!d_xyz || !d_out))) { setLastError("null pointer"); return HPSDF_ERR_INVALID_ARG; }
-        // the kernel reads the tree's device pointers: it must run on the tree's device (the caller's stream belongs to it)
-        int cur = -1;
-        if (cudaGetDevice(&cur) != cudaSuccess || cur != tree->device)
-        { setLastError("hpsdf_query_device: the current CUDA device is not the tree's device"); return HPSDF_ERR_INVALID_ARG; }
+        hpsdf_status st = onTreeDevice(tree, "hpsdf_query_device");
+        if (st != HPSDF_OK) return st;
         HPSDF_CUDA(launchQuery(tree->view, d_xyz, n, d_out, tree->ctx->smCount, (cudaStream_t)stream));
         return HPSDF_OK;
     }
@@ -169,25 +178,19 @@ extern "C"
     HPSDF_API hpsdf_status hpsdf_query_with_gradient(const hpsdf_octree* tree, const double* xyz, size_t n, double* out, double* unit_grad)
     {
         if (!tree || (n && (!xyz || !out || !unit_grad))) { setLastError("null pointer"); return HPSDF_ERR_INVALID_ARG; }
-        if (!n) return HPSDF_OK;
-        HPSDF_CUDA(cudaSetDevice(tree->device));
-        double *dIn = nullptr, *dOut = nullptr, *dG = nullptr;
-        HPSDF_CUDA(cudaMalloc((void**)&dIn, n * 24));
-        cudaError_t e = cudaMalloc((void**)&dOut, n * 8);
-        if (e == cudaSuccess) e = cudaMalloc((void**)&dG, n * 24);
-        if (e == cudaSuccess) e = cudaMemset(dG, 0, n * 24);
-        if (e == cudaSuccess) e = cudaMemcpy(dIn, xyz, n * 24, cudaMemcpyHostToDevice);
-        if (e == cudaSuccess) e = launchQueryGradient(tree->view, dIn, n, dOut, dG, nullptr);
-        if (e == cudaSuccess) e = cudaMemcpy(out, dOut, n * 8, cudaMemcpyDeviceToHost);
-        if (e == cudaSuccess) e = cudaMemcpy(unit_grad, dG, n * 24, cudaMemcpyDeviceToHost);
-        cudaFree(dIn); cudaFree(dOut); cudaFree(dG);
-        if (e != cudaSuccess) return failCuda(e, "hpsdf_query_with_gradient");
-        return HPSDF_OK;
+        return stageHostBatch(*tree->ctx, n, { { xyz, 24 } }, { { out, 8 }, { unit_grad, 24 } },
+                              [&](char* const* in, char* const* o, size_t m, cudaStream_t s)
+                              {
+                                  // the kernel writes no gradient outside the root, and the staging buffer holds an earlier chunk's
+                                  cudaError_t e = cudaMemsetAsync(o[1], 0, m * 24, s);
+                                  if (e != cudaSuccess) return e;
+                                  return launchQueryGradient(tree->view, (const double*)in[0], m, (double*)o[0], (double*)o[1], s);
+                              }, "hpsdf_query_with_gradient");
     }
 
     static hpsdf_status derivativesArgs(const hpsdf_octree* tree, const void* xyz, size_t n, const void* value, const void* grad)
     {
-        if (hpsdf_device_count() == 0) { setLastError("no CUDA device available: this library has no CPU path"); return HPSDF_ERR_NO_DEVICE; }
+        if (hpsdf_device_count() == 0) return noDevice();
         if (!tree || (n && (!xyz || !value || !grad))) { setLastError("null pointer"); return HPSDF_ERR_INVALID_ARG; }
         return HPSDF_OK;
     }
@@ -196,31 +199,21 @@ extern "C"
                                                    double* hess)
     {
         hpsdf_status st = derivativesArgs(tree, xyz, n, value, grad);
-        if (st != HPSDF_OK || !n) return st;
-        HPSDF_CUDA(cudaSetDevice(tree->device));
-        double *dIn = nullptr, *dV = nullptr, *dG = nullptr, *dH = nullptr;
-        HPSDF_CUDA(cudaMalloc((void**)&dIn, n * 24));
-        cudaError_t e = cudaMalloc((void**)&dV, n * 8);
-        if (e == cudaSuccess) e = cudaMalloc((void**)&dG, n * 24);
-        if (e == cudaSuccess && hess) e = cudaMalloc((void**)&dH, n * 48);
-        if (e == cudaSuccess) e = cudaMemcpy(dIn, xyz, n * 24, cudaMemcpyHostToDevice);
-        if (e == cudaSuccess) e = launchQueryDerivatives(tree->view, dIn, n, dV, dG, dH, tree->ctx->smCount, nullptr);
-        if (e == cudaSuccess) e = cudaMemcpy(value, dV, n * 8, cudaMemcpyDeviceToHost);
-        if (e == cudaSuccess) e = cudaMemcpy(grad, dG, n * 24, cudaMemcpyDeviceToHost);
-        if (e == cudaSuccess && hess) e = cudaMemcpy(hess, dH, n * 48, cudaMemcpyDeviceToHost);
-        cudaFree(dIn); cudaFree(dV); cudaFree(dG); cudaFree(dH);
-        if (e != cudaSuccess) return failCuda(e, "hpsdf_query_derivatives");
-        return HPSDF_OK;
+        if (st != HPSDF_OK) return st;
+        return stageHostBatch(*tree->ctx, n, { { xyz, 24 } }, { { value, 8 }, { grad, 24 }, { hess, 48 } },
+                              [&](char* const* in, char* const* o, size_t m, cudaStream_t s)
+                              {
+                                  return launchQueryDerivatives(tree->view, (const double*)in[0], m, (double*)o[0], (double*)o[1], (double*)o[2],
+                                                                tree->ctx->smCount, s);
+                              }, "hpsdf_query_derivatives");
     }
 
     HPSDF_API hpsdf_status hpsdf_query_derivatives_device(const hpsdf_octree* tree, const double* d_xyz, size_t n, double* d_value,
                                                           double* d_grad, double* d_hess, void* stream)
     {
         hpsdf_status st = derivativesArgs(tree, d_xyz, n, d_value, d_grad);
+        if (st == HPSDF_OK) st = onTreeDevice(tree, "hpsdf_query_derivatives_device");
         if (st != HPSDF_OK) return st;
-        int cur = -1;
-        if (cudaGetDevice(&cur) != cudaSuccess || cur != tree->device)
-        { setLastError("hpsdf_query_derivatives_device: the current CUDA device is not the tree's device"); return HPSDF_ERR_INVALID_ARG; }
         HPSDF_CUDA(launchQueryDerivatives(tree->view, d_xyz, n, d_value, d_grad, d_hess, tree->ctx->smCount, (cudaStream_t)stream));
         return HPSDF_OK;
     }
@@ -229,28 +222,18 @@ extern "C"
                                            unsigned char* hit, double* t)
     {
         if (!tree || (n && (!origins || !directions || !hit || !t))) { setLastError("null pointer"); return HPSDF_ERR_INVALID_ARG; }
-        if (!n) return HPSDF_OK;
-        HPSDF_CUDA(cudaSetDevice(tree->device));
-        double *dO = nullptr, *dD = nullptr, *dT = nullptr;
-        unsigned char* dH = nullptr;
-        HPSDF_CUDA(cudaMalloc((void**)&dO, n * 24));
-        cudaError_t e = cudaMalloc((void**)&dD, n * 24);
-        if (e == cudaSuccess) e = cudaMalloc((void**)&dT, n * 8);
-        if (e == cudaSuccess) e = cudaMalloc((void**)&dH, n);
-        if (e == cudaSuccess) e = cudaMemcpy(dO, origins, n * 24, cudaMemcpyHostToDevice);
-        if (e == cudaSuccess) e = cudaMemcpy(dD, directions, n * 24, cudaMemcpyHostToDevice);
-        if (e == cudaSuccess) e = launchQueryRay(tree->view, dO, dD, n, t_max, dH, dT, nullptr);
-        if (e == cudaSuccess) e = cudaMemcpy(hit, dH, n, cudaMemcpyDeviceToHost);
-        if (e == cudaSuccess) e = cudaMemcpy(t, dT, n * 8, cudaMemcpyDeviceToHost);
-        cudaFree(dO); cudaFree(dD); cudaFree(dT); cudaFree(dH);
-        if (e != cudaSuccess) return failCuda(e, "hpsdf_query_ray");
-        return HPSDF_OK;
+        return stageHostBatch(*tree->ctx, n, { { origins, 24 }, { directions, 24 } }, { { hit, 1 }, { t, 8 } },
+                              [&](char* const* in, char* const* o, size_t m, cudaStream_t s)
+                              {
+                                  return launchQueryRay(tree->view, (const double*)in[0], (const double*)in[1], m, t_max, (unsigned char*)o[0],
+                                                        (double*)o[1], s);
+                              }, "hpsdf_query_ray");
     }
 
     static hpsdf_status raycastArgs(const hpsdf_octree* tree, const void* origins, const void* directions, size_t n, double t_min,
                                     double t_max, double iso, const void* t_hit, const char* fn)
     {
-        if (hpsdf_device_count() == 0) { setLastError("no CUDA device available: this library has no CPU path"); return HPSDF_ERR_NO_DEVICE; }
+        if (hpsdf_device_count() == 0) return noDevice();
         if (!tree || (n && (!origins || !directions || !t_hit))) { setLastError("null pointer"); return HPSDF_ERR_INVALID_ARG; }
         if (!std::isfinite(t_min) || !std::isfinite(iso) || !(t_max >= t_min))
         { setLastError(std::string(fn) + ": t_min and iso must be finite and t_max >= t_min"); return HPSDF_ERR_INVALID_ARG; }
@@ -261,31 +244,21 @@ extern "C"
                                          double t_max, double iso, double* t_hit, double* normals)
     {
         hpsdf_status st = raycastArgs(tree, origins, directions, n, t_min, t_max, iso, t_hit, "hpsdf_raycast");
-        if (st != HPSDF_OK || !n) return st;
-        HPSDF_CUDA(cudaSetDevice(tree->device));
-        double *dO = nullptr, *dD = nullptr, *dT = nullptr, *dN = nullptr;
-        HPSDF_CUDA(cudaMalloc((void**)&dO, n * 24));
-        cudaError_t e = cudaMalloc((void**)&dD, n * 24);
-        if (e == cudaSuccess) e = cudaMalloc((void**)&dT, n * 8);
-        if (e == cudaSuccess && normals) e = cudaMalloc((void**)&dN, n * 24);
-        if (e == cudaSuccess) e = cudaMemcpy(dO, origins, n * 24, cudaMemcpyHostToDevice);
-        if (e == cudaSuccess) e = cudaMemcpy(dD, directions, n * 24, cudaMemcpyHostToDevice);
-        if (e == cudaSuccess) e = launchRaycast(tree->view, dO, dD, n, t_min, t_max, iso, dT, dN, tree->ctx->smCount, nullptr);
-        if (e == cudaSuccess) e = cudaMemcpy(t_hit, dT, n * 8, cudaMemcpyDeviceToHost);
-        if (e == cudaSuccess && normals) e = cudaMemcpy(normals, dN, n * 24, cudaMemcpyDeviceToHost);
-        cudaFree(dO); cudaFree(dD); cudaFree(dT); cudaFree(dN);
-        if (e != cudaSuccess) return failCuda(e, "hpsdf_raycast");
-        return HPSDF_OK;
+        if (st != HPSDF_OK) return st;
+        return stageHostBatch(*tree->ctx, n, { { origins, 24 }, { directions, 24 } }, { { t_hit, 8 }, { normals, 24 } },
+                              [&](char* const* in, char* const* o, size_t m, cudaStream_t s)
+                              {
+                                  return launchRaycast(tree->view, (const double*)in[0], (const double*)in[1], m, t_min, t_max, iso, (double*)o[0],
+                                                       (double*)o[1], tree->ctx->smCount, s);
+                              }, "hpsdf_raycast");
     }
 
     HPSDF_API hpsdf_status hpsdf_raycast_device(const hpsdf_octree* tree, const double* d_origins, const double* d_directions, size_t n,
                                                 double t_min, double t_max, double iso, double* d_t_hit, double* d_normals, void* stream)
     {
         hpsdf_status st = raycastArgs(tree, d_origins, d_directions, n, t_min, t_max, iso, d_t_hit, "hpsdf_raycast_device");
+        if (st == HPSDF_OK) st = onTreeDevice(tree, "hpsdf_raycast_device");
         if (st != HPSDF_OK) return st;
-        int cur = -1;
-        if (cudaGetDevice(&cur) != cudaSuccess || cur != tree->device)
-        { setLastError("hpsdf_raycast_device: the current CUDA device is not the tree's device"); return HPSDF_ERR_INVALID_ARG; }
         HPSDF_CUDA(launchRaycast(tree->view, d_origins, d_directions, n, t_min, t_max, iso, d_t_hit, d_normals, tree->ctx->smCount,
                                  (cudaStream_t)stream));
         return HPSDF_OK;
@@ -295,7 +268,7 @@ extern "C"
                                                     const double box_max[3], double iso, size_t* n_vertices, float** vertices,
                                                     size_t* n_triangles, uint32_t** tri_indices)
     {
-        if (hpsdf_device_count() == 0) { setLastError("no CUDA device available: this library has no CPU path"); return HPSDF_ERR_NO_DEVICE; }
+        if (hpsdf_device_count() == 0) return noDevice();
         if (!tree || !resolution || !n_vertices || !vertices || !n_triangles || !tri_indices) { setLastError("null pointer"); return HPSDF_ERR_INVALID_ARG; }
         *n_vertices = 0; *vertices = nullptr; *n_triangles = 0; *tri_indices = nullptr;
         if (!box_min != !box_max) { setLastError("hpsdf_extract_isosurface: give both box corners or neither"); return HPSDF_ERR_INVALID_ARG; }
@@ -627,7 +600,7 @@ extern "C"
                                                        double* d_xyz, void* stream)
     {
         if (n && (!lo || !hi || !d_xyz)) { setLastError("null pointer"); return HPSDF_ERR_INVALID_ARG; }
-        if (hpsdf_device_count() == 0) { setLastError("no CUDA device available: this library has no CPU path"); return HPSDF_ERR_NO_DEVICE; }
+        if (hpsdf_device_count() == 0) return noDevice();
         HPSDF_CUDA(launchUniformPoints(seed, first_index, n, lo, hi, d_xyz, (cudaStream_t)stream));
         return HPSDF_OK;
     }

@@ -1,6 +1,9 @@
 // device_ctx.h — per-device tables and the host-callable launchers of kernels.cu.
 #pragma once
 #include <cuda_runtime.h>
+#include <functional>
+#include <initializer_list>
+#include <mutex>
 #include <string>
 #include "hp_common.h"
 
@@ -77,6 +80,15 @@ namespace hpsdf
         cudaEvent_t          evFork = nullptr, evJoin[4] = { nullptr, nullptr, nullptr, nullptr };
     };
 
+    // Device side of the host-array entry points (stageHostBatch): chunk k runs on streams[k % 3] in buf[k % 3], which holds
+    // that chunk's inputs and outputs. Its own mutex, so that a running build does not block host queries.
+    struct HostStaging
+    {
+        std::mutex      m;
+        cudaStream_t    streams[3] = { nullptr, nullptr, nullptr };
+        DeviceBuf<char> buf[3];
+    };
+
     struct DeviceCtx
     {
         int           device = -1;
@@ -86,6 +98,7 @@ namespace hpsdf
         const double* glRoots = nullptr;      // all 64 rules, rule n at n(n-1)/2, ascending nodes
         const double* glWeights = nullptr;
         BuildWorkspace ws;
+        HostStaging    staging;
         void*          wsMutex = nullptr;     // std::mutex*, serialises builds on this device
         void*          blobCache = nullptr;   // released tree allocations kept for reuse (context.cpp)
         uint32_t*      matchCount = nullptr;  // 3 x 13 x 13: entries of an analytic face block per (dim, degree, degree) (continuity.cpp)
@@ -106,6 +119,17 @@ namespace hpsdf
 
     // Lazily creates the context of `device` (uploads tables and constant memory). nullptr + err on failure.
     DeviceCtx* getDeviceCtx(int device, std::string& err);
+
+    // One host array of a batch of independent items: `bytes` per item. A null HostOut::p is an absent optional output.
+    struct HostIn  { const void* p; size_t bytes; };
+    struct HostOut { void* p; size_t bytes; };
+    // Enqueues the work of m items on `stream`: dIn / dOut hold the device copies of the inputs / outputs in list order
+    // (nullptr for an absent output).
+    using StageLaunch = std::function<cudaError_t(char* const* dIn, char* const* dOut, size_t m, cudaStream_t stream)>;
+    // Runs `launch` over n items of host arrays in chunks on ctx.staging, and returns when every output is in host memory.
+    // A CUDA error is returned as failCuda(e, what). n == 0 touches nothing.
+    hpsdf_status stageHostBatch(DeviceCtx& ctx, size_t n, std::initializer_list<HostIn> in, std::initializer_list<HostOut> out,
+                                const StageLaunch& launch, const char* what);
 
     // kernels.cu
     void        uploadConstants();

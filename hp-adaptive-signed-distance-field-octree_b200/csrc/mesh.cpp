@@ -211,17 +211,9 @@ extern "C"
     HPSDF_API hpsdf_status hpsdf_mesh_signed_distance(const hpsdf_mesh* mesh, const float* xyz, size_t n, float* out)
     {
         if (!mesh || (n && (!xyz || !out))) { setLastError("null pointer"); return HPSDF_ERR_INVALID_ARG; }
-        if (!n) return HPSDF_OK;
-        HPSDF_CUDA(cudaSetDevice(mesh->device));
-        float *dIn = nullptr, *dOut = nullptr;
-        HPSDF_CUDA(cudaMalloc((void**)&dIn, n * 12));
-        cudaError_t e = cudaMalloc((void**)&dOut, n * 4);
-        if (e == cudaSuccess) e = cudaMemcpy(dIn, xyz, n * 12, cudaMemcpyHostToDevice);
-        if (e == cudaSuccess) e = launchMeshDistance(mesh->dView, dIn, n, dOut, nullptr);
-        if (e == cudaSuccess) e = cudaMemcpy(out, dOut, n * 4, cudaMemcpyDeviceToHost);
-        cudaFree(dIn); cudaFree(dOut);
-        if (e != cudaSuccess) return failCuda(e, "hpsdf_mesh_signed_distance");
-        return HPSDF_OK;
+        return stageHostBatch(*mesh->ctx, n, { { xyz, 12 } }, { { out, 4 } },
+                              [&](char* const* in, char* const* o, size_t m, cudaStream_t s)
+                              { return launchMeshDistance(mesh->dView, (const float*)in[0], m, (float*)o[0], s); }, "hpsdf_mesh_signed_distance");
     }
 
     HPSDF_API hpsdf_status hpsdf_mesh_aabb(const hpsdf_mesh* mesh, float mn[3], float mx[3])

@@ -1,7 +1,6 @@
 // octree.h — host-side objects behind the C ABI: the octree handle (hpsdf_octree), meshes, communicators.
 #pragma once
 #include <cuda_runtime.h>
-#include <mutex>
 #include <string>
 #include <vector>
 #include "hp_common.h"
@@ -70,13 +69,6 @@ struct hpsdf_octree
     double              cutTotalBeforeLast = 0.0, cutCheck = 0.0;
     bool                cutLogPending = false, cutQueueEmpty = false;
 
-    // scratch of the host-pointer Query path
-    std::mutex          queryMutex;
-    double*             dScratchIn[3]  = { nullptr, nullptr, nullptr };
-    double*             dScratchOut[3] = { nullptr, nullptr, nullptr };
-    size_t              scratchPts = 0;
-    cudaStream_t        qStreams[3] = { nullptr, nullptr, nullptr };
-
     ~hpsdf_octree();
 };
 
@@ -105,7 +97,6 @@ namespace hpsdf
     hpsdf_status  continuityPostProcess(hpsdf_octree& t, const hpsdf_build_opts& opts, cudaStream_t stream);
     hpsdf_status  toMemoryBlock(const hpsdf_octree& t, size_t* size, void** ptr);
     hpsdf_status  fromMemoryBlock(hpsdf_octree& t, const void* ptr, size_t size);
-    hpsdf_status  queryHost(hpsdf_octree& t, const double* xyz, size_t n, double* out);
     const std::string& lastError();
     const DeviceMeshView* meshDeviceView(const hpsdf_mesh* m);      // mesh.cpp
     int           meshDevice(const hpsdf_mesh* m);

@@ -12,11 +12,6 @@ hpsdf_octree::~hpsdf_octree()
 {
     if (ctx) { cudaSetDevice(device); hpsdf::releaseBlob(*ctx, dBlob, dBlobBytes); }
     else cudaFree(dBlob);
-    for (int i = 0; i < 3; ++i)
-    {
-        cudaFree(dScratchIn[i]); cudaFree(dScratchOut[i]);
-        if (qStreams[i]) cudaStreamDestroy(qStreams[i]);
-    }
 }
 
 namespace hpsdf
@@ -286,40 +281,6 @@ namespace hpsdf
             memcpy(&n.child, q, 8); memcpy(n.mn, q + 8, 12); memcpy(n.mx, q + 20, 12);
             memcpy(&n.cstart, q + 32, 8); n.degree = q[40]; n.depth = q[48];
         }
-        return HPSDF_OK;
-    }
-
-    // Octree::Query for host arrays: chunks of points go H2D -> kernel -> D2H on three rotating streams so the copies of
-    // one chunk overlap the kernel of another (PCIe is full duplex).
-    hpsdf_status queryHost(hpsdf_octree& t, const double* xyz, size_t n, double* out)
-    {
-        if (!n) return HPSDF_OK;
-        std::lock_guard<std::mutex> lock(t.queryMutex);
-        HPSDF_CUDA(cudaSetDevice(t.device));
-        // at least 8 chunks for a large call, so the H2D copy of one chunk overlaps the kernel and the D2H copy of the previous
-        // ones (a single 2^22-point chunk serialised the three: 1.55e9 points/s where the H2D engine alone allows 2.2e9)
-        const size_t chunk = std::min<size_t>(std::max<size_t>((n + 7) / 8, (size_t)1 << 16), (size_t)1 << 22);
-        if (t.scratchPts < chunk)
-        {
-            for (int i = 0; i < 3; ++i)
-            {
-                cudaFree(t.dScratchIn[i]); cudaFree(t.dScratchOut[i]);
-                t.dScratchIn[i] = t.dScratchOut[i] = nullptr;
-                HPSDF_CUDA(cudaMalloc((void**)&t.dScratchIn[i], chunk * 24));
-                HPSDF_CUDA(cudaMalloc((void**)&t.dScratchOut[i], chunk * 8));
-                if (!t.qStreams[i]) HPSDF_CUDA(cudaStreamCreateWithFlags(&t.qStreams[i], cudaStreamNonBlocking));
-            }
-            t.scratchPts = chunk;
-        }
-        int s = 0;
-        for (size_t off = 0; off < n; off += chunk, s = (s + 1) % 3)
-        {
-            const size_t m = std::min(chunk, n - off);
-            HPSDF_CUDA(cudaMemcpyAsync(t.dScratchIn[s], xyz + 3 * off, m * 24, cudaMemcpyHostToDevice, t.qStreams[s]));
-            HPSDF_CUDA(launchQuery(t.view, t.dScratchIn[s], m, t.dScratchOut[s], t.ctx->smCount, t.qStreams[s]));
-            HPSDF_CUDA(cudaMemcpyAsync(out + off, t.dScratchOut[s], m * 8, cudaMemcpyDeviceToHost, t.qStreams[s]));
-        }
-        for (int i = 0; i < 3; ++i) HPSDF_CUDA(cudaStreamSynchronize(t.qStreams[i]));
         return HPSDF_OK;
     }
 }
