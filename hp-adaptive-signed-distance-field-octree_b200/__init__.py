@@ -129,6 +129,7 @@ EXPORTS = [
     "hpsdf_comm_destroy", "hpsdf_shard_range", "hpsdf_set_jit", "hpsdf_jit_compile_check", "hpsdf_query_ray",
     "hpsdf_get_config", "hpsdf_get_device", "hpsdf_uniform_points_device", "hpsdf_extract_isosurface",
     "hpsdf_raycast", "hpsdf_raycast_device", "hpsdf_query_derivatives", "hpsdf_query_derivatives_device",
+    "hpsdf_query_bounds", "hpsdf_query_bounds_device",
 ]
 
 _lib = None
@@ -174,6 +175,8 @@ def lib():
     L.hpsdf_raycast_device.argtypes = [vp, vp, vp, sz, dbl, dbl, dbl, vp, vp, vp]
     L.hpsdf_query_derivatives.argtypes = [vp, vp, sz, vp, vp, vp]
     L.hpsdf_query_derivatives_device.argtypes = [vp, vp, sz, vp, vp, vp, vp]
+    L.hpsdf_query_bounds.argtypes = [vp, vp, vp, sz, vp, vp]
+    L.hpsdf_query_bounds_device.argtypes = [vp, vp, vp, sz, vp, vp, vp]
     L.hpsdf_extract_isosurface.argtypes = [vp, vp, vp, vp, dbl, C.POINTER(sz), C.POINTER(vp), C.POINTER(sz), C.POINTER(vp)]
     L.hpsdf_to_memory_block.argtypes = [vp, C.POINTER(sz), C.POINTER(vp)]
     L.hpsdf_from_memory_block.argtypes = [vp, sz, i32, C.POINTER(vp)]
@@ -369,6 +372,23 @@ class Octree:
         """QueryDerivatives with device pointers (e.g. torch tensors' data_ptr()), asynchronous on `stream` (cudaStream_t as
         int); d_hess = None skips the Hessians."""
         _check(lib().hpsdf_query_derivatives_device(self._h, d_xyz, n, d_value, d_grad, d_hess, stream))
+
+    def QueryBounds(self, box_lo, box_hi):
+        """Certified bounds of Query over closed boxes [box_lo[i], box_hi[i]] ((n,3) float64 each; hpsdf_query_bounds, DESIGN §14)
+        -> (f_lo (n,), f_hi (n,)) with f_lo <= Query(x) <= f_hi for every x in box i. f_hi is DBL_MAX when part of the box is
+        outside the root, both are when all of it is; a NaN or inverted box gives NaN."""
+        lo = np.ascontiguousarray(box_lo, np.float64).reshape(-1, 3)
+        hi = np.ascontiguousarray(box_hi, np.float64).reshape(-1, 3)
+        if len(lo) != len(hi):
+            raise HpsdfError(ERR_INVALID_ARG, "box_lo and box_hi differ in length")
+        f_lo = np.empty(len(lo), np.float64)
+        f_hi = np.empty(len(lo), np.float64)
+        _check(lib().hpsdf_query_bounds(self._h, lo.ctypes.data, hi.ctypes.data, len(lo), f_lo.ctypes.data, f_hi.ctypes.data))
+        return f_lo, f_hi
+
+    def QueryBoundsDevice(self, d_lo, d_hi, n, d_flo, d_fhi, stream=None):
+        """QueryBounds with device pointers (e.g. torch tensors' data_ptr()), asynchronous on `stream` (cudaStream_t as int)."""
+        _check(lib().hpsdf_query_bounds_device(self._h, d_lo, d_hi, n, d_flo, d_fhi, stream))
 
     def QueryTorch(self, x):
         """Query as a differentiable torch function: x is a contiguous CUDA float64 (n,3) tensor on the tree's device, the

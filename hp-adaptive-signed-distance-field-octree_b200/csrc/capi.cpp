@@ -218,6 +218,40 @@ extern "C"
         return HPSDF_OK;
     }
 
+    static hpsdf_status boundsArgs(const hpsdf_octree* tree, const void* lo, const void* hi, size_t n, const void* fLo, const void* fHi)
+    {
+        if (hpsdf_device_count() == 0) return noDevice();
+        if (!tree || (n && (!lo || !hi || !fLo || !fHi))) { setLastError("null pointer"); return HPSDF_ERR_INVALID_ARG; }
+        return HPSDF_OK;
+    }
+
+    HPSDF_API hpsdf_status hpsdf_query_bounds(const hpsdf_octree* tree, const double* box_lo, const double* box_hi, size_t n, double* f_lo,
+                                              double* f_hi)
+    {
+        hpsdf_status st = boundsArgs(tree, box_lo, box_hi, n, f_lo, f_hi);
+        if (st != HPSDF_OK || !n) return st;
+        const double2* table = nullptr;
+        if ((st = ensureBoundsTable(*const_cast<hpsdf_octree*>(tree), &table)) != HPSDF_OK) return st;
+        return stageHostBatch(*tree->ctx, n, { { box_lo, 24 }, { box_hi, 24 } }, { { f_lo, 8 }, { f_hi, 8 } },
+                              [&](char* const* in, char* const* o, size_t m, cudaStream_t s)
+                              {
+                                  return launchBounds(tree->view, table, (const double*)in[0], (const double*)in[1], m, (double*)o[0],
+                                                      (double*)o[1], tree->ctx->smCount, s);
+                              }, "hpsdf_query_bounds");
+    }
+
+    HPSDF_API hpsdf_status hpsdf_query_bounds_device(const hpsdf_octree* tree, const double* d_box_lo, const double* d_box_hi, size_t n,
+                                                     double* d_f_lo, double* d_f_hi, void* stream)
+    {
+        hpsdf_status st = boundsArgs(tree, d_box_lo, d_box_hi, n, d_f_lo, d_f_hi);
+        if (st == HPSDF_OK) st = onTreeDevice(tree, "hpsdf_query_bounds_device");
+        if (st != HPSDF_OK || !n) return st;
+        const double2* table = nullptr;
+        if ((st = ensureBoundsTable(*const_cast<hpsdf_octree*>(tree), &table)) != HPSDF_OK) return st;
+        HPSDF_CUDA(launchBounds(tree->view, table, d_box_lo, d_box_hi, n, d_f_lo, d_f_hi, tree->ctx->smCount, (cudaStream_t)stream));
+        return HPSDF_OK;
+    }
+
     HPSDF_API hpsdf_status hpsdf_query_ray(const hpsdf_octree* tree, const double* origins, const double* directions, size_t n, double t_max,
                                            unsigned char* hit, double* t)
     {

@@ -157,6 +157,11 @@ namespace hpsdf
     // hpsdf_raycast (raycast_kernels.cuh): first crossing of F = iso per ray; dNormals may be nullptr
     cudaError_t launchRaycast(const DeviceTreeView& view, const double* dOrigins, const double* dDirs, size_t n, double tMin, double tMax,
                               double iso, double* dT, double* dNormals, int smCount, cudaStream_t stream);
+    // hpsdf_query_bounds (bounds_kernels.cuh): the per-node enclosure table (dCells: 4 bytes per node of scratch), then the
+    // bounds of n boxes
+    cudaError_t launchBoundsTable(const DeviceTreeView& view, double2* dTable, uint32_t* dCells, cudaStream_t stream);
+    cudaError_t launchBounds(const DeviceTreeView& view, const double2* dTable, const double* dLo, const double* dHi, size_t n,
+                             double* dFLo, double* dFHi, int smCount, cudaStream_t stream);
     cudaError_t launchQueryGradient(const DeviceTreeView& view, const double* dXyz, size_t n, double* dOut, double* dGrad, cudaStream_t stream);
     // hpsdf_query_derivatives (query_kernels.cuh): value, gradient, and the Hessian when dHess is not nullptr
     cudaError_t launchQueryDerivatives(const DeviceTreeView& view, const double* dXyz, size_t n, double* dValue, double* dGrad,

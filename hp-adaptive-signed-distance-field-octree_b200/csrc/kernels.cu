@@ -25,6 +25,7 @@ namespace hpsdf
 #include "mesh_build.cuh"
 #include "isosurface_kernels.cuh"
 #include "raycast_kernels.cuh"
+#include "bounds_kernels.cuh"
 
 namespace hpsdf
 {
@@ -105,6 +106,35 @@ namespace hpsdf
     {
         if (!n) return cudaSuccess;
         raycastKernel<<<persistentGrid(n, 2, smCount), kQueryThreads, 0, stream>>>(view, dOrigins, dDirs, n, RayArgs{ tMin, tMax, iso }, dT, dNormals);
+        return cudaGetLastError();
+    }
+
+    cudaError_t launchBoundsTable(const DeviceTreeView& view, double2* dTable, uint32_t* dCells, cudaStream_t stream)
+    {
+        const unsigned blocks = (view.nNodes + 127) / 128;
+        cudaError_t e = cudaMemsetAsync(dCells, 0, 4, stream);                   // the root is cell (0, 0, 0)
+        for (int d = 0; d <= kMaxDepth && e == cudaSuccess; ++d)
+        {
+            boundsLeafTableKernel<<<blocks, 128, 0, stream>>>(view, d, dCells, dTable);
+            e = cudaGetLastError();
+        }
+        for (int d = kMaxDepth - 1; d >= 0 && e == cudaSuccess; --d)
+        {
+            boundsInternalTableKernel<<<blocks, 128, 0, stream>>>(view, d, dTable);
+            e = cudaGetLastError();
+        }
+        return e;
+    }
+
+    cudaError_t launchBounds(const DeviceTreeView& view, const double2* dTable, const double* dLo, const double* dHi, size_t n,
+                             double* dFLo, double* dFHi, int smCount, cudaStream_t stream)
+    {
+        if (!n) return cudaSuccess;
+        static int perSm = 0;
+        if (!perSm && cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSm, boundsKernel, kBoundsThreads, 0) != cudaSuccess) perSm = 1;
+        const unsigned grid = (unsigned)std::min((size_t)(smCount > 0 ? smCount : 148) * std::max(perSm, 1),
+                                                 (n + kBoundsThreads / 32 - 1) / (kBoundsThreads / 32));
+        boundsKernel<<<grid, kBoundsThreads, 0, stream>>>(view, dTable, dLo, dHi, n, dFLo, dFHi);
         return cudaGetLastError();
     }
 

@@ -1,6 +1,7 @@
 // octree.h — host-side objects behind the C ABI: the octree handle (hpsdf_octree), meshes, communicators.
 #pragma once
 #include <cuda_runtime.h>
+#include <mutex>
 #include <string>
 #include <vector>
 #include "hp_common.h"
@@ -61,6 +62,11 @@ struct hpsdf_octree
     double*             dLeafErr = nullptr;      // current error per node at termination (input of the cut-tie log)
     bool                logOnDevice = false;
 
+    // enclosure table of hpsdf_query_bounds (16 B per node, then 4 B per node of scratch), built on the first bounds query
+    std::mutex          boundsMutex;
+    void*               dBoundsBlob = nullptr;
+    size_t              dBoundsBytes = 0;
+
     hpsdf_build_stats   stats{};
     std::vector<hpsdf_decision_log_entry> decisionLog;
     std::vector<hpsdf_apply_log_entry>    applyLog;
@@ -81,6 +87,8 @@ namespace hpsdf
     size_t        paddedCoeffCount(const hpsdf_octree& t);
     // Host copy of the node array, read back from the device image if the build left it on the device.
     hpsdf_status  ensureHostNodes(hpsdf_octree& t);
+    // The enclosure table of hpsdf_query_bounds, built on the tree's device on first use (blocks until it is ready).
+    hpsdf_status  ensureBoundsTable(hpsdf_octree& t, const double2** table);
     // Completes the decision log of a device-scheduled build (the equal-error group at the termination cut).
     void          ensureDecisionLog(hpsdf_octree& t);
     // Fetches the apply log of a device-scheduled build.

@@ -10,8 +10,8 @@
 
 hpsdf_octree::~hpsdf_octree()
 {
-    if (ctx) { cudaSetDevice(device); hpsdf::releaseBlob(*ctx, dBlob, dBlobBytes); }
-    else cudaFree(dBlob);
+    if (ctx) { cudaSetDevice(device); hpsdf::releaseBlob(*ctx, dBlob, dBlobBytes); hpsdf::releaseBlob(*ctx, dBoundsBlob, dBoundsBytes); }
+    else { cudaFree(dBlob); cudaFree(dBoundsBlob); }
 }
 
 namespace hpsdf
@@ -47,6 +47,31 @@ namespace hpsdf
         t.dApplyLog = (hpsdf_apply_log_entry*)p; p += bLog;
         t.dLeafErr = (double*)p;
         t.imageValid = false; t.logOnDevice = false;
+        return HPSDF_OK;
+    }
+
+    hpsdf_status ensureBoundsTable(hpsdf_octree& t, const double2** table)
+    {
+        std::lock_guard<std::mutex> lock(t.boundsMutex);
+        if (!t.dBoundsBlob)
+        {
+            HPSDF_CUDA(cudaSetDevice(t.device));
+            void* blob = nullptr;
+            size_t bytes = 0;
+            HPSDF_CUDA(acquireBlob(*t.ctx, t.nNodes * (sizeof(double2) + sizeof(uint32_t)), &blob, &bytes));
+            cudaStream_t s = nullptr;
+            cudaError_t e = cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking);
+            if (e == cudaSuccess) e = launchBoundsTable(t.view, (double2*)blob, (uint32_t*)((double2*)blob + t.nNodes), s);
+            if (s)
+            {
+                const cudaError_t es = cudaStreamSynchronize(s);
+                if (e == cudaSuccess) e = es;
+                cudaStreamDestroy(s);
+            }
+            if (e != cudaSuccess) { releaseBlob(*t.ctx, blob, bytes); return failCuda(e, "hpsdf_query_bounds: enclosure table"); }
+            t.dBoundsBlob = blob; t.dBoundsBytes = bytes;
+        }
+        *table = (const double2*)t.dBoundsBlob;
         return HPSDF_OK;
     }
 

@@ -239,6 +239,22 @@ HPSDF_API hpsdf_status hpsdf_query_derivatives(const hpsdf_octree* tree, const d
 HPSDF_API hpsdf_status hpsdf_query_derivatives_device(const hpsdf_octree* tree, const double* d_xyz, size_t n, double* d_value,
                                                       double* d_grad, double* d_hess, void* stream);
 
+/* Bounds of the field hpsdf_query evaluates over n closed axis-aligned boxes [box_lo[i], box_hi[i]] (n x 3 f64, AoS, user
+ * space): for every x in box i, f_lo[i] <= hpsdf_query(x) <= f_hi[i], DBL_MAX outside the root included (DESIGN.md §14; no
+ * counterpart in the reference). f_hi[i] = DBL_MAX when part of the box is outside the root, f_lo[i] = f_hi[i] = DBL_MAX when
+ * all of it is; (NaN, NaN) for a box with a NaN coordinate or box_lo > box_hi on an axis. Infinite coordinates (half-spaces)
+ * and degenerate boxes (planes, segments, points) are allowed. The result is a deterministic function of the tree and the
+ * box: per leaf the hull of the Bernstein coefficients of its polynomial on the box, widened by a stated rounding allowance.
+ * The first call on a tree builds a per-node table (16 bytes per node) on the tree's device and blocks until it is ready.
+ * HOST pointers; blocks the calling thread. HPSDF_ERR_NO_DEVICE without a GPU; HPSDF_ERR_INVALID_ARG for a null tree, or a
+ * null array when n > 0. */
+HPSDF_API hpsdf_status hpsdf_query_bounds(const hpsdf_octree* tree, const double* box_lo, const double* box_hi, size_t n,
+                                          double* f_lo, double* f_hi);
+/* Same with DEVICE pointers, asynchronous on `stream`; the current device must be the tree's (HPSDF_ERR_INVALID_ARG otherwise).
+ * 8-byte alignment. */
+HPSDF_API hpsdf_status hpsdf_query_bounds_device(const hpsdf_octree* tree, const double* d_box_lo, const double* d_box_hi, size_t n,
+                                                 double* d_f_lo, double* d_f_hi, void* stream);
+
 /* Octree::QueryRay (Octree.cpp:705-746, Ray.cpp:5-65) for n rays: origins / directions n x 3 f64, hit n bytes (1 = the march
  * reached a field value below 1e-4 within 200 steps and t_max), t n f64 (the reference stores the last field value there).
  * Statement-by-statement mirror of the reference, see query_kernels.cuh for what that implies outside the default root box. */

@@ -6,8 +6,9 @@
 //                                                                  SubtractSDF / IntersectSDF / Clear / FromMemoryBlock /
 //                                                                  ToMemoryBlock / GetRootAABB, copy + move; plus
 //                                                                  ExtractIsosurface / Raycast / RaycastDevice /
-//                                                                  QueryDerivatives / QueryDerivativesDevice (no
-//                                                                  counterpart in the reference)
+//                                                                  QueryDerivatives / QueryDerivativesDevice /
+//                                                                  QueryBounds / QueryBoundsDevice (no counterpart in
+//                                                                  the reference)
 //     MemoryBlock                 Include/Utility/MemoryBlock.h:5-9
 //
 // Differences, all forced by the device: (1) Create takes an SDF::Program (closed-form primitives / meshes / trees
@@ -246,6 +247,19 @@ namespace SDF
         void QueryDerivativesDevice(const double* dXyz_, size_t n_, double* dValue_, double* dGrad_, double* dHess_, void* stream_) const
         {
             check(hpsdf_query_derivatives_device(need(), dXyz_, n_, dValue_, dGrad_, dHess_, stream_));
+        }
+
+        /// Certified bounds of Query over n_ closed boxes [boxLo_[i], boxHi_[i]] (n_ x 3 each): fLo_[i] <= Query(x) <= fHi_[i] for
+        /// every x in box i, DBL_MAX outside the root included (hpsdf_query_bounds). Host pointers.
+        void QueryBounds(const double* boxLo_, const double* boxHi_, size_t n_, double* fLo_, double* fHi_) const
+        {
+            check(hpsdf_query_bounds(need(), boxLo_, boxHi_, n_, fLo_, fHi_));
+        }
+
+        /// QueryBounds with device pointers, asynchronous on stream_ (hpsdf_query_bounds_device).
+        void QueryBoundsDevice(const double* dBoxLo_, const double* dBoxHi_, size_t n_, double* dFLo_, double* dFHi_, void* stream_) const
+        {
+            check(hpsdf_query_bounds_device(need(), dBoxLo_, dBoxHi_, n_, dFLo_, dFHi_, stream_));
         }
 
         /// The level set F = iso_ as a triangle mesh (hpsdf_extract_isosurface): marching tetrahedra over resolution_ cells per axis
