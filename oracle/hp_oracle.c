@@ -892,6 +892,8 @@ static double builtin_ext(uint32_t op, const void* handle, const double x[3])
 
 void* hporacle_mesh_create(const float* verts, size_t nv, const uint32_t* tris, size_t nt) { return omesh_create(verts, nv, tris, nt); }
 void  hporacle_mesh_destroy(void* m) { omesh_free((OMesh*)m); }
+/* The half-edge twins of a created mesh, 3 per triangle (for tests of the pairing rule). */
+void  hporacle_mesh_half_edges(const void* m, uint32_t* out) { memcpy(out, ((const OMesh*)m)->he, 3 * ((const OMesh*)m)->nt * 4); }
 void  hporacle_mesh_sdf(void* m, const float* xyz, size_t n, float* out, int useBvh, int threads)
 {
     (void)threads;

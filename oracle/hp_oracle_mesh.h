@@ -235,21 +235,29 @@ static OMesh* omesh_create(const float* verts, size_t nv, const uint32_t* tris, 
     m->v = (mv3*)malloc(nv * sizeof(mv3)); memcpy(m->v, verts, nv * 12);
     m->tri = (uint32_t*)malloc(3 * nt * 4); memcpy(m->tri, tris, 3 * nt * 4);
     m->he = (uint32_t*)malloc(3 * nt * 4); memset(m->he, 0xFF, 3 * nt * 4);
-    /* CreateHalfEdges with a sort instead of the std::map: pair every directed edge (a,b) with the first (b,a) */
+    /* CreateHalfEdges (Mesh.cpp:96-118) with a sort instead of the std::map: half-edges sorted by their UNDIRECTED edge, in
+     * index order inside each run, then per run the map's find / insert sequence: "is the reverse edge stored? pair with it :
+     * store this edge unless one of the same direction is already stored". On a non-manifold edge (more than two half-edges)
+     * or a degenerate triangle (a, a, b) this can leave a half-edge unpaired, and the mesh is rejected as the reference does. */
     OEdge* e = (OEdge*)malloc(3 * nt * sizeof(OEdge));
     for (uint32_t i = 0; i < 3 * nt; ++i)
     {
         const uint32_t a = m->tri[i], b = (i % 3 == 2) ? m->tri[i - 2] : m->tri[i + 1];
-        e[i].key = ((uint64_t)a << 32) | b; e[i].idx = i;
+        e[i].key = a < b ? (((uint64_t)a << 32) | b) : (((uint64_t)b << 32) | a); e[i].idx = i;
     }
     qsort(e, 3 * nt, sizeof(OEdge), oedge_cmp);
-    for (uint32_t i = 0; i < 3 * nt; ++i)
+    for (size_t r = 0; r < 3 * nt;)
     {
-        const uint32_t a = m->tri[i], b = (i % 3 == 2) ? m->tri[i - 2] : m->tri[i + 1];
-        const uint64_t rev = ((uint64_t)b << 32) | a;
-        size_t lo = 0, hi = 3 * nt;
-        while (lo < hi) { const size_t mid = (lo + hi) / 2; if (e[mid].key < rev) lo = mid + 1; else hi = mid; }
-        if (lo < 3 * nt && e[lo].key == rev) m->he[i] = e[lo].idx;
+        const uint32_t lo = (uint32_t)(e[r].key >> 32);
+        uint32_t stored[2] = { 0xFFFFFFFFu, 0xFFFFFFFFu };                 /* [0] lo -> hi, [1] hi -> lo */
+        size_t q = r;
+        for (; q < 3 * nt && e[q].key == e[r].key; ++q)
+        {
+            const uint32_t i = e[q].idx, dir = m->tri[i] == lo ? 0u : 1u;
+            if (stored[dir ^ 1u] != 0xFFFFFFFFu) { m->he[stored[dir ^ 1u]] = i; m->he[i] = stored[dir ^ 1u]; }
+            else if (stored[dir] == 0xFFFFFFFFu) stored[dir] = i;
+        }
+        r = q;
     }
     free(e);
     for (uint32_t i = 0; i < 3 * nt; ++i) if (m->he[i] == 0xFFFFFFFFu) { omesh_free(m); return NULL; }

@@ -58,6 +58,7 @@ def lib():
     L.hporacle_mesh_create.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t]
     L.hporacle_mesh_destroy.argtypes = [C.c_void_p]
     L.hporacle_mesh_sdf.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_int, C.c_int]
+    L.hporacle_mesh_half_edges.argtypes = [C.c_void_p, C.c_void_p]
     L.hporacle_set_nearness_mc.argtypes = [C.c_int, C.c_uint64]
     _lib = L
     return L
@@ -162,6 +163,12 @@ class OracleMesh:
         p = np.ascontiguousarray(pts, np.float32)
         out = np.empty(len(p), np.float32)
         lib().hporacle_mesh_sdf(self.h, p.ctypes.data, len(p), out.ctypes.data, 1 if use_bvh else 0, threads)
+        return out
+
+    def half_edges(self):
+        """Twin of every half-edge (3 per triangle, half-edge 3t + k runs from vertex k to vertex k + 1 of triangle t)."""
+        out = np.empty(3 * len(self.t), np.uint32)
+        lib().hporacle_mesh_half_edges(self.h, out.ctypes.data)
         return out
 
     def close(self):

@@ -8,51 +8,9 @@ and errors must be bitwise equal: any box that cut off a closer triangle would s
 import numpy as np
 import pytest
 
-from meshgen import bumpy_torus, mesh_root
+from meshgen import box_mesh, bumpy_torus, mesh_root, tetrahedron
 
 pytestmark = pytest.mark.gpu
-
-
-def box_mesh(k, half=0.3):
-    """Closed axis-aligned cube, every face split into k x k squares of two triangles, counter-clockwise seen from outside:
-    face normals ±x, ±y, ±z (the normal -z and the axis-aligned frames of the wide nodes)."""
-    index, verts, tris = {}, [], []
-
-    def vid(p):
-        if p not in index:
-            index[p] = len(verts)
-            verts.append(p)
-        return index[p]
-
-    for a in range(3):
-        b, c = (a + 1) % 3, (a + 2) % 3
-        for side in (0, k):
-            for i in range(k):
-                for j in range(k):
-                    q = []
-                    for di, dj in ((0, 0), (1, 0), (1, 1), (0, 1)):
-                        p = [0, 0, 0]
-                        p[a], p[b], p[c] = side, i + di, j + dj
-                        q.append(vid(tuple(p)))
-                    if side == k:           # b x c = +a: counter-clockwise in (b, c) faces +a
-                        tris += [(q[0], q[1], q[2]), (q[0], q[2], q[3])]
-                    else:
-                        tris += [(q[0], q[2], q[1]), (q[0], q[3], q[2])]
-    v = (np.array(verts, np.float64) / k * 2 - 1) * half
-    return v.astype(np.float32), np.array(tris, np.uint32)
-
-
-def tetrahedron(s=0.3):
-    """Closed mesh of 4 triangles: one BVH leaf, so the wide tree is the single-leaf root."""
-    v = np.array([[1, 1, 1], [1, -1, -1], [-1, 1, -1], [-1, -1, 1]], np.float64) * s
-    tris = []
-    for f in ((0, 1, 2), (0, 1, 3), (0, 2, 3), (1, 2, 3)):
-        other = ({0, 1, 2, 3} - set(f)).pop()
-        a, b, c = v[list(f)]
-        if np.dot(np.cross(b - a, c - a), a - v[other]) < 0:
-            f = (f[0], f[2], f[1])
-        tris.append(f)
-    return v.astype(np.float32), np.array(tris, np.uint32)
 
 
 MESHES = {
