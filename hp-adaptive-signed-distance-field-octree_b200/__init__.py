@@ -129,7 +129,7 @@ EXPORTS = [
     "hpsdf_comm_destroy", "hpsdf_shard_range", "hpsdf_set_jit", "hpsdf_jit_compile_check", "hpsdf_query_ray",
     "hpsdf_get_config", "hpsdf_get_device", "hpsdf_uniform_points_device", "hpsdf_extract_isosurface",
     "hpsdf_raycast", "hpsdf_raycast_device", "hpsdf_query_derivatives", "hpsdf_query_derivatives_device",
-    "hpsdf_query_bounds", "hpsdf_query_bounds_device",
+    "hpsdf_query_bounds", "hpsdf_query_bounds_device", "hpsdf_extract_isosurface_sparse",
 ]
 
 _lib = None
@@ -178,6 +178,7 @@ def lib():
     L.hpsdf_query_bounds.argtypes = [vp, vp, vp, sz, vp, vp]
     L.hpsdf_query_bounds_device.argtypes = [vp, vp, vp, sz, vp, vp, vp]
     L.hpsdf_extract_isosurface.argtypes = [vp, vp, vp, vp, dbl, C.POINTER(sz), C.POINTER(vp), C.POINTER(sz), C.POINTER(vp)]
+    L.hpsdf_extract_isosurface_sparse.argtypes = L.hpsdf_extract_isosurface.argtypes
     L.hpsdf_to_memory_block.argtypes = [vp, C.POINTER(sz), C.POINTER(vp)]
     L.hpsdf_from_memory_block.argtypes = [vp, sz, i32, C.POINTER(vp)]
     L.hpsdf_clone.argtypes = [vp, C.POINTER(vp)]
@@ -484,15 +485,23 @@ class Octree:
         `resolution` cells per axis (an int or 3 ints, each 1..1024) spanning box = (min xyz, max xyz), or the root box.
         Returns (vertices (n,3) float32, triangles (m,3) uint32), counter-clockwise seen from the side where F >= iso; closed
         when the surface stays inside the box. hp.Mesh(vertices, triangles) takes it as it is."""
+        return self._extract(lib().hpsdf_extract_isosurface, 1024, resolution, iso, box)
+
+    def ExtractIsosurfaceSparse(self, resolution, iso=0.0, box=None):
+        """ExtractIsosurface's mesh, bit for bit, on grids of up to 16384 cells per axis (hpsdf_extract_isosurface_sparse,
+        DESIGN §15): only the blocks of 16^3 cells whose certified bounds (QueryBounds) reach iso are evaluated, so the work
+        and device memory grow with the surface, not with the grid."""
+        return self._extract(lib().hpsdf_extract_isosurface_sparse, 16384, resolution, iso, box)
+
+    def _extract(self, fn, limit, resolution, iso, box):
         res = [int(resolution)] * 3 if np.ndim(resolution) == 0 else [int(r) for r in resolution]
         if len(res) != 3 or not all(0 <= r <= 0xFFFFFFFF for r in res):
-            raise HpsdfError(ERR_INVALID_ARG, "resolution must be one or three counts in [1, 1024]")
+            raise HpsdfError(ERR_INVALID_ARG, "resolution must be one or three counts in [1, %d]" % limit)
         lo = hi = None
         if box is not None:
             lo, hi = ((C.c_double * 3)(*[float(x) for x in b]) for b in box)
         nv, nt, pv, pt = C.c_size_t(), C.c_size_t(), C.c_void_p(), C.c_void_p()
-        _check(lib().hpsdf_extract_isosurface(self._h, (C.c_uint32 * 3)(*res), lo, hi, float(iso), C.byref(nv), C.byref(pv),
-                                              C.byref(nt), C.byref(pt)))
+        _check(fn(self._h, (C.c_uint32 * 3)(*res), lo, hi, float(iso), C.byref(nv), C.byref(pv), C.byref(nt), C.byref(pt)))
         try:
             v = np.ctypeslib.as_array((C.c_float * (3 * nv.value)).from_address(pv.value)).reshape(-1, 3).copy() if nv.value else np.empty((0, 3), np.float32)
             t = np.ctypeslib.as_array((C.c_uint32 * (3 * nt.value)).from_address(pt.value)).reshape(-1, 3).copy() if nt.value else np.empty((0, 3), np.uint32)

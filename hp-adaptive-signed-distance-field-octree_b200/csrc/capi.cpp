@@ -8,6 +8,12 @@
 #include <vector>
 #include "octree.h"
 
+// Grid points from which both isosurface entry points take the sparse pipeline (DESIGN §15 has the measured crossover);
+// set at build time only to measure one pipeline alone (0: always sparse; ~0ull: dense wherever it applies).
+#ifndef HPSDF_ISO_SPARSE_MIN_POINTS
+#define HPSDF_ISO_SPARSE_MIN_POINTS 16974593ull        // 257³: a grid of 256³ cells
+#endif
+
 namespace hpsdf { void printMeshStats(); }      // fit_kernels.cuh (HPSDF_MESH_STATS)
 using namespace hpsdf;
 
@@ -298,25 +304,33 @@ extern "C"
         return HPSDF_OK;
     }
 
-    HPSDF_API hpsdf_status hpsdf_extract_isosurface(const hpsdf_octree* tree, const uint32_t resolution[3], const double box_min[3],
-                                                    const double box_max[3], double iso, size_t* n_vertices, float** vertices,
-                                                    size_t* n_triangles, uint32_t** tri_indices)
+    // Arguments of both extraction entry points: `limit` cells per axis at most.
+    static hpsdf_status isoArgs(const hpsdf_octree* tree, const uint32_t resolution[3], const double box_min[3], const double box_max[3],
+                                double iso, size_t* n_vertices, float** vertices, size_t* n_triangles, uint32_t** tri_indices,
+                                uint32_t limit, const char* fn, IsoGrid& g)
     {
         if (hpsdf_device_count() == 0) return noDevice();
         if (!tree || !resolution || !n_vertices || !vertices || !n_triangles || !tri_indices) { setLastError("null pointer"); return HPSDF_ERR_INVALID_ARG; }
         *n_vertices = 0; *vertices = nullptr; *n_triangles = 0; *tri_indices = nullptr;
-        if (!box_min != !box_max) { setLastError("hpsdf_extract_isosurface: give both box corners or neither"); return HPSDF_ERR_INVALID_ARG; }
-        IsoGrid g;
+        if (!box_min != !box_max) { setLastError(std::string(fn) + ": give both box corners or neither"); return HPSDF_ERR_INVALID_ARG; }
         g.iso = iso;
         for (int a = 0; a < 3; ++a)
         {
-            if (resolution[a] < 1 || resolution[a] > 1024) { setLastError("hpsdf_extract_isosurface: resolution outside [1, 1024]"); return HPSDF_ERR_INVALID_ARG; }
+            if (resolution[a] < 1 || resolution[a] > limit)
+            { setLastError(std::string(fn) + ": resolution outside [1, " + std::to_string(limit) + "]"); return HPSDF_ERR_INVALID_ARG; }
             const double lo = box_min ? box_min[a] : (double)tree->cfg.root_min[a], hi = box_max ? box_max[a] : (double)tree->cfg.root_max[a];
-            if (!(lo < hi) || !std::isfinite(lo) || !std::isfinite(hi)) { setLastError("hpsdf_extract_isosurface: the box needs finite min < max"); return HPSDF_ERR_INVALID_ARG; }
+            if (!(lo < hi) || !std::isfinite(lo) || !std::isfinite(hi)) { setLastError(std::string(fn) + ": the box needs finite min < max"); return HPSDF_ERR_INVALID_ARG; }
             g.n[a] = resolution[a];
             g.lo[a] = lo;
             g.h[a] = (hi - lo) / (double)resolution[a];
         }
+        return HPSDF_OK;
+    }
+
+    // The dense pipeline (isosurface_kernels.cuh, DESIGN §11): every grid point, 18 B of scratch each; 1024 cells per axis at most.
+    static hpsdf_status isoDense(const hpsdf_octree* tree, const IsoGrid& g, size_t* n_vertices, float** vertices, size_t* n_triangles,
+                                 uint32_t** tri_indices)
+    {
         const uint32_t nPoints = (g.n[0] + 1) * (g.n[1] + 1) * (g.n[2] + 1);        // <= 1025^3 < 2^32
         HPSDF_CUDA(cudaSetDevice(tree->device));
         // HPSDF_ISO_TIMES: device time of the phases on stderr (grid, count + scans, emit, copy)
@@ -381,6 +395,191 @@ extern "C"
         if (st != HPSDF_OK) { free(hV); free(hT); return st; }
         *n_vertices = nv; *vertices = hV; *n_triangles = nt; *tri_indices = hT;
         return HPSDF_OK;
+    }
+
+    // The sparse pipeline (isosurface_sparse_kernels.cuh, DESIGN §15): only the blocks whose certified bounds reach iso.
+    static hpsdf_status isoSparse(const hpsdf_octree* tree, const IsoGrid& g, size_t* n_vertices, float** vertices, size_t* n_triangles,
+                                  uint32_t** tri_indices, const char* fn)
+    {
+        HPSDF_CUDA(cudaSetDevice(tree->device));
+        const double2* table = nullptr;
+        hpsdf_status st = ensureBoundsTable(*const_cast<hpsdf_octree*>(tree), &table);
+        if (st != HPSDF_OK) return st;
+        // HPSDF_ISO_TIMES: device time of the phases on stderr (culling, block pass, scans, emit, copy), active blocks per
+        // culling level and peak scratch
+        const bool timed = getenv("HPSDF_ISO_TIMES") != nullptr;
+        cudaStream_t stream = nullptr;
+        cudaEvent_t ev[8] = {};
+        std::vector<std::pair<void*, size_t>> live;          // scratch: every device allocation of the call, freed at the end
+        size_t liveBytes = 0, peakBytes = 0;
+        char* dOut = nullptr;
+        float* hV = nullptr;
+        uint32_t* hT = nullptr;
+        cudaError_t e = cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking);
+        for (int i = 0; i < 8 && timed && e == cudaSuccess; ++i) e = cudaEventCreate(&ev[i]);
+        auto mark = [&](int i) { if (timed && e == cudaSuccess) e = cudaEventRecord(ev[i], stream); };
+        auto take = [&](size_t bytes) -> void*
+        {
+            void* p = nullptr;
+            if (e == cudaSuccess && (e = cudaMallocAsync(&p, std::max<size_t>(bytes, 256), stream)) == cudaSuccess)
+            {
+                live.push_back({ p, bytes });
+                peakBytes = std::max(peakBytes, liveBytes += bytes);
+            }
+            return p;
+        };
+        auto give = [&](void* p)
+        {
+            for (size_t i = 0; i < live.size(); ++i)
+                if (live[i].first == p) { cudaFreeAsync(p, stream); liveBytes -= live[i].second; live.erase(live.begin() + i); return; }
+        };
+        uint32_t hCounters[2] = { 0, 0 };        // culling counters
+        uint32_t* dCounters = (uint32_t*)take(64);
+
+        // Culling: the top level has at most 32 blocks per axis; every level halves the block edge down to kIsoBlock.
+        int level = 0;
+        while (((g.n[0] - 1) >> level) / kIsoBlock >= 32 || ((g.n[1] - 1) >> level) / kIsoBlock >= 32 || ((g.n[2] - 1) >> level) / kIsoBlock >= 32) ++level;
+        uint32_t nb[3];
+        for (int a = 0; a < 3; ++a) nb[a] = (g.n[a] + (kIsoBlock << level) - 1) / (kIsoBlock << level);
+        uint32_t m = nb[0] * nb[1] * nb[2];
+        std::string levels;
+        mark(0);
+        uint32_t* keys = (uint32_t*)take((size_t)m * 4);
+        if (e == cudaSuccess) e = launchIsoCullTop(nb, keys, stream);
+        for (int L = level; L >= 0 && e == cudaSuccess && m; --L)
+        {
+            const uint32_t cells = kIsoBlock << L;
+            double* box = (double*)take((size_t)m * 64);
+            uint32_t* out = (uint32_t*)take((size_t)m * 4 * (L ? 8 : 1));
+            if (e == cudaSuccess) e = launchIsoCullLevel(tree->view, table, g, cells, L == 0, keys, m, box, out, dCounters, tree->ctx->smCount, stream);
+            if (e == cudaSuccess) e = cudaMemcpyAsync(hCounters, dCounters, 8, cudaMemcpyDeviceToHost, stream);
+            if (e == cudaSuccess) e = cudaStreamSynchronize(stream);
+            if (e != cudaSuccess) break;
+            levels += (levels.empty() ? "" : ", ") + std::to_string(cells) + ": " + std::to_string(hCounters[0]) + " / " + std::to_string(m);
+            give(box);
+            give(keys);
+            keys = out;
+            m = hCounters[1];
+        }
+        mark(1);
+
+        // Active blocks in key order, the rank of every row, the block pass and the scans.
+        IsoBlocks B{};
+        B.n = m;
+        size_t nRows[2] = { 0, 0 };
+        unsigned long long totals[2] = { 0, 0 };
+        if (e == cudaSuccess && m)
+        {
+            uint32_t* alt = (uint32_t*)take((size_t)m * 4);
+            size_t tmpBytes = isoSparseTempBytes(m, 0, 0);
+            void* tmp = take(tmpBytes);
+            uint32_t* sorted = nullptr;
+            if (e == cudaSuccess) e = launchIsoSortBlocks(keys, alt, m, tmp, tmpBytes, &sorted, stream);
+            give(sorted == keys ? alt : keys);                // the other buffer of the sort's pair
+            B.keys = sorted;
+            B.metaV = (IsoRowMeta*)take((size_t)m * sizeof(IsoRowMeta));
+            B.metaT = (IsoRowMeta*)take((size_t)m * sizeof(IsoRowMeta));
+            unsigned long long* w = (unsigned long long*)take(((size_t)m + 1) * 64);
+            if (e == cudaSuccess) e = launchIsoRowMeta(g, B, w, tmp, tmpBytes, (unsigned long long*)dCounters, stream);
+            unsigned long long hRows[2] = { 0, 0 };
+            if (e == cudaSuccess) e = cudaMemcpyAsync(hRows, dCounters, 16, cudaMemcpyDeviceToHost, stream);
+            if (e == cudaSuccess) e = cudaStreamSynchronize(stream);
+            give(w);
+            give(tmp);
+            if (e == cudaSuccess)
+            {
+                nRows[0] = hRows[0];
+                nRows[1] = hRows[1];
+                B.tab = (uint16_t*)take((size_t)m * kIsoBlockPts * 2);
+                B.cntV = (uint32_t*)take((nRows[0] + 1) * 4);
+                B.cntT = (uint32_t*)take((nRows[1] + 1) * 4);
+                B.baseV = (unsigned long long*)take((nRows[0] + 1) * 8);
+                B.baseT = (unsigned long long*)take((nRows[1] + 1) * 8);
+                tmpBytes = isoSparseTempBytes(m, nRows[0], nRows[1]);
+                tmp = take(tmpBytes);
+                if (e == cudaSuccess) e = cudaMemsetAsync(B.cntV + nRows[0], 0, 4, stream);
+                if (e == cudaSuccess) e = cudaMemsetAsync(B.cntT + nRows[1], 0, 4, stream);
+                mark(2);
+                if (e == cudaSuccess) e = launchIsoBlockCount(tree->view, g, B, nRows[0], nRows[1], tmp, tmpBytes, stream, timed ? ev[3] : nullptr);
+                if (e == cudaSuccess) e = cudaMemcpyAsync(&totals[0], B.baseV + nRows[0], 8, cudaMemcpyDeviceToHost, stream);
+                if (e == cudaSuccess) e = cudaMemcpyAsync(&totals[1], B.baseT + nRows[1], 8, cudaMemcpyDeviceToHost, stream);
+                mark(4);
+                if (e == cudaSuccess) e = cudaStreamSynchronize(stream);
+                give(tmp);
+                give(B.cntV);
+                give(B.cntT);
+            }
+        }
+        const size_t nv = (size_t)totals[0], nt = (size_t)totals[1];
+        if (e == cudaSuccess && (totals[0] > 0xFFFFFFFFull || totals[1] > 0xFFFFFFFFull))
+        {
+            setLastError(std::string(fn) + ": " + std::to_string(totals[0]) + " vertices and " + std::to_string(totals[1]) +
+                         " triangles: a count above 2^32 - 1 does not fit the uint32 indices");
+            st = HPSDF_ERR_UNSUPPORTED;
+        }
+        const size_t vBytes = (nv * 12 + 255) & ~(size_t)255;
+        if (e == cudaSuccess && st == HPSDF_OK && nv)
+        {
+            dOut = (char*)take(vBytes + nt * 12);
+            hV = (float*)malloc(nv * 12);
+            hT = (uint32_t*)malloc(nt * 12);
+            if (e == cudaSuccess && (!hV || !hT)) { setLastError(std::string(fn) + ": host allocation failed"); st = HPSDF_ERR_OOM; }
+            mark(5);
+            if (e == cudaSuccess && st == HPSDF_OK) e = launchIsoBlockEmit(tree->view, g, B, (float*)dOut, (uint32_t*)(dOut + vBytes), stream);
+            mark(6);
+            if (e == cudaSuccess && st == HPSDF_OK) e = cudaMemcpyAsync(hV, dOut, nv * 12, cudaMemcpyDeviceToHost, stream);
+            if (e == cudaSuccess && st == HPSDF_OK) e = cudaMemcpyAsync(hT, dOut + vBytes, nt * 12, cudaMemcpyDeviceToHost, stream);
+            mark(7);
+            if (e == cudaSuccess) e = cudaStreamSynchronize(stream);
+        }
+        if (timed && e == cudaSuccess && st == HPSDF_OK)
+        {
+            float ms[5] = { 0, 0, 0, 0, 0 };
+            cudaEventElapsedTime(&ms[0], ev[0], ev[1]);
+            if (m) { cudaEventElapsedTime(&ms[1], ev[2], ev[3]); cudaEventElapsedTime(&ms[2], ev[3], ev[4]); }
+            if (nv) { cudaEventElapsedTime(&ms[3], ev[5], ev[6]); cudaEventElapsedTime(&ms[4], ev[6], ev[7]); }
+            fprintf(stderr, "%s: %u x %u x %u cells, %zu vertices, %zu triangles; culling %.3f ms (uncertified / blocks by edge %s), "
+                    "block pass %.3f ms, scans %.3f ms, emit %.3f ms, copy %.3f ms; %u active blocks, %zu + %zu rows, peak scratch %zu bytes\n",
+                    fn, g.n[0], g.n[1], g.n[2], nv, nt, ms[0], levels.c_str(), ms[1], ms[2], ms[3], ms[4], m, nRows[0], nRows[1], peakBytes);
+        }
+        for (auto& p : live) cudaFreeAsync(p.first, stream);
+        if (stream) cudaStreamSynchronize(stream);
+        for (int i = 0; i < 8; ++i) if (ev[i]) cudaEventDestroy(ev[i]);
+        if (stream) cudaStreamDestroy(stream);
+        if (e != cudaSuccess) st = failCuda(e, fn);
+        if (st != HPSDF_OK) { free(hV); free(hT); return st; }
+        *n_vertices = nv; *vertices = hV; *n_triangles = nt; *tri_indices = hT;
+        return HPSDF_OK;
+    }
+
+    // Both pipelines give the same bits. Below HPSDF_ISO_SPARSE_MIN_POINTS grid points the dense one is faster: the sparse
+    // one pays per-level culling launches and read-backs that do not shrink with the grid (crossover measured in DESIGN §15).
+    static hpsdf_status isoExtract(const hpsdf_octree* tree, const uint32_t resolution[3], const double box_min[3], const double box_max[3],
+                                   double iso, size_t* n_vertices, float** vertices, size_t* n_triangles, uint32_t** tri_indices,
+                                   uint32_t limit, const char* fn)
+    {
+        IsoGrid g;
+        const hpsdf_status st = isoArgs(tree, resolution, box_min, box_max, iso, n_vertices, vertices, n_triangles, tri_indices, limit, fn, g);
+        if (st != HPSDF_OK) return st;
+        const uint64_t points = (uint64_t)(g.n[0] + 1) * (g.n[1] + 1) * (g.n[2] + 1);
+        if (g.n[0] <= 1024 && g.n[1] <= 1024 && g.n[2] <= 1024 && points < (uint64_t)HPSDF_ISO_SPARSE_MIN_POINTS)
+            return isoDense(tree, g, n_vertices, vertices, n_triangles, tri_indices);
+        return isoSparse(tree, g, n_vertices, vertices, n_triangles, tri_indices, fn);
+    }
+
+    HPSDF_API hpsdf_status hpsdf_extract_isosurface(const hpsdf_octree* tree, const uint32_t resolution[3], const double box_min[3],
+                                                    const double box_max[3], double iso, size_t* n_vertices, float** vertices,
+                                                    size_t* n_triangles, uint32_t** tri_indices)
+    {
+        return isoExtract(tree, resolution, box_min, box_max, iso, n_vertices, vertices, n_triangles, tri_indices, 1024, "hpsdf_extract_isosurface");
+    }
+
+    HPSDF_API hpsdf_status hpsdf_extract_isosurface_sparse(const hpsdf_octree* tree, const uint32_t resolution[3], const double box_min[3],
+                                                           const double box_max[3], double iso, size_t* n_vertices, float** vertices,
+                                                           size_t* n_triangles, uint32_t** tri_indices)
+    {
+        return isoExtract(tree, resolution, box_min, box_max, iso, n_vertices, vertices, n_triangles, tri_indices, 16384,
+                          "hpsdf_extract_isosurface_sparse");
     }
 
     HPSDF_API hpsdf_status hpsdf_to_memory_block(const hpsdf_octree* tree, size_t* size, void** ptr)

@@ -190,6 +190,41 @@ namespace hpsdf
     // masks, labels, the two scans; hostTotals[0..1] hold the vertex and triangle totals once the stream has drained
     cudaError_t launchIsoCount(const IsoGrid& g, const IsoScratch& s, int smCount, unsigned long long* hostTotals, cudaStream_t stream);
     cudaError_t launchIsoEmit(const IsoGrid& g, const IsoScratch& s, float* dVerts, uint32_t* dTris, cudaStream_t stream);
+    // hpsdf_extract_isosurface_sparse (isosurface_sparse_kernels.cuh): the same mesh from the blocks of kIsoBlock³ cells whose
+    // certified bounds reach iso; grids of up to 16384 cells per axis
+    constexpr uint32_t kIsoBlock = 16, kIsoSide = kIsoBlock + 1, kIsoBlockPts = kIsoSide * kIsoSide * kIsoSide;
+    struct IsoRowMeta { unsigned long long base, strideK, strideJ; };   // rank of a block's local row (lj, lk): base + lk sK + lj sJ
+    struct IsoBlocks
+    {
+        const uint32_t* keys;     // active leaf blocks bi | bj << 10 | bk << 20, ascending
+        uint32_t  n;
+        IsoRowMeta* metaV;        // ranks of the rows of owned points and of cells
+        IsoRowMeta* metaT;
+        uint16_t* tab;            // per block, (B+1)³ entries: owned point's crossing mask | vertices before it in its row << 8
+        uint32_t* cntV;           // vertices / triangles per row in the dense order, then one 0
+        uint32_t* cntT;
+        unsigned long long* baseV;    // their exclusive scans: first vertex / triangle of each row, the totals last
+        unsigned long long* baseT;
+    };
+    // keys of all blocks of `cells` cells per axis in an nb[0] x nb[1] x nb[2] grid of them
+    cudaError_t launchIsoCullTop(const uint32_t nb[3], uint32_t* dKeys, cudaStream_t stream);
+    // bounds of the m blocks of `cells` cells in dKeys (dBox: 8 doubles per block), then the children of `cells / 2` of the
+    // uncertified ones (leaf: the blocks themselves) into dOut; dCounters[0] = uncertified, [1] = written (zeroed here)
+    cudaError_t launchIsoCullLevel(const DeviceTreeView& view, const double2* dTable, const IsoGrid& g, uint32_t cells, bool leaf,
+                                   const uint32_t* dKeys, uint32_t m, double* dBox, uint32_t* dOut, uint32_t* dCounters, int smCount,
+                                   cudaStream_t stream);
+    size_t      isoSparseTempBytes(uint32_t nBlocks, size_t nRowsV, size_t nRowsT);
+    // sorts dKeys (dAlt: as long) and returns the sorted copy
+    cudaError_t launchIsoSortBlocks(uint32_t* dKeys, uint32_t* dAlt, uint32_t n, void* tmp, size_t tmpBytes, uint32_t** sorted,
+                                    cudaStream_t stream);
+    // B.metaV / B.metaT from the sorted keys; dW: 8 (n + 1) u64 of scratch; dRows[0..1] = point rows, cell rows
+    cudaError_t launchIsoRowMeta(const IsoGrid& g, const IsoBlocks& B, unsigned long long* dW, void* tmp, size_t tmpBytes,
+                                 unsigned long long* dRows, cudaStream_t stream);
+    // block pass, then the scans of the row counts (B.cntV / B.cntT need a trailing 0)
+    cudaError_t launchIsoBlockCount(const DeviceTreeView& view, const IsoGrid& g, const IsoBlocks& B, size_t nRowsV, size_t nRowsT,
+                                    void* tmp, size_t tmpBytes, cudaStream_t stream, cudaEvent_t scanStart);
+    cudaError_t launchIsoBlockEmit(const DeviceTreeView& view, const IsoGrid& g, const IsoBlocks& B, float* dVerts, uint32_t* dTris,
+                                   cudaStream_t stream);
     // continuity (continuity_kernels.cuh)
     cudaError_t launchFaceEmit(const FaceJobDev* dFaces, uint32_t nFaces, const DeviceCtx& ctx, uint64_t* keys, double* vals, uint32_t n, cudaStream_t stream);
     size_t      faceEnumTempBytes(uint32_t nNodes);

@@ -26,6 +26,7 @@ namespace hpsdf
 #include "isosurface_kernels.cuh"
 #include "raycast_kernels.cuh"
 #include "bounds_kernels.cuh"
+#include "isosurface_sparse_kernels.cuh"
 
 namespace hpsdf
 {
@@ -605,6 +606,101 @@ namespace hpsdf
         const uint32_t n = isoPoints(g), blocks = (uint32_t)(((size_t)n + 255) / 256);
         isoEmitKernel<<<blocks, 256, 0, stream>>>(g, s.vals, s.mask, s.vbase, dVerts);
         isoTriKernel<<<blocks, 256, 0, stream>>>(g, s.label, s.mask, s.vbase, s.tbase, dTris);
+        return cudaGetLastError();
+    }
+
+    // ---- hpsdf_extract_isosurface_sparse (isosurface_sparse_kernels.cuh) ------------------------------------------------------
+    cudaError_t launchIsoCullTop(const uint32_t nb[3], uint32_t* dKeys, cudaStream_t stream)
+    {
+        const uint32_t n = nb[0] * nb[1] * nb[2];
+        isoCullTopKernel<<<(n + 255) / 256, 256, 0, stream>>>(nb[0], nb[1], n, dKeys);
+        return cudaGetLastError();
+    }
+
+    cudaError_t launchIsoCullLevel(const DeviceTreeView& view, const double2* dTable, const IsoGrid& g, uint32_t cells, bool leaf,
+                                   const uint32_t* dKeys, uint32_t m, double* dBox, uint32_t* dOut, uint32_t* dCounters, int smCount,
+                                   cudaStream_t stream)
+    {
+        double *lo = dBox, *hi = dBox + 3 * (size_t)m, *fLo = dBox + 6 * (size_t)m, *fHi = dBox + 7 * (size_t)m;
+        cudaError_t e = cudaMemsetAsync(dCounters, 0, 8, stream);
+        if (e != cudaSuccess || !m) return e;
+        isoCullBoxesKernel<<<(m + 255) / 256, 256, 0, stream>>>(g, cells, dKeys, m, lo, hi);
+        if ((e = launchBounds(view, dTable, lo, hi, m, fLo, fHi, smCount, stream)) != cudaSuccess) return e;
+        isoCullSplitKernel<<<(m + 255) / 256, 256, 0, stream>>>(g, leaf ? 0u : cells / 2, dKeys, m, fLo, fHi, dOut, dCounters);
+        return cudaGetLastError();
+    }
+
+    size_t isoSparseTempBytes(uint32_t nBlocks, size_t nRowsV, size_t nRowsT)
+    {
+        size_t sort = 0, scanW = 0, scanV = 0, scanT = 0;
+        cub::DeviceRadixSort::SortKeys(nullptr, sort, (uint32_t*)nullptr, (uint32_t*)nullptr, (int)nBlocks, 0, 30, (cudaStream_t)0);
+        cub::DeviceScan::ExclusiveSum(nullptr, scanW, (unsigned long long*)nullptr, (unsigned long long*)nullptr, (int)nBlocks + 1, (cudaStream_t)0);
+        cub::DeviceScan::ExclusiveScan(nullptr, scanV, (uint32_t*)nullptr, (unsigned long long*)nullptr, cub::Sum(), 0ull, nRowsV + 1, (cudaStream_t)0);
+        cub::DeviceScan::ExclusiveScan(nullptr, scanT, (uint32_t*)nullptr, (unsigned long long*)nullptr, cub::Sum(), 0ull, nRowsT + 1, (cudaStream_t)0);
+        return std::max(std::max(sort, scanW), std::max(scanV, scanT)) + 256;
+    }
+
+    cudaError_t launchIsoSortBlocks(uint32_t* dKeys, uint32_t* dAlt, uint32_t n, void* tmp, size_t tmpBytes, uint32_t** sorted, cudaStream_t stream)
+    {
+        cub::DoubleBuffer<uint32_t> kb(dKeys, dAlt);
+        const cudaError_t e = cub::DeviceRadixSort::SortKeys(tmp, tmpBytes, kb, (int)n, 0, 30, stream);
+        *sorted = kb.Current();
+        return e;
+    }
+
+    cudaError_t launchIsoRowMeta(const IsoGrid& g, const IsoBlocks& B, unsigned long long* dW, void* tmp, size_t tmpBytes,
+                                 unsigned long long* dRows, cudaStream_t stream)
+    {
+        const size_t stride = (size_t)B.n + 1;
+        unsigned long long* ps = dW + 4 * stride;
+        isoRowWeightsKernel<<<(B.n + 256) / 256, 256, 0, stream>>>(g, B.keys, B.n, dW);
+        cudaError_t e = cudaGetLastError();
+        for (int k = 0; k < 4 && e == cudaSuccess; ++k)
+        {
+            size_t tb = tmpBytes;
+            e = cub::DeviceScan::ExclusiveSum(tmp, tb, dW + k * stride, ps + k * stride, (int)stride, stream);
+        }
+        if (e != cudaSuccess) return e;
+        isoRowMetaKernel<<<(B.n + 255) / 256, 256, 0, stream>>>(B.keys, B.n, ps, B.metaV, B.metaT);
+        if ((e = cudaGetLastError()) != cudaSuccess) return e;
+        e = cudaMemcpyAsync(dRows, ps + 1 * stride + B.n, 8, cudaMemcpyDeviceToDevice, stream);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(dRows + 1, ps + 3 * stride + B.n, 8, cudaMemcpyDeviceToDevice, stream);
+        return e;
+    }
+
+    static cudaError_t isoBlockSmem(const void* kernel)
+    {
+        static bool set[2][16] = {};
+        int dev = 0;
+        cudaGetDevice(&dev);
+        bool& done = set[kernel == (const void*)isoBlockEmitKernel][dev & 15];
+        if (done) return cudaSuccess;
+        const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kIsoBlockSmem);
+        done = e == cudaSuccess;
+        return e;
+    }
+
+    cudaError_t launchIsoBlockCount(const DeviceTreeView& view, const IsoGrid& g, const IsoBlocks& B, size_t nRowsV, size_t nRowsT,
+                                    void* tmp, size_t tmpBytes, cudaStream_t stream, cudaEvent_t scanStart)
+    {
+        cudaError_t e = isoBlockSmem((const void*)isoBlockCountKernel);
+        if (e != cudaSuccess) return e;
+        isoBlockCountKernel<<<B.n, kQueryThreads, kIsoBlockSmem, stream>>>(view, g, B);
+        if ((e = cudaGetLastError()) != cudaSuccess) return e;
+        if (scanStart && (e = cudaEventRecord(scanStart, stream)) != cudaSuccess) return e;
+        size_t tb = tmpBytes;
+        e = cub::DeviceScan::ExclusiveScan(tmp, tb, B.cntV, B.baseV, cub::Sum(), 0ull, nRowsV + 1, stream);
+        tb = tmpBytes;
+        if (e == cudaSuccess) e = cub::DeviceScan::ExclusiveScan(tmp, tb, B.cntT, B.baseT, cub::Sum(), 0ull, nRowsT + 1, stream);
+        return e;
+    }
+
+    cudaError_t launchIsoBlockEmit(const DeviceTreeView& view, const IsoGrid& g, const IsoBlocks& B, float* dVerts, uint32_t* dTris,
+                                   cudaStream_t stream)
+    {
+        const cudaError_t e = isoBlockSmem((const void*)isoBlockEmitKernel);
+        if (e != cudaSuccess) return e;
+        isoBlockEmitKernel<<<B.n, kQueryThreads, kIsoBlockSmem, stream>>>(view, g, B, dVerts, dTris);
         return cudaGetLastError();
     }
 }

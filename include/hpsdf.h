@@ -296,6 +296,18 @@ HPSDF_API hpsdf_status hpsdf_extract_isosurface(const hpsdf_octree* tree, const 
                                                 size_t* n_vertices, float** vertices,
                                                 size_t* n_triangles, uint32_t** tri_indices);
 
+/* hpsdf_extract_isosurface on grids of 1..16384 cells per axis. The output is the same bit for bit (same vertices, same
+ * triangles, same order) as hpsdf_extract_isosurface for every input that function accepts. On larger grids the same
+ * contract holds unchanged, with 64-bit point and cell indices. The work and device memory grow with the number of grid
+ * blocks (16^3 cells) whose certified bounds (hpsdf_query_bounds) reach iso, not with the grid. The first call on a tree
+ * builds the bounds table, as hpsdf_query_bounds does. Argument rules are those of hpsdf_extract_isosurface, with 16384 as
+ * the limit; HPSDF_ERR_UNSUPPORTED when either count exceeds 2^32 - 1. Both entry points run the same two pipelines and
+ * pick one by grid-point count: the dense one below 257^3 points, the sparse one above (DESIGN.md §15). */
+HPSDF_API hpsdf_status hpsdf_extract_isosurface_sparse(const hpsdf_octree* tree, const uint32_t resolution[3],
+                                                       const double box_min[3], const double box_max[3], double iso,
+                                                       size_t* n_vertices, float** vertices,
+                                                       size_t* n_triangles, uint32_t** tri_indices);
+
 /* Octree::ToMemoryBlock (Octree.cpp:424-456): *ptr is malloc()ed, the CALLER free()s it. LP64 layout. */
 HPSDF_API hpsdf_status hpsdf_to_memory_block(const hpsdf_octree* tree, size_t* size, void** ptr);
 /* Octree::FromMemoryBlock (Octree.cpp:403-421): copies; the caller keeps ownership of the block. */

@@ -5,7 +5,8 @@
 //     SDF::Octree                 Include/HP/Octree.h:36-86        Create / Query / QueryWithGradient / QueryRay / UnionSDF /
 //                                                                  SubtractSDF / IntersectSDF / Clear / FromMemoryBlock /
 //                                                                  ToMemoryBlock / GetRootAABB, copy + move; plus
-//                                                                  ExtractIsosurface / Raycast / RaycastDevice /
+//                                                                  ExtractIsosurface / ExtractIsosurfaceSparse /
+//                                                                  Raycast / RaycastDevice /
 //                                                                  QueryDerivatives / QueryDerivativesDevice /
 //                                                                  QueryBounds / QueryBoundsDevice (no counterpart in
 //                                                                  the reference)
@@ -268,14 +269,15 @@ namespace SDF
         void ExtractIsosurface(const uint32_t resolution_[3], double iso_, std::vector<float>& vertices_, std::vector<uint32_t>& triIndices_,
                                const double* boxMin_ = nullptr, const double* boxMax_ = nullptr) const
         {
-            size_t nv = 0, nt = 0;
-            float* v = nullptr;
-            uint32_t* t = nullptr;
-            check(hpsdf_extract_isosurface(need(), resolution_, boxMin_, boxMax_, iso_, &nv, &v, &nt, &t));
-            std::unique_ptr<float, void (*)(void*)> ownV(v, std::free);
-            std::unique_ptr<uint32_t, void (*)(void*)> ownT(t, std::free);
-            vertices_.assign(v, v + 3 * nv);
-            triIndices_.assign(t, t + 3 * nt);
+            extract(hpsdf_extract_isosurface, resolution_, iso_, vertices_, triIndices_, boxMin_, boxMax_);
+        }
+
+        /// The same mesh, bit for bit, on grids of up to 16384 cells per axis (hpsdf_extract_isosurface_sparse): only the blocks
+        /// of the grid whose certified bounds reach iso_ are evaluated, so work and device memory grow with the surface.
+        void ExtractIsosurfaceSparse(const uint32_t resolution_[3], double iso_, std::vector<float>& vertices_, std::vector<uint32_t>& triIndices_,
+                                     const double* boxMin_ = nullptr, const double* boxMax_ = nullptr) const
+        {
+            extract(hpsdf_extract_isosurface_sparse, resolution_, iso_, vertices_, triIndices_, boxMin_, boxMax_);
         }
 
         /// The aabb of the root node (Octree.cpp:106-109)
@@ -287,6 +289,19 @@ namespace SDF
     private:
         hpsdf_octree* h_ = nullptr;
         const hpsdf_octree* need() const { if (!h_) throw Error(HPSDF_ERR_INVALID_ARG, "octree is empty"); return h_; }
+        template <typename Fn>
+        void extract(Fn fn_, const uint32_t resolution_[3], double iso_, std::vector<float>& vertices_, std::vector<uint32_t>& triIndices_,
+                     const double* boxMin_, const double* boxMax_) const
+        {
+            size_t nv = 0, nt = 0;
+            float* v = nullptr;
+            uint32_t* t = nullptr;
+            check(fn_(need(), resolution_, boxMin_, boxMax_, iso_, &nv, &v, &nt, &t));
+            std::unique_ptr<float, void (*)(void*)> ownV(v, std::free);
+            std::unique_ptr<uint32_t, void (*)(void*)> ownT(t, std::free);
+            vertices_.assign(v, v + 3 * nv);
+            triIndices_.assign(t, t + 3 * nt);
+        }
         void combine(const Program& F_, uint32_t op_, const hpsdf_build_opts* opts_)
         {
             Octree oldTree = std::move(*this);                          // keeps the old tree alive until Create returns (Octree.cpp:366)
